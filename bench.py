@@ -2,7 +2,7 @@
 """Benchmark of the TZDDPC hot path: closed-loop steps/sec over batched scenarios.
 
     python bench.py [--gpus N] [--steps K] [--warmup W] [--impl reference] [--workload fivedim|pulley|double_integrator]
-                    [--scaling strong|weak] [--scenarios S]
+                    [--scaling strong|weak] [--scenarios S] [--dump-outputs DIR]
     python -m torch.distributed.run --nnodes=1 --nproc-per-node N ... bench.py --gpus N --steps K --warmup W
 
 A "step" is ONE fused closed-loop step (solve + tube + plant/nominal/error update,
@@ -289,6 +289,37 @@ class ClosedLoop:
         self.ops.closed_loop_step(self.h, self.x, self.xbar, self.e, self.noise[t % self.nring], self.x0, self.At, self.Bt,
                                   self.status[r], self.cost[r], self.v[r], None if self.ablate >= 2 else self.traj[r],
                                   None if self.ablate >= 1 else self.ze1[r], None, self.iters[r], self.warm, self.stats[t], self.po)
+
+    def outputs(self, t):
+        """What the caller of `step(t)`, the latest step, received: the updated state and the step's results, each (rows, S)."""
+        r = t % self.ring
+        out = {"x": self.x, "xbar": self.xbar, "e": self.e, "status": self.status[r][None], "cost": self.cost[r][None],
+               "v": self.v[r], "iters": self.iters[r][None]}
+        if self.ablate < 2:
+            out["xbar_traj"] = self.traj[r]
+        if self.ablate < 1:
+            out["tube"] = self.ze1[r]
+        return out
+
+
+DUMP_BYTES = 60_000_000      # --dump-outputs stays below 64 MB: a fixed sample of the scenarios when a step's outputs are larger
+
+
+def dump_outputs(out_dir, loop, t, s_begin):
+    """Writes what step t of `loop` returned as out_dir/<name>.npy in float64, scenarios along the last axis.  When all
+    scenarios do not fit in DUMP_BYTES, every array keeps the same seeded sample of them; scenario.npy holds the global
+    index of each column.  stats.npy is the step's statistics row, summed with atomics (equal up to summation order)."""
+    torch = loop.torch
+    os.makedirs(out_dir, exist_ok=True)
+    arrays = loop.outputs(t)
+    per_scenario = 8 * (1 + sum(a.shape[0] for a in arrays.values()))
+    k = min(loop.S, DUMP_BYTES // per_scenario)
+    idx = np.arange(loop.S) if k == loop.S else np.sort(np.random.default_rng(0).choice(loop.S, k, replace=False))
+    sel = torch.as_tensor(idx, device=loop.dev)
+    np.save(os.path.join(out_dir, "scenario.npy"), (s_begin + idx).astype(np.float64))
+    for name, a in arrays.items():
+        np.save(os.path.join(out_dir, f"{name}.npy"), a.index_select(1, sel).cpu().numpy().astype(np.float64))
+    np.save(os.path.join(out_dir, "stats.npy"), loop.stats[t].cpu().numpy())
 
 
 def _nvtx_push(torch, msg):
@@ -843,6 +874,8 @@ def run_gpu(args):
     cnt = max(tot_stats[7], 1.0)
     if args.dump_steps and rank == 0:
         np.savez(args.dump_steps, kern_ms=np.asarray(kern_ms), stats=stats.cpu().numpy())
+    if args.dump_outputs and rank == 0:          # before any later leg reuses `dense`
+        dump_outputs(args.dump_outputs, dense, W_steps + K_steps - 1, s_begin)
     value = S_total * K_steps / (elapsed_ms * 1e-3)
     rows_headline = nnz if args.packed else n * (1 + g1)
     bstep = algorithmic_bytes_per_scenario_step(n, m, N, g1, rows_headline)
@@ -1008,6 +1041,8 @@ def main():
     ap.add_argument("--cpu-scen", type=int, default=48, help="scenarios per core of the CPU baseline")
     ap.add_argument("--cpu-cores", type=int, default=0, help="processes of the CPU baseline (0 = all host cores)")
     ap.add_argument("--dump-steps", default="", help="write per-step kernel ms and solver statistics to this .npz (diagnostics)")
+    ap.add_argument("--dump-outputs", default="", metavar="DIR",
+                    help="write the outputs of the last timed step as DIR/<name>.npy (float64, under 64 MB; rank 0's shard)")
     ap.add_argument("--ablate", type=int, default=0, help="diagnostics only: 1 = do not write Ze[1].Z, 2 = nor the trajectory")
     ap.add_argument("--hot-path", type=int, default=1, help="0: the ADMM kernel for every tile (diagnostics)")
     ap.add_argument("--packed", type=int, default=0, help="1: packed tube in the device-timed headline leg (diagnostics)")
@@ -1019,6 +1054,10 @@ def main():
     ap.add_argument("--no-e2e", action="store_true")
     ap.add_argument("--no-cpu-baseline", action="store_true")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and (args.impl == "reference" or args.workload == "stress"):
+        ap.error("--dump-outputs writes the native closed-loop step; it has no meaning for --impl reference or --workload stress")
     if args.warmup < 3:
         args.warmup = 3
     if args.workload == "stress":

@@ -4,6 +4,7 @@ import ctypes as C
 import os
 import re
 import subprocess
+from pathlib import Path
 
 import pytest
 
@@ -27,11 +28,13 @@ def test_library_exports_every_declared_symbol(cuda_lib):
         assert hasattr(cuda_lib, name), f"libtzddpc.so does not export {name}"
 
 
-def test_library_is_sm100a_and_self_contained():
-    from tzddpc_b200 import _abi
-    out = subprocess.run(["cuobjdump", "--list-elf", str(_abi.LIB_PATH)], capture_output=True, text=True)
-    if out.returncode != 0:
+def test_library_is_sm100a_and_self_contained(cuda_lib):
+    from tzddpc_b200 import _abi, build
+    cuobjdump = Path(build._nvcc()).with_name("cuobjdump")       # the toolkit that built the library, whether on PATH or not
+    if not cuobjdump.exists():
         pytest.skip("cuobjdump not available")
+    out = subprocess.run([str(cuobjdump), "--list-elf", str(_abi.LIB_PATH)], capture_output=True, text=True)
+    assert out.returncode == 0, out.stderr
     assert "sm_100a" in out.stdout
     ldd = subprocess.run(["ldd", str(_abi.LIB_PATH)], capture_output=True, text=True).stdout
     assert "libtorch" not in ldd and "libcudart" not in ldd        # plain C ABI, static CUDA runtime
