@@ -124,8 +124,13 @@ typedef struct TzSolverOpts {
   int32_t check_every;/* residual check period                     default 8    */
   int32_t polish;    /* masked augmented-Lagrangian polish: number of iterations, 0 = off   default 3 */
   int32_t warm_start;/* 0 cold; 1 reuse (x, y) of the previous call from the `warm` buffer; 2 active-set hint:
-                        the previous call's optimal active set is tried first (KKT-certified, so a stale
-                        hint only costs the test); the buffer carries one word per lane        default 0 */
+                        the previous call's optimal active set is tried first and accepted only when the KKT
+                        conditions hold there; a code that cannot mean anything for its row (equality on a row
+                        whose bounds differ, kink on a row without an |.| cost, a missing bound) rejects the
+                        hint.  So a stale or arbitrary hint only costs the test (tested against an exact
+                        optimum for every hint with up to two active rows and for random words, two-variable
+                        programs; against the oracle for larger ones); the buffer carries one word per lane
+                        default 0 */
   int32_t cert_first;/* first iteration at which the active-set KKT certificate is tried (then on a
                         geometric schedule); a certified iterate is an exact solution and ends the
                         solve at once.  0 = off (terminate on residuals only)        default 3    */
@@ -219,8 +224,9 @@ int tz_closed_loop_step_set(const TzProgramSet* set, const TzSolverOpts* opts, i
  * copies overlap compute; synchronises before returning.  `dev_scratch` is caller-owned
  * device memory of at least tz_closed_loop_step_host_scratch_bytes(prog, S).  With opts->warm_start != 0 its tail
  * carries the solver's warm-start rows (active-set hints) from one call to the next: zero it once before the first
- * call of a run and pass the same buffer every step (a stale or foreign hint is KKT-checked before use, so it can cost
- * time but not correctness).  With opts->tube_packed, ze1_host is n_nz x S. */
+ * call of a run and pass the same buffer every step (a stale or foreign hint is KKT-checked before use, and rejected
+ * when a code does not fit its row, so it can cost time but not correctness; see warm_start).  With opts->tube_packed,
+ * ze1_host is n_nz x S. */
 size_t tz_closed_loop_step_host_scratch_bytes(const TzProgram* prog, int64_t S);
 int tz_closed_loop_step_host(const TzProgram* prog, const TzSolverOpts* opts, int64_t S,
                              double* x_host, double* xbar_host, double* e_host, const double* noise_host,

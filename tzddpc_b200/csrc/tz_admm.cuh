@@ -419,6 +419,12 @@ __device__ __forceinline__ bool admm_certify(const LaneQp<BK>& qp, double inv_al
     const double ax = axs[k];
     const unsigned c = cof(k);
     bad |= (qp.lower(k) - ax > ptol) || (ax - qp.upper(k) > ptol);                 // primal feasibility
+    // the code is caller memory when it comes from a hint: it must mean something for its row -- 6 only where the bounds
+    // coincide, 3 only on a row with a |.| cost, 1 / 2 only on a finite bound, and a |.| row is on its kink, on a side of
+    // it or on a bound (never 0 / 7, which would drop its cost).  active_code writes nothing else.
+    const bool kinked = k < N2 && qp.wk[(k < N2 ? k : 0) * G] > 0.0;
+    bad |= (c == 6u && qp.lower(k) < qp.upper(k)) || (c == 3u && !kinked) || (c == 1u && !(qp.lower(k) > -INFINITY)) ||
+           (c == 2u && !(qp.upper(k) < INFINITY)) || (kinked && (c == 0u || c == 7u));
     if ((am >> k) & 1u) {
       const double rl = k < N2 ? rlx[k < N2 ? k : 0] * inv_alpha : 0.0;
       bad |= fabs(ax - tgt[k] * inv_alpha) > etol;                                // active rows on their bound

@@ -130,11 +130,20 @@ __device__ __forceinline__ Cert2Result certify2(const QpProg<BK>& pg, const doub
   const double trP = P00 + P11;
   double x0 = 0.0, x1 = 0.0, la = 0.0, lb = 0.0;
   double a0 = 0.0, a1 = 0.0, b0_ = 0.0, b1_ = 0.0;
+  // the bound or kink an active row's code pins it to.  The hint is caller memory, so a code that means nothing for its
+  // row is rejected: 6 (equality) on a row whose bounds differ, 3 on a slot without a |.| cost, 1 / 2 on a missing bound
+  // -- pinned anyway, such a row makes a feasible vertex pass every KKT test that follows (its multiplier sign is never
+  // tested).  The predicates are those of active_code, so a hint the solver wrote itself always passes them.
   auto target = [&](int i, unsigned c, double& A0, double& A1) {
     const double r = row_shift<BK>(pg, i, w);
+    const double lo = pg.l0[i] + r, hi = pg.u0[i] + r;
     A0 = pg.A[i][0];
     A1 = pg.A[i][1];
-    return (c == 2u ? pg.u0[i] : (c == 3u ? pg.kink0[i % NK] : pg.l0[i])) + r;
+    if (c == 6u) bad = bad || (lo < hi);
+    else if (c == 3u) bad = bad || !(i < NK && pg.wabs[i < NK ? i : 0] > 0.0);
+    else if (c == 1u) bad = bad || !(lo > -INFINITY);
+    else bad = bad || !(hi < INFINITY);
+    return c == 2u ? hi : (c == 3u ? pg.kink0[i % NK] + r : lo);
   };
   if (na == 0) {
     const double det = P00 * P11 - P01 * P01;
