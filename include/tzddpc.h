@@ -196,6 +196,24 @@ int tz_closed_loop_run(const TzProgram* prog, const TzSolverOpts* opts, int64_t 
                        double* e_hist, int32_t* status, int32_t* iters, double* warm, double* stats, void* stream);
 
 /* ------------------------------------------------------------------------------------
+ * A plant per scenario: tz_closed_loop_step / tz_closed_loop_run (and tz_closed_loop_step_set below) with
+ *   AB_true       n(n+m) x S   (SoA) in place of A_true, B_true: entry (i, k) of scenario s's [A_true B_true] at
+ *                 AB_true[(i (n+m) + k) S + s] -- the layout tz_sample_plants writes.
+ * Run a closed loop per plant of a set (e.g. plants drawn from M_Sigma, to check the tube guarantee on every plant the data
+ * cannot rule out), or each data set's closed loop on the system that produced its data.  With every column equal to
+ * [A_true B_true] the results equal the shared-plant call bit for bit.
+ * ------------------------------------------------------------------------------------ */
+int tz_closed_loop_step_plants(const TzProgram* prog, const TzSolverOpts* opts, int64_t S,
+                               double* x, double* xbar, double* e, const double* noise, const double* x_restart,
+                               const double* AB_true,
+                               double* cost, double* v, double* xbar_traj, double* ze1, double* u_out,
+                               int32_t* status, int32_t* iters, double* warm, double* stats, void* stream);
+int tz_closed_loop_run_plants(const TzProgram* prog, const TzSolverOpts* opts, int64_t S, int32_t nsteps, double* x, double* xbar,
+                              double* e, const double* noise, const double* x_restart, const double* AB_true,
+                              double* cost, double* v, double* xbar_traj, double* ze1, double* u_out, double* x_hist, double* xbar_hist,
+                              double* e_hist, int32_t* status, int32_t* iters, double* warm, double* stats, void* stream);
+
+/* ------------------------------------------------------------------------------------
  * Data-set axis (BASELINE.json north_star: scenarios = noise realisations x initial states x data sets).
  * The reference builds one TZDDPC object -- one model M_Sigma, one problem -- per data set (tzddpc/tzddpc.py:20-28,
  * 67-85,132-241) and runs them one after another.  A program set runs D such programs in ONE launch: scenarios
@@ -218,6 +236,12 @@ int tz_closed_loop_step_set(const TzProgramSet* set, const TzSolverOpts* opts, i
                             const double* A_true, const double* B_true,
                             double* cost, double* v, double* xbar_traj, double* ze1, double* u_out,
                             int32_t* status, int32_t* iters, double* warm, double* stats, void* stream);
+/* tz_closed_loop_step_set with a plant per scenario, AB_true n(n+m) x S as tz_closed_loop_step_plants */
+int tz_closed_loop_step_set_plants(const TzProgramSet* set, const TzSolverOpts* opts, int64_t S,
+                                   double* x, double* xbar, double* e, const double* noise, const double* x_restart,
+                                   const double* AB_true,
+                                   double* cost, double* v, double* xbar_traj, double* ze1, double* u_out,
+                                   int32_t* status, int32_t* iters, double* warm, double* stats, void* stream);
 
 /* Same step with HOST buffers (pinned or pageable): H2D of (x, xbar, e, noise), the fused
  * kernel, D2H of every non-NULL output, chunked over `nchunks` internal streams so that
@@ -352,6 +376,22 @@ int tz_sample_noise(int64_t S, int64_t ld, int32_t n, int32_t gW, const double* 
 int tz_generate_trajectories(int64_t S, int32_t T, int32_t n, int32_t m, int32_t g0, int32_t gU, int32_t gW,
                              const double* A, const double* B, const double* X0Z, const double* UZ, const double* WZ,
                              uint64_t seed, int64_t scenario_offset, double* U, double* X, void* stream);
+/* The same with a plant per data set: A S x n x n, B S x n x m (data set s from A + s n n, B + s n m). */
+int tz_generate_trajectories_plants(int64_t S, int32_t T, int32_t n, int32_t m, int32_t g0, int32_t gU, int32_t gW,
+                                    const double* A, const double* B, const double* X0Z, const double* UZ, const double* WZ,
+                                    uint64_t seed, int64_t scenario_offset, double* U, double* X, void* stream);
+
+/* Plants drawn from the data-consistent model set M_Sigma = (X1 - M_w) pinv([X0; U0]) (tzddpc/tzddpc.py:81-83), one per scenario:
+ *   [A B] = AB_d - G_W R,   R[k, :] = sum_j beta_kj Pinv_d[j, :],   beta_kj ~ U[-1, 1)
+ * i.e. AB_d + sum_g beta_g G_g over the generators G_g = -G_W[:, k] Pinv_d[j, :], g = k (T-1) + j, of the UN-REDUCED M_Sigma
+ * (the order-1 box of tz_identify's dAB is larger than M_Sigma: a plant drawn from it is not covered by the tube).
+ *   AB    D x n x (n+m), Pinv  D x (T-1) x (n+m)   as tz_identify writes them;  WZ  n x (1+gW)
+ *   dataset  S int32: data set d of each scenario (an index outside [0, D) gives a NaN plant), or NULL: data set 0
+ *   AB_out   n(n+m) x S  -- the AB_true layout of tz_closed_loop_step_plants
+ * Draws: Philox stream (seed, scenario_offset + s, t = 0, purpose 6, draw g); gW (T-1) <= 131072. */
+int tz_sample_plants(int64_t S, int32_t D, int32_t T, int32_t n, int32_t m, int32_t gW, const double* AB, const double* Pinv,
+                     const double* WZ, const int32_t* dataset, uint64_t seed, int64_t scenario_offset, double* AB_out,
+                     void* stream);
 
 /* Generic batched ADMM QP on an explicit instance batch (the solver stage alone):
  *   minimise 0.5 z'Pz + q_s'z  s.t. l_s <= A z <= u_s   with (P, A) from `prog`

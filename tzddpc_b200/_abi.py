@@ -45,7 +45,8 @@ EXPORTS = ["tz_version", "tz_last_error", "tz_device_cc", "tz_program_create", "
            "tz_program_tube_pattern", "tz_program_set_create", "tz_program_set_destroy", "tz_program_set_scenarios",
            "tz_solve_set", "tz_closed_loop_step_set", "tz_gain_synthesis", "tz_gain_robust_samples", "tz_gain_adversary", "tz_program_dims",
            "tz_program_set_dims", "tz_closed_loop_run_host", "tz_program_create_batch",
-           "tz_program_batch_get", "tz_program_batch_destroy", "tz_closed_loop_run"]
+           "tz_program_batch_get", "tz_program_batch_destroy", "tz_closed_loop_run", "tz_closed_loop_step_plants",
+           "tz_closed_loop_step_set_plants", "tz_closed_loop_run_plants", "tz_sample_plants", "tz_generate_trajectories_plants"]
 
 
 def lib() -> C.CDLL:
@@ -84,6 +85,10 @@ def lib() -> C.CDLL:
     L.tz_closed_loop_step.argtypes = [vp, C.POINTER(TzSolverOpts), i64] + [vp] * 17
     L.tz_closed_loop_run.restype = C.c_int
     L.tz_closed_loop_run.argtypes = [vp, C.POINTER(TzSolverOpts), i64, C.c_int32] + [vp] * 20
+    L.tz_closed_loop_step_plants.restype = C.c_int
+    L.tz_closed_loop_step_plants.argtypes = [vp, C.POINTER(TzSolverOpts), i64] + [vp] * 16
+    L.tz_closed_loop_run_plants.restype = C.c_int
+    L.tz_closed_loop_run_plants.argtypes = [vp, C.POINTER(TzSolverOpts), i64, C.c_int32] + [vp] * 19
     L.tz_program_dims.restype = C.c_int
     L.tz_program_dims.argtypes = [vp, vp]
     L.tz_program_set_dims.restype = C.c_int
@@ -100,6 +105,8 @@ def lib() -> C.CDLL:
     L.tz_solve_set.argtypes = [vp, C.POINTER(TzSolverOpts), i64] + [vp] * 10
     L.tz_closed_loop_step_set.restype = C.c_int
     L.tz_closed_loop_step_set.argtypes = [vp, C.POINTER(TzSolverOpts), i64] + [vp] * 17
+    L.tz_closed_loop_step_set_plants.restype = C.c_int
+    L.tz_closed_loop_step_set_plants.argtypes = [vp, C.POINTER(TzSolverOpts), i64] + [vp] * 16
     L.tz_closed_loop_step_host_scratch_bytes.restype = C.c_size_t
     L.tz_closed_loop_step_host_scratch_bytes.argtypes = [vp, i64]
     L.tz_closed_loop_step_host.restype = C.c_int
@@ -121,6 +128,10 @@ def lib() -> C.CDLL:
     L.tz_sample_noise.argtypes = [i64, i64, i32, i32, vp, i32, u64, i64, u32, vp, vp]
     L.tz_generate_trajectories.restype = C.c_int
     L.tz_generate_trajectories.argtypes = [i64] + [i32] * 6 + [vp] * 5 + [u64, i64, vp, vp, vp]
+    L.tz_generate_trajectories_plants.restype = C.c_int
+    L.tz_generate_trajectories_plants.argtypes = [i64] + [i32] * 6 + [vp] * 5 + [u64, i64, vp, vp, vp]
+    L.tz_sample_plants.restype = C.c_int
+    L.tz_sample_plants.argtypes = [i64] + [i32] * 5 + [vp] * 4 + [u64, i64, vp, vp]
     L.tz_identify.restype = C.c_int
     L.tz_identify.argtypes = [i64, i32, i32, i32, i32] + [vp] * 10
     L.tz_gain_synthesis.restype = C.c_int

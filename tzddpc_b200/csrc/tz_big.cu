@@ -195,6 +195,8 @@ __device__ bool certify_w(const BigDev& B, const Scratch& S, const double* q, in
   return ok;
 }
 
+// PL: a plant per scenario (StepArgs::AB_true)
+template <bool PL = false>
 __global__ void __launch_bounds__(kBigWarps * 32) big_step_kernel(const BigArgs g) {
   extern __shared__ __align__(16) double smem_d[];
   const BigDev& B = g.p;
@@ -493,8 +495,14 @@ __global__ void __launch_bounds__(kBigWarps * 32) big_step_kernel(const BigArgs 
     if (lane < n) {
       const int i = lane;
       double xn = a.noise ? a.noise[(int64_t)i * LD + s] : 0.0;
-      for (int k = 0; k < n; ++k) xn = fma(a.A_true[i * n + k], a.x[(int64_t)k * LD + s], xn);
-      for (int k = 0; k < m; ++k) xn = fma(a.B_true[i * m + k], u[k], xn);
+      if constexpr (PL) {
+        const double* ab = a.AB_true + (int64_t)i * (n + m) * LD + s;
+        for (int k = 0; k < n; ++k) xn = fma(ab[(int64_t)k * LD], a.x[(int64_t)k * LD + s], xn);
+        for (int k = 0; k < m; ++k) xn = fma(ab[(int64_t)(n + k) * LD], u[k], xn);
+      } else {
+        for (int k = 0; k < n; ++k) xn = fma(a.A_true[i * n + k], a.x[(int64_t)k * LD + s], xn);
+        for (int k = 0; k < m; ++k) xn = fma(a.B_true[i * m + k], u[k], xn);
+      }
       double xb1 = 0.0;
       for (int j = 0; j < nwc; ++j) xb1 = fma(B.XB[(n + i) * nwc + j], S.om[j], xb1);
       double en = xn - xb1;
@@ -635,9 +643,10 @@ int big_launch(const BigProgram* bp, const SolverParams& sp, const StepArgs& a, 
   g.a = a;
   const size_t smem = (size_t)kBigWarps * bp->dev.scratch_doubles * sizeof(double);
   if (smem > 200 * 1024) return fail(TZ_ERANGE, "program needs %zu bytes of shared memory per CTA", smem);
-  TZ_CUDA(cudaFuncSetAttribute(big_step_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
+  auto kernel = a.AB_true != nullptr ? big_step_kernel<true> : big_step_kernel<false>;
+  TZ_CUDA(cudaFuncSetAttribute(kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
   const unsigned grid = (unsigned)((a.S + kBigWarps - 1) / kBigWarps);
-  big_step_kernel<<<grid, kBigWarps * 32, smem, st>>>(g);
+  kernel<<<grid, kBigWarps * 32, smem, st>>>(g);
   TZ_CUDA(cudaGetLastError());
   return TZ_OK;
 }

@@ -57,7 +57,11 @@ constexpr int fast_ctas_per_sm(int tpb) { return tpb >= 512 ? 1 : 512 / tpb; }
 // (Measured and dropped, round 2 again: the zeros as bulk copies -- cp.async.bulk shared -> global of a TPB * 8-byte block
 // of zeros, one 2 KB copy per zero row and CTA block, issued by the block's threads a row each, either all behind the
 // staging barrier or spread over the drip sites: 0.072-0.073 ms against 0.060-0.061 with the dripped 16-byte stores.)
-template <class BK, int TPB, int NSLOT, int H = 1>
+// PL: a plant per scenario (StepArgs::AB_true), read at the update.  Loads there come after the step's first stores, so every
+// thread prefetches its scenario's n(n+m) plant entries into L2 together with the step's other loads; holding them in registers
+// instead would need 2 n(n+m) = 60 of them for the 5-dim system on top of a budget of 128, and staging them in shared memory
+// next to x and the noise 30 rows of om, 60 KB per 256-thread CTA (one resident CTA per SM instead of two).
+template <class BK, int TPB, int NSLOT, int H = 1, bool PL = false>
 __global__ void __launch_bounds__(TPB * H, fast_ctas_per_sm(TPB * H))
     fast_step_kernel(const QpProg<BK>* __restrict__ gpg, const Aux ax, const SolverParams sp, const StepArgs a,
                      const SetEntry* __restrict__ entries, const int32_t* __restrict__ tile_prog, const int slot_bytes) {
@@ -91,7 +95,7 @@ __global__ void __launch_bounds__(TPB * H, fast_ctas_per_sm(TPB * H))
   };
   auto stage_plant = [&](unsigned char* slot) {              // (caller-owned arrays: behind pdl_wait)
     double* td = reinterpret_cast<double*>(slot + QPB);
-    if (closed) {
+    if (closed && !PL) {
       for (int i = tix; i < n * n; i += NT) cp_async8(td + n_tab + i, a.A_true + i);
       for (int i = tix; i < n * m; i += NT) cp_async8(td + n_tab + n * n + i, a.B_true + i);
     }
@@ -219,6 +223,10 @@ __global__ void __launch_bounds__(TPB * H, fast_ctas_per_sm(TPB * H))
           if (a.noise) cp_async8(&om[OM_NS + i][tid], a.noise + (int64_t)i * LD + sc);
         }
       cp_async_commit();
+      if constexpr (PL) {
+        const int nm = n + m;
+        for (int r = 0; r < n * nm; ++r) asm volatile("prefetch.global.L2 [%0];" ::"l"(a.AB_true + (int64_t)r * LD + sc));
+      }
     }
     if (!staged) {
       cp_async_wait<0>();
@@ -435,12 +443,22 @@ __global__ void __launch_bounds__(TPB * H, fast_ctas_per_sm(TPB * H))
         for (int i = 0; i < HP; ++i) {
           if (i < n) {
             double acc = a.noise ? omc[(OM_NS + i) * TPB] : 0.0;
+            if constexpr (PL) {
+              const double* ab = a.AB_true + (int64_t)i * (n + m) * LD + s;        // row i of this scenario's [A_true B_true]
 #pragma unroll
-            for (int k = 0; k < HP; ++k)
-              if (k < n) acc = fma(sA[i * n + k], xo[k], acc);
+              for (int k = 0; k < HP; ++k)
+                if (k < n) acc = fma(ab[(int64_t)k * LD], xo[k], acc);
 #pragma unroll
-            for (int k = 0; k < kMaxM; ++k)
-              if (k < m) acc = fma(sB[i * m + k], us[k], acc);
+              for (int k = 0; k < kMaxM; ++k)
+                if (k < m) acc = fma(ab[(int64_t)(n + k) * LD], us[k], acc);
+            } else {
+#pragma unroll
+              for (int k = 0; k < HP; ++k)
+                if (k < n) acc = fma(sA[i * n + k], xo[k], acc);
+#pragma unroll
+              for (int k = 0; k < kMaxM; ++k)
+                if (k < m) acc = fma(sB[i * m + k], us[k], acc);
+            }
             double xb = xb1[i];                                                      // xbar+ = xbar_traj[1]
             double en = acc - xb;                                                    // e+ = x+ - xbar+
             if (!good) {
@@ -506,21 +524,29 @@ int fast_resident(const TzProgram* p, int tpb, int nslot, int h = 1) {
   return by_smem < by_regs ? (by_smem > 0 ? by_smem : 1) : by_regs;
 }
 
-template <class BK, int TPB, int NSLOT, int H = 1>
-int launch_fast_tpb(const TzProgram* p, const SolverParams& sp, const StepArgs& a, const SetEntry* entries, const int32_t* tile_prog,
-                    cudaStream_t st) {
+template <class BK, int TPB, int NSLOT, int H, bool PL>
+int launch_fast_tpb_pl(const TzProgram* p, const SolverParams& sp, const StepArgs& a, const SetEntry* entries, const int32_t* tile_prog,
+                       cudaStream_t st) {
+  constexpr auto kernel = fast_step_kernel<BK, TPB, NSLOT, H, PL>;
   const size_t slot = fast_slot_bytes<BK>(p, H);
   constexpr size_t om_bytes = sizeof(double) * (BK::NW + 3 * (BK::NPAR / 2)) * TPB + sizeof(int) * TPB;      // om + the H > 1 flags
   const size_t smem = (NSLOT > 1 ? NSLOT : 1) * slot + om_bytes;
   static std::atomic<unsigned long long> configured{0ull};
   const size_t smem_max = (NSLOT > 1 ? NSLOT : 1) * (((sizeof(QpProg<BK>) + 15) & ~(size_t)15) + kMaxTabBytes) + om_bytes;
-  if (const int rc = ensure_dynamic_smem(fast_step_kernel<BK, TPB, NSLOT, H>, (int)smem_max, p->device, configured)) return rc;
+  if (const int rc = ensure_dynamic_smem(kernel, (int)smem_max, p->device, configured)) return rc;
   const int64_t nblk = (a.S + TPB - 1) / TPB;
   const int64_t wave = (int64_t)p->num_sms * fast_resident<BK>(p, TPB, NSLOT, H);
   const unsigned grid = (unsigned)(NSLOT == 0 ? (nblk < wave ? nblk : wave) : nblk);
-  TZ_CUDA(launch_kernel(fast_step_kernel<BK, TPB, NSLOT, H>, grid, TPB * H, smem, st, pdl_enabled(a.S),
+  TZ_CUDA(launch_kernel(kernel, grid, TPB * H, smem, st, pdl_enabled(a.S),
                         reinterpret_cast<const QpProg<BK>*>(p->packed_dev), p->aux, sp, a, entries, tile_prog, (int)slot));
   return TZ_OK;
+}
+
+template <class BK, int TPB, int NSLOT, int H = 1>
+int launch_fast_tpb(const TzProgram* p, const SolverParams& sp, const StepArgs& a, const SetEntry* entries, const int32_t* tile_prog,
+                    cudaStream_t st) {
+  return a.AB_true != nullptr ? launch_fast_tpb_pl<BK, TPB, NSLOT, H, true>(p, sp, a, entries, tile_prog, st)
+                              : launch_fast_tpb_pl<BK, TPB, NSLOT, H, false>(p, sp, a, entries, tile_prog, st);
 }
 
 // CTA size by batch size, measured on 148 SMs (profiles/r2_fast_cta_size_sweep.txt; ms per dense 5-dim step):

@@ -511,7 +511,8 @@ static SolverParams to_params(const TzSolverOpts* o) {
 
 // two scenarios per lane in the output phase need 16-byte aligned rows: S, ld even and aligned base pointers
 static int vec2_ok(const StepArgs& a) {
-  const void* ptrs[] = {a.x, a.xbar, a.e, a.noise, a.x_restart, a.cost, a.v, a.xbar_traj, a.ze1, a.u_out, a.xbar0, a.e0, a.x_hist, a.xbar_hist, a.e_hist};
+  const void* ptrs[] = {a.x, a.xbar, a.e, a.noise, a.x_restart, a.cost, a.v, a.xbar_traj, a.ze1, a.u_out, a.xbar0, a.e0, a.x_hist, a.xbar_hist, a.e_hist,
+                        a.AB_true};
   bool ok = (a.S % 2 == 0) && (a.ld % 2 == 0);
   for (const void* q : ptrs) ok = ok && ((reinterpret_cast<uintptr_t>(q) & 15u) == 0);
   ok = ok && ((reinterpret_cast<uintptr_t>(a.status) & 7u) == 0) && ((reinterpret_cast<uintptr_t>(a.iters) & 7u) == 0);
@@ -568,36 +569,81 @@ extern "C" int tz_solve(const TzProgram* prog, const TzSolverOpts* opts, int64_t
   return launch(prog, opts, a, stream);
 }
 
+// The arguments of one closed-loop step.  The plant is either shared (A_true, B_true) or per scenario (AB_true, the _plants entry
+// points); the arguments are checked before any CUDA call.
+static int closed_loop_args(int64_t S, double* x, double* xbar, double* e, const double* noise, const double* x_restart,
+                            const double* A_true, const double* B_true, const double* AB_true, double* cost, double* v,
+                            double* xbar_traj, double* ze1, double* u_out, int32_t* status, int32_t* iters, double* warm,
+                            double* stats, StepArgs* out) {
+  if (AB_true == nullptr)
+    TZ_REQUIRE(S == 0 || (x && xbar && e && A_true && B_true && status), "x, xbar, e, A_true, B_true, status are required");
+  else
+    TZ_REQUIRE(S == 0 || (x && xbar && e && status), "x, xbar, e, AB_true, status are required");
+  StepArgs a{};
+  a.S = S; a.ld = S; a.xbar0 = xbar; a.e0 = e; a.x = x; a.xbar = xbar; a.e = e; a.noise = noise; a.x_restart = x_restart; a.A_true = A_true; a.B_true = B_true;
+  a.cost = cost; a.v = v; a.xbar_traj = xbar_traj; a.ze1 = ze1; a.u_out = u_out; a.status = status; a.iters = iters;
+  a.warm = warm; a.stats = stats;
+  a.AB_true = AB_true;
+  *out = a;
+  return TZ_OK;
+}
+
 extern "C" int tz_closed_loop_step(const TzProgram* prog, const TzSolverOpts* opts, int64_t S, double* x, double* xbar,
                                    double* e, const double* noise, const double* x_restart, const double* A_true,
                                    const double* B_true,
                                    double* cost, double* v, double* xbar_traj, double* ze1, double* u_out,
                                    int32_t* status, int32_t* iters, double* warm, double* stats, void* stream) {
-  TZ_REQUIRE(S == 0 || (x && xbar && e && A_true && B_true && status), "x, xbar, e, A_true, B_true, status are required");
-  StepArgs a{};
-  a.S = S; a.ld = S; a.xbar0 = xbar; a.e0 = e; a.x = x; a.xbar = xbar; a.e = e; a.noise = noise; a.x_restart = x_restart; a.A_true = A_true; a.B_true = B_true;
-  a.cost = cost; a.v = v; a.xbar_traj = xbar_traj; a.ze1 = ze1; a.u_out = u_out; a.status = status; a.iters = iters;
-  a.warm = warm; a.stats = stats;
+  StepArgs a;
+  if (const int rc = closed_loop_args(S, x, xbar, e, noise, x_restart, A_true, B_true, nullptr, cost, v, xbar_traj, ze1, u_out, status,
+                                      iters, warm, stats, &a)) return rc;
+  return launch(prog, opts, a, stream);
+}
+
+extern "C" int tz_closed_loop_step_plants(const TzProgram* prog, const TzSolverOpts* opts, int64_t S, double* x, double* xbar,
+                                          double* e, const double* noise, const double* x_restart, const double* AB_true,
+                                          double* cost, double* v, double* xbar_traj, double* ze1, double* u_out,
+                                          int32_t* status, int32_t* iters, double* warm, double* stats, void* stream) {
+  TZ_REQUIRE(S == 0 || AB_true != nullptr, "AB_true is required");
+  StepArgs a;
+  if (const int rc = closed_loop_args(S, x, xbar, e, noise, x_restart, nullptr, nullptr, AB_true, cost, v, xbar_traj, ze1, u_out,
+                                      status, iters, warm, stats, &a)) return rc;
   return launch(prog, opts, a, stream);
 }
 
 // ---- fused run: K closed-loop steps in one launch (small batches: the launch per step is what the step costs) -----------
+static int closed_loop_run(const TzProgram* prog, const TzSolverOpts* opts, int64_t S, int32_t nsteps, double* x, double* xbar,
+                           double* e, const double* noise, const double* x_restart, const double* A_true, const double* B_true,
+                           const double* AB_true, double* cost, double* v, double* xbar_traj, double* ze1, double* u_out,
+                           double* x_hist, double* xbar_hist, double* e_hist, int32_t* status, int32_t* iters, double* warm,
+                           double* stats, void* stream) {
+  TZ_REQUIRE(prog != nullptr, "null program");
+  TZ_REQUIRE(nsteps >= 1, "nsteps must be >= 1");
+  StepArgs a;
+  if (const int rc = closed_loop_args(S, x, xbar, e, noise, x_restart, A_true, B_true, AB_true, cost, v, xbar_traj, ze1, u_out,
+                                      status, iters, warm, stats, &a)) return rc;
+  TZ_REQUIRE(prog->bucket >= 0 && prog->bucket <= 3, "tz_closed_loop_run serves the register-bucket programs (up to 12 variables)");
+  a.nsteps = nsteps; a.x_hist = x_hist; a.xbar_hist = xbar_hist; a.e_hist = e_hist;
+  // (two-scenarios-per-lane output: vec2_ok wants an even batch, and then every per-step block starts 16-byte aligned too)
+  return launch(prog, opts, a, stream);
+}
+
 extern "C" int tz_closed_loop_run(const TzProgram* prog, const TzSolverOpts* opts, int64_t S, int32_t nsteps, double* x, double* xbar,
                                   double* e, const double* noise, const double* x_restart, const double* A_true,
                                   const double* B_true, double* cost, double* v, double* xbar_traj, double* ze1, double* u_out,
                                   double* x_hist, double* xbar_hist, double* e_hist, int32_t* status, int32_t* iters, double* warm,
                                   double* stats, void* stream) {
-  TZ_REQUIRE(prog != nullptr, "null program");
-  TZ_REQUIRE(nsteps >= 1, "nsteps must be >= 1");
-  TZ_REQUIRE(S == 0 || (x && xbar && e && A_true && B_true && status), "x, xbar, e, A_true, B_true, status are required");
-  TZ_REQUIRE(prog->bucket >= 0 && prog->bucket <= 3, "tz_closed_loop_run serves the register-bucket programs (up to 12 variables)");
-  StepArgs a{};
-  a.S = S; a.ld = S; a.xbar0 = xbar; a.e0 = e; a.x = x; a.xbar = xbar; a.e = e; a.noise = noise; a.x_restart = x_restart; a.A_true = A_true; a.B_true = B_true;
-  a.cost = cost; a.v = v; a.xbar_traj = xbar_traj; a.ze1 = ze1; a.u_out = u_out; a.status = status; a.iters = iters;
-  a.warm = warm; a.stats = stats;
-  a.nsteps = nsteps; a.x_hist = x_hist; a.xbar_hist = xbar_hist; a.e_hist = e_hist;
-  // (two-scenarios-per-lane output: vec2_ok wants an even batch, and then every per-step block starts 16-byte aligned too)
-  return launch(prog, opts, a, stream);
+  return closed_loop_run(prog, opts, S, nsteps, x, xbar, e, noise, x_restart, A_true, B_true, nullptr, cost, v, xbar_traj, ze1, u_out,
+                         x_hist, xbar_hist, e_hist, status, iters, warm, stats, stream);
+}
+
+extern "C" int tz_closed_loop_run_plants(const TzProgram* prog, const TzSolverOpts* opts, int64_t S, int32_t nsteps, double* x,
+                                         double* xbar, double* e, const double* noise, const double* x_restart, const double* AB_true,
+                                         double* cost, double* v, double* xbar_traj, double* ze1, double* u_out, double* x_hist,
+                                         double* xbar_hist, double* e_hist, int32_t* status, int32_t* iters, double* warm,
+                                         double* stats, void* stream) {
+  TZ_REQUIRE(S == 0 || AB_true != nullptr, "AB_true is required");
+  return closed_loop_run(prog, opts, S, nsteps, x, xbar, e, noise, x_restart, nullptr, nullptr, AB_true, cost, v, xbar_traj, ze1,
+                         u_out, x_hist, xbar_hist, e_hist, status, iters, warm, stats, stream);
 }
 
 // ---- tube pattern (packed Ze[1].Z) ------------------------------------------------------------------
@@ -748,11 +794,20 @@ extern "C" int tz_closed_loop_step_set(const TzProgramSet* set, const TzSolverOp
                                        const double* B_true, double* cost, double* v, double* xbar_traj, double* ze1,
                                        double* u_out, int32_t* status, int32_t* iters, double* warm, double* stats,
                                        void* stream) {
-  TZ_REQUIRE(S == 0 || (x && xbar && e && A_true && B_true && status), "x, xbar, e, A_true, B_true, status are required");
-  StepArgs a{};
-  a.S = S; a.ld = S; a.xbar0 = xbar; a.e0 = e; a.x = x; a.xbar = xbar; a.e = e; a.noise = noise; a.x_restart = x_restart; a.A_true = A_true; a.B_true = B_true;
-  a.cost = cost; a.v = v; a.xbar_traj = xbar_traj; a.ze1 = ze1; a.u_out = u_out; a.status = status; a.iters = iters;
-  a.warm = warm; a.stats = stats;
+  StepArgs a;
+  if (const int rc = closed_loop_args(S, x, xbar, e, noise, x_restart, A_true, B_true, nullptr, cost, v, xbar_traj, ze1, u_out, status,
+                                      iters, warm, stats, &a)) return rc;
+  return launch_set(set, opts, a, stream);
+}
+
+extern "C" int tz_closed_loop_step_set_plants(const TzProgramSet* set, const TzSolverOpts* opts, int64_t S, double* x, double* xbar,
+                                              double* e, const double* noise, const double* x_restart, const double* AB_true,
+                                              double* cost, double* v, double* xbar_traj, double* ze1, double* u_out,
+                                              int32_t* status, int32_t* iters, double* warm, double* stats, void* stream) {
+  TZ_REQUIRE(S == 0 || AB_true != nullptr, "AB_true is required");
+  StepArgs a;
+  if (const int rc = closed_loop_args(S, x, xbar, e, noise, x_restart, nullptr, nullptr, AB_true, cost, v, xbar_traj, ze1, u_out,
+                                      status, iters, warm, stats, &a)) return rc;
   return launch_set(set, opts, a, stream);
 }
 

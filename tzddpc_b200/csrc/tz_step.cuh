@@ -78,6 +78,9 @@ struct StepArgs {
   double* x_hist;
   double* xbar_hist;
   double* e_hist;
+  // plant per scenario (tz_closed_loop_*_plants): [A_true B_true] of scenario s, entry (i, k), at AB_true[(i (n+m) + k) ld + s];
+  // NULL: A_true / B_true, shared by the whole batch.  Selects the kernel instantiation (template parameter PL) on the host.
+  const double* AB_true;
 };
 
 // Shared-memory image of one CTA: the program (read-only after staging) and, per warp, the
@@ -122,6 +125,8 @@ __device__ __forceinline__ void vstcs(double* p, Vec<2> v) { __stcg(reinterpret_
 #endif
 __device__ __forceinline__ Vec<1> vfma(double c, Vec<1> x, Vec<1> acc) { return Vec<1>{fma(c, x.a, acc.a)}; }
 __device__ __forceinline__ Vec<2> vfma(double c, Vec<2> x, Vec<2> acc) { return Vec<2>{fma(c, x.a, acc.a), fma(c, x.b, acc.b)}; }
+__device__ __forceinline__ Vec<1> vfma2(Vec<1> c, Vec<1> x, Vec<1> acc) { return Vec<1>{fma(c.a, x.a, acc.a)}; }
+__device__ __forceinline__ Vec<2> vfma2(Vec<2> c, Vec<2> x, Vec<2> acc) { return Vec<2>{fma(c.a, x.a, acc.a), fma(c.b, x.b, acc.b)}; }
 __device__ __forceinline__ Vec<1> vmul(double c, Vec<1> x) { return Vec<1>{c * x.a}; }
 __device__ __forceinline__ Vec<2> vmul(double c, Vec<2> x) { return Vec<2>{c * x.a, c * x.b}; }
 __device__ __forceinline__ Vec<1> vsub(Vec<1> x, Vec<1> y) { return Vec<1>{x.a - y.a}; }
@@ -213,7 +218,7 @@ __device__ __forceinline__ void zero_fill(const Aux& ax, const StepArgs& a, int6
 // Output phase of one output tile (SPO >= 16 consecutive scenarios = TPO solve tiles): lane -> (W consecutive
 // scenarios, slice); one store instruction of the warp covers NSL entries x SPO scenarios = NSL runs of SPO*8 >= 128
 // contiguous bytes (full lines) of the scenario-fastest arrays.
-template <class BK, int W>
+template <class BK, int W, bool PL>
 __device__ __forceinline__ void output_phase(WarpBuf<BK>& wb, const double (*pre)[BK::SPO], const Aux& ax, const StepArgs& a,
                                              const double* __restrict__ tabd, const int* __restrict__ tabi, int64_t tile, int lane,
                                              bool zero_done, bool packed) {
@@ -306,10 +311,19 @@ __device__ __forceinline__ void output_phase(WarpBuf<BK>& wb, const double (*pre
       }
       for (int i = slice; i < n; i += NSL) {
         V acc = a.noise ? vld(&pre[3 * n + i][sc0], vt) : vzero(vt);
-        for (int k = 0; k < n; ++k) acc = vfma(sA[i * n + k], vld(&pre[2 * n + k][sc0], vt), acc);
+        if constexpr (PL) {
+          // this scenario's plant, row i of [A_true B_true]: the same W-scenario vector loads as x (vec2_ok checks AB_true)
+          const double* ab = a.AB_true + (int64_t)i * (n + m) * LD + so;
+          for (int k = 0; k < n; ++k) acc = vfma2(vld(ab + (int64_t)k * LD, vt), vld(&pre[2 * n + k][sc0], vt), acc);
 #pragma unroll
-        for (int k = 0; k < kMaxM; ++k)
-          if (k < m) acc = vfma(sB[i * m + k], us[k], acc);
+          for (int k = 0; k < kMaxM; ++k)
+            if (k < m) acc = vfma2(vld(ab + (int64_t)(n + k) * LD, vt), us[k], acc);
+        } else {
+          for (int k = 0; k < n; ++k) acc = vfma(sA[i * n + k], vld(&pre[2 * n + k][sc0], vt), acc);
+#pragma unroll
+          for (int k = 0; k < kMaxM; ++k)
+            if (k < m) acc = vfma(sB[i * m + k], us[k], acc);
+        }
         const double* row = sXB + (n + i) * NW;                                // xbar+ = xbar_traj[1]
         V xb1 = vzero(vt);
 #pragma unroll
@@ -370,7 +384,7 @@ __device__ __forceinline__ void output_phase(WarpBuf<BK>& wb, const double (*pre
 // tile_first + w + tile_stride, ... below tile_limit of that program's scenarios [0, a.S).
 // step_kernel calls it once (tiles strided over the whole grid); step_kernel_set (data-set axis: many programs in one
 // launch) calls it once per program that intersects the CTA's contiguous range of tiles.
-template <class BK>
+template <class BK, bool PL>
 __device__ __forceinline__ void run_program(unsigned char* smem_raw, const QpProg<BK>* __restrict__ gpg, const Aux& ax,
                                             const SolverParams& sp, const StepArgs& a, const int64_t tile_first,
                                             const int64_t tile_stride, const int64_t tile_limit, const unsigned zseed,
@@ -407,7 +421,7 @@ __device__ __forceinline__ void run_program(unsigned char* smem_raw, const QpPro
     for (int i = tid; i < NCH; i += TPB) cp_async16(dst + 16 * i, src + 16 * i);
     if (tid == 0 && (sizeof(QpProg<BK>) % 16) != 0) cp_async8(dst + 16 * NCH, src + 16 * NCH);
     for (int i = tid; i < ax.n_dbl; i += TPB) cp_async8(tabd + i, ax.tab + i);
-    if (a.x != nullptr) {
+    if (a.x != nullptr && !PL) {
       for (int i = tid; i < n * n; i += TPB) cp_async8(tabd + ax.n_dbl + i, a.A_true + i);
       for (int i = tid; i < n * m; i += TPB) cp_async8(tabd + ax.n_dbl + n * n + i, a.B_true + i);
     }
@@ -708,8 +722,8 @@ __device__ __forceinline__ void run_program(unsigned char* smem_raw, const QpPro
    }     // solve tiles of this output tile
     if (explicit_qp) continue;
     __syncwarp();
-    if (TZ_LIKELY(a.vec2)) output_phase<BK, 2>(wb, pre, ax, a, tabd, tabi, otile, lane, zslot < BK::TPO, sp.tube_packed != 0);
-    else output_phase<BK, 1>(wb, pre, ax, a, tabd, tabi, otile, lane, zslot < BK::TPO, sp.tube_packed != 0);
+    if (TZ_LIKELY(a.vec2)) output_phase<BK, 2, PL>(wb, pre, ax, a, tabd, tabi, otile, lane, zslot < BK::TPO, sp.tube_packed != 0);
+    else output_phase<BK, 1, PL>(wb, pre, ax, a, tabd, tabi, otile, lane, zslot < BK::TPO, sp.tube_packed != 0);
     __syncwarp();     // wb is rewritten by the next tile
   }
   if (a.stats != nullptr && a.x != nullptr) {
@@ -723,8 +737,8 @@ __device__ __forceinline__ void run_program(unsigned char* smem_raw, const QpPro
   }
 }
 
-// Persistent kernel of one program: one wave of CTAs.
-template <class BK>
+// Persistent kernel of one program: one wave of CTAs.  PL: a plant per scenario (StepArgs::AB_true).
+template <class BK, bool PL = false>
 __global__ void __launch_bounds__(BK::TPB, BK::MINB) step_kernel(const QpProg<BK>* __restrict__ gpg, const Aux ax,
                                                                 const SolverParams sp, const StepArgs a) {
   extern __shared__ __align__(16) unsigned char smem_raw[];
@@ -736,8 +750,8 @@ __global__ void __launch_bounds__(BK::TPB, BK::MINB) step_kernel(const QpProg<BK
     const int64_t cnt = *reinterpret_cast<volatile const int32_t*>(a.defer);
     ntiles = cnt < 0 ? 0 : (cnt < ntiles ? cnt : ntiles);          // (a foreign scratch buffer cannot send the kernel out of bounds)
     if ((int64_t)blockIdx.x * BK::WPB < ntiles)
-      run_program<BK>(smem_raw, gpg, ax, sp, a, (int64_t)blockIdx.x * BK::WPB, (int64_t)gridDim.x * BK::WPB, ntiles,
-                      blockIdx.x * BK::WPB);
+      run_program<BK, PL>(smem_raw, gpg, ax, sp, a, (int64_t)blockIdx.x * BK::WPB, (int64_t)gridDim.x * BK::WPB, ntiles,
+                          blockIdx.x * BK::WPB);
     __syncthreads();
     if (threadIdx.x == 0) {
       const int t = atomicAdd(a.defer + 1, 1);
@@ -746,7 +760,7 @@ __global__ void __launch_bounds__(BK::TPB, BK::MINB) step_kernel(const QpProg<BK
     return;
   }
   if (a.nsteps <= 1) {
-    run_program<BK>(smem_raw, gpg, ax, sp, a, (int64_t)blockIdx.x * BK::WPB, (int64_t)gridDim.x * BK::WPB, ntiles,
+    run_program<BK, PL>(smem_raw, gpg, ax, sp, a, (int64_t)blockIdx.x * BK::WPB, (int64_t)gridDim.x * BK::WPB, ntiles,
                     blockIdx.x * BK::WPB);
     return;
   }
@@ -770,8 +784,8 @@ __global__ void __launch_bounds__(BK::TPB, BK::MINB) step_kernel(const QpProg<BK
     if (ak.x_hist) ak.x_hist += (int64_t)k * ax.n * LD;
     if (ak.xbar_hist) ak.xbar_hist += (int64_t)k * ax.n * LD;
     if (ak.e_hist) ak.e_hist += (int64_t)k * ax.n * LD;
-    run_program<BK>(smem_raw, gpg, ax, sp, ak, (int64_t)blockIdx.x * BK::WPB, (int64_t)gridDim.x * BK::WPB, ntiles,
-                    blockIdx.x * BK::WPB + k, k == 0);
+    run_program<BK, PL>(smem_raw, gpg, ax, sp, ak, (int64_t)blockIdx.x * BK::WPB, (int64_t)gridDim.x * BK::WPB, ntiles,
+                        blockIdx.x * BK::WPB + k, k == 0);
     __threadfence_block();
     __syncwarp();
   }
@@ -792,17 +806,19 @@ struct SetEntry {
   int64_t tile_begin;     // number of output tiles of the programs before it
 };
 
+template <bool PL>
 __device__ __forceinline__ StepArgs shift_args(const StepArgs& a, int64_t b, int64_t cnt) {
   StepArgs r = a;
   r.S = cnt;
 #define TZ_SH(f) if (r.f) r.f += b;
   TZ_SH(xbar0) TZ_SH(e0) TZ_SH(x) TZ_SH(xbar) TZ_SH(e) TZ_SH(noise) TZ_SH(x_restart) TZ_SH(cost) TZ_SH(v) TZ_SH(xbar_traj)
   TZ_SH(ze1) TZ_SH(u_out) TZ_SH(status) TZ_SH(iters) TZ_SH(warm)
+  if constexpr (PL) r.AB_true += b;
 #undef TZ_SH
   return r;
 }
 
-template <class BK>
+template <class BK, bool PL = false>
 __global__ void __launch_bounds__(BK::TPB, BK::MINB) step_kernel_set(const SetEntry* __restrict__ entries, const int nprog,
                                                                     const int64_t total_tiles, const Aux ax0,
                                                                     const SolverParams sp, const StepArgs a0) {
@@ -828,13 +844,13 @@ __global__ void __launch_bounds__(BK::TPB, BK::MINB) step_kernel_set(const SetEn
       if (tend <= t) continue;                     // (an empty program)
       Aux ax = ax0;
       ax.tab = en.tab;
-      const StepArgs a = shift_args(a0, en.begin, en.end - en.begin);
+      const StepArgs a = shift_args<PL>(a0, en.begin, en.end - en.begin);
       const bool stage = staged != j;
       if (stage && staged >= 0) __syncthreads();   // every warp is done with the previous program's image
       staged = j;
       // warp w takes tile (t + w) of the round when it belongs to this program (tile_stride: beyond the limit)
-      run_program<BK>(smem_raw, reinterpret_cast<const QpProg<BK>*>(en.pg), ax, sp, a, t - en.tile_begin, BK::WPB,
-                      tend - en.tile_begin, (unsigned)(base % 1024), stage);
+      run_program<BK, PL>(smem_raw, reinterpret_cast<const QpProg<BK>*>(en.pg), ax, sp, a, t - en.tile_begin, BK::WPB,
+                          tend - en.tile_begin, (unsigned)(base % 1024), stage);
       t = tend;
     }
   }
@@ -843,7 +859,7 @@ __global__ void __launch_bounds__(BK::TPB, BK::MINB) step_kernel_set(const SetEn
 // The tiles fast_step_kernel deferred, for a program set: listed tile t (a global 16-scenario tile) belongs to program
 // tile_prog[t]; a CTA takes one listed tile at a time (its first warp solves it), re-staging the program image when the
 // program changes.  Every CTA takes an exit ticket and the last one clears the list, as step_kernel does.
-template <class BK>
+template <class BK, bool PL = false>
 __global__ void __launch_bounds__(BK::TPB, BK::MINB) step_kernel_set_list(const SetEntry* __restrict__ entries,
                                                                          const int32_t* __restrict__ tile_prog, const Aux ax0,
                                                                          const SolverParams sp, const StepArgs a0) {
@@ -861,13 +877,13 @@ __global__ void __launch_bounds__(BK::TPB, BK::MINB) step_kernel_set_list(const 
     const SetEntry en = entries[j];
     Aux ax = ax0;
     ax.tab = en.tab;
-    StepArgs a = shift_args(a0, en.begin, en.end - en.begin);
+    StepArgs a = shift_args<PL>(a0, en.begin, en.end - en.begin);
     a.list_mode = 0;
     const bool stage = staged != j;
     if (stage && staged >= 0) __syncthreads();     // every warp is done with the previous program's image
     staged = j;
     const int64_t tl = t - en.begin / BK::SPO;     // the tile within its program (programs start on whole tiles)
-    run_program<BK>(smem_raw, reinterpret_cast<const QpProg<BK>*>(en.pg), ax, sp, a, tl, BK::WPB, tl + 1, (unsigned)(t % 1024), stage);
+    run_program<BK, PL>(smem_raw, reinterpret_cast<const QpProg<BK>*>(en.pg), ax, sp, a, tl, BK::WPB, tl + 1, (unsigned)(t % 1024), stage);
   }
   __syncthreads();
   if (threadIdx.x == 0) {
@@ -922,48 +938,70 @@ constexpr int kMaxTabBytes = 24 * 1024;
 
 namespace tz {
 
-template <class BK>
-int launch_bucket(const TzProgram* p, const SolverParams& sp, const StepArgs& a, cudaStream_t st) {
+template <class BK, bool PL>
+int launch_bucket_pl(const TzProgram* p, const SolverParams& sp, const StepArgs& a, cudaStream_t st) {
+  constexpr auto kernel = step_kernel<BK, PL>;
   const size_t smem = sizeof(Smem<BK>) + p->smem_tab;
   static std::atomic<unsigned long long> configured{0ull};
-  if (const int rc = ensure_dynamic_smem(step_kernel<BK>, (int)(sizeof(Smem<BK>) + kMaxTabBytes), p->device, configured)) return rc;
+  if (const int rc = ensure_dynamic_smem(kernel, (int)(sizeof(Smem<BK>) + kMaxTabBytes), p->device, configured)) return rc;
   // persistent grid: one wave of CTAs (MINB per SM); every warp loops over tiles of SPW scenarios
   const int64_t ntiles = (a.S + BK::SPO - 1) / BK::SPO;
   const int64_t need = (ntiles + BK::WPB - 1) / BK::WPB;
   // (list mode -- the tiles fast_step_kernel deferred, normally none or a handful: one CTA per SM keeps the empty pass short)
   const int64_t wave = (int64_t)p->num_sms * (a.list_mode ? 1 : BK::MINB);
   const unsigned grid = (unsigned)(need < wave ? need : wave);
-  TZ_CUDA(launch_kernel(step_kernel<BK>, grid, BK::TPB, smem, st, pdl_enabled(a.S), reinterpret_cast<const QpProg<BK>*>(p->packed_dev), p->aux,
+  TZ_CUDA(launch_kernel(kernel, grid, BK::TPB, smem, st, pdl_enabled(a.S), reinterpret_cast<const QpProg<BK>*>(p->packed_dev), p->aux,
                         sp, a));
   return TZ_OK;
 }
 
-// data-set axis: one launch over `nprog` programs (entries on the device); see step_kernel_set
 template <class BK>
-int launch_bucket_set(const TzProgram* p0, const SetEntry* entries_dev, int nprog, int64_t total_tiles, const SolverParams& sp,
-                      const StepArgs& a, cudaStream_t st) {
+int launch_bucket(const TzProgram* p, const SolverParams& sp, const StepArgs& a, cudaStream_t st) {
+  return a.AB_true != nullptr ? launch_bucket_pl<BK, true>(p, sp, a, st) : launch_bucket_pl<BK, false>(p, sp, a, st);
+}
+
+// data-set axis: one launch over `nprog` programs (entries on the device); see step_kernel_set
+template <class BK, bool PL>
+int launch_bucket_set_pl(const TzProgram* p0, const SetEntry* entries_dev, int nprog, int64_t total_tiles, const SolverParams& sp,
+                         const StepArgs& a, cudaStream_t st) {
+  constexpr auto kernel = step_kernel_set<BK, PL>;
   const size_t smem = sizeof(Smem<BK>) + p0->smem_tab;
   static std::atomic<unsigned long long> configured{0ull};
-  if (const int rc = ensure_dynamic_smem(step_kernel_set<BK>, (int)(sizeof(Smem<BK>) + kMaxTabBytes), p0->device, configured)) return rc;
+  if (const int rc = ensure_dynamic_smem(kernel, (int)(sizeof(Smem<BK>) + kMaxTabBytes), p0->device, configured)) return rc;
   static_assert(BK::SPO == TZ_SPO_MIN, "tz_program_set_create counts output tiles of TZ_SPO_MIN scenarios");
   // one wave of CTAs, each with an equal contiguous share of the tiles of all programs (at least one tile per warp)
   const int64_t wave = (int64_t)p0->num_sms * BK::MINB;
   const int64_t need = (total_tiles + BK::WPB - 1) / BK::WPB;
   const unsigned grid = (unsigned)(need < wave ? need : wave);
-  TZ_CUDA(launch_kernel(step_kernel_set<BK>, grid, BK::TPB, smem, st, pdl_enabled(a.S), entries_dev, nprog, total_tiles, p0->aux, sp, a));
+  TZ_CUDA(launch_kernel(kernel, grid, BK::TPB, smem, st, pdl_enabled(a.S), entries_dev, nprog, total_tiles, p0->aux, sp, a));
+  return TZ_OK;
+}
+
+template <class BK>
+int launch_bucket_set(const TzProgram* p0, const SetEntry* entries_dev, int nprog, int64_t total_tiles, const SolverParams& sp,
+                      const StepArgs& a, cudaStream_t st) {
+  return a.AB_true != nullptr ? launch_bucket_set_pl<BK, true>(p0, entries_dev, nprog, total_tiles, sp, a, st)
+                              : launch_bucket_set_pl<BK, false>(p0, entries_dev, nprog, total_tiles, sp, a, st);
+}
+
+template <class BK, bool PL>
+int launch_bucket_set_list_pl(const TzProgram* p0, const SetEntry* entries_dev, const int32_t* tile_prog, const SolverParams& sp,
+                              const StepArgs& a, cudaStream_t st) {
+  constexpr auto kernel = step_kernel_set_list<BK, PL>;
+  const size_t smem = sizeof(Smem<BK>) + p0->smem_tab;
+  static std::atomic<unsigned long long> configured{0ull};
+  if (const int rc = ensure_dynamic_smem(kernel, (int)(sizeof(Smem<BK>) + kMaxTabBytes), p0->device, configured)) return rc;
+  const int64_t ntiles = (a.S + BK::SPO - 1) / BK::SPO;
+  const unsigned grid = (unsigned)(ntiles < p0->num_sms ? ntiles : p0->num_sms);
+  TZ_CUDA(launch_kernel(kernel, grid, BK::TPB, smem, st, pdl_enabled(a.S), entries_dev, tile_prog, p0->aux, sp, a));
   return TZ_OK;
 }
 
 template <class BK>
 int launch_bucket_set_list(const TzProgram* p0, const SetEntry* entries_dev, const int32_t* tile_prog, const SolverParams& sp,
                            const StepArgs& a, cudaStream_t st) {
-  const size_t smem = sizeof(Smem<BK>) + p0->smem_tab;
-  static std::atomic<unsigned long long> configured{0ull};
-  if (const int rc = ensure_dynamic_smem(step_kernel_set_list<BK>, (int)(sizeof(Smem<BK>) + kMaxTabBytes), p0->device, configured)) return rc;
-  const int64_t ntiles = (a.S + BK::SPO - 1) / BK::SPO;
-  const unsigned grid = (unsigned)(ntiles < p0->num_sms ? ntiles : p0->num_sms);
-  TZ_CUDA(launch_kernel(step_kernel_set_list<BK>, grid, BK::TPB, smem, st, pdl_enabled(a.S), entries_dev, tile_prog, p0->aux, sp, a));
-  return TZ_OK;
+  return a.AB_true != nullptr ? launch_bucket_set_list_pl<BK, true>(p0, entries_dev, tile_prog, sp, a, st)
+                              : launch_bucket_set_list_pl<BK, false>(p0, entries_dev, tile_prog, sp, a, st);
 }
 
 }  // namespace tz

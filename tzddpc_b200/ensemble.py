@@ -95,6 +95,7 @@ class _LazyControllers:
             c.verbose = False
             ok = c._adopt_model(self._z, self._AB[d], self._dAB[d], self._dK[d], self._th[d])
             assert ok
+            c._Pinv = None if self._ens._Pinv is None else self._ens._Pinv[d]
             c._program = self._ens._batch.programs[d]
             c.problem_full, c.horizon = c._program, self._h
             c.parameters, c.variables = ("e0", "xbar0"), ("v", "xbar", "Ze")
@@ -109,6 +110,7 @@ class _LazyControllers:
 class TZDDPCEnsemble(object):
     _solve_op = staticmethod(ops.solve_set)
     _step_op = staticmethod(ops.closed_loop_step_set)
+    _step_plants_op = staticmethod(ops.closed_loop_step_set_plants)
 
     def __init__(self, controllers: Sequence[TZDDPC], scenarios_per_dataset: Union[int, Sequence[int]]):
         """controllers: D `TZDDPC` objects on which `build_problem` has been called with the same horizon, cost and
@@ -131,6 +133,11 @@ class TZDDPCEnsemble(object):
         self.dim_x, self.dim_u, self.horizon, self._dims = c0.dim_x, c0.dim_u, c0.horizon, list(c0._dims)
         self.zonotopes = c0.zonotopes
         self.num_scenarios = int(self.begin[-1])
+        # the data sets' models for sample_plants (controllers whose model was adopted from elsewhere carry no pseudo-inverse)
+        pinvs = [getattr(c, "_Pinv", None) for c in controllers]
+        ok = all(p_ is not None and p_.shape == pinvs[0].shape for p_ in pinvs)
+        self._ABd = c0._t(np.stack([c._AB for c in controllers])) if ok else None
+        self._Pinv = torch.stack(pinvs).contiguous() if ok else None
 
     @classmethod
     def from_datasets(cls, datasets: Sequence[Data], zonotopes: SystemZonotopes, horizon: int, build_loss, build_constraints=None,
@@ -207,6 +214,7 @@ class TZDDPCEnsemble(object):
         cbatch = _canonicalise_chunks(canon, D)
         pbatch = _abi_batch(cbatch, K_h, c0.device)
         ens = cls.__new__(cls)
+        ens._ABd, ens._Pinv = AB, Pinv
         ens._init_from_batch(pbatch, datasets, zonotopes, AB_h, dAB_h, dK_h, thetas, int(horizon), scenarios_per_dataset, c0.device)
         ens.theta_info = info
         return ens
@@ -246,6 +254,19 @@ class TZDDPCEnsemble(object):
 
     _t = TZDDPC._t
     solve_batch = TZDDPC.solve_batch
+    _plant_batch = TZDDPC._plant_batch
+    _split_plants = TZDDPC._split_plants
+
+    def sample_plants(self, seed: int, scenario_offset: int = 0):
+        """A plant per scenario, drawn from the model set M_Sigma of the scenario's own data set (as TZDDPC.sample_plants; the
+        draws of scenario s are those of global scenario scenario_offset + s).  Returns CUDA tensors A (S, n, n), B (S, n, m)."""
+        if getattr(self, "_Pinv", None) is None:
+            raise RuntimeError("sample_plants needs every data set's pseudo-inverse pinv([X0; U0]); these controllers carry none "
+                               "(build them with build_zonotopes, or the ensemble with from_datasets)")
+        S = self.num_scenarios
+        ds = torch.as_tensor(self.dataset_of().astype(np.int32), device=self.device)
+        AB = ops.sample_plants(self._ABd, self._Pinv, self._t(self.zonotopes.W.Z), ds, S, int(seed), int(scenario_offset))
+        return self._split_plants(AB)
 
     def simulate(self, A_true, B_true, x0, *args, **kwargs):
         x0 = np.atleast_2d(np.asarray(x0, dtype=np.float64))

@@ -187,6 +187,76 @@ def closed_loop_run(prog: int, steps: int, x: Tensor, xbar: Tensor, e: Tensor, n
     _abi.check(rc, "tz_closed_loop_run")
 
 
+def _chk_plants(AB_true: Tensor, n: int, m: int, S: int) -> None:
+    """AB_true: (n(n+m), S), entry (i, k) of scenario s's [A_true B_true] at [i (n+m) + k, s] -- the layout sample_plants returns."""
+    _chk(AB_true)
+    assert tuple(AB_true.shape) == (n * (n + m), S), f"AB_true: expected ({n * (n + m)}, {S}), got {tuple(AB_true.shape)}"
+
+
+@torch.library.custom_op("tzddpc::closed_loop_step_plants",
+                         mutates_args=("x", "xbar", "e", "cost", "v", "traj", "ze1", "u", "status", "iters", "warm", "stats"),
+                         device_types="cuda")
+def closed_loop_step_plants(prog: int, x: Tensor, xbar: Tensor, e: Tensor, noise: Tensor, x_restart: Optional[Tensor],
+                            AB_true: Tensor, status: Tensor, cost: Optional[Tensor], v: Optional[Tensor], traj: Optional[Tensor],
+                            ze1: Optional[Tensor], u: Optional[Tensor], iters: Optional[Tensor], warm: Optional[Tensor],
+                            stats: Optional[Tensor], opts: List[float]) -> None:
+    """`closed_loop_step` with a plant per scenario: AB_true (n(n+m), S) in place of A_true, B_true."""
+    _chk(x), _chk(xbar), _chk(e), _chk(noise), _chk(status, torch.int32)
+    S = x.shape[1]
+    o = _opts(opts)
+    d = _abi.program_dims(prog)
+    assert x.shape == (d[0], S) and xbar.shape == x.shape and e.shape == x.shape and noise.shape == x.shape, "x, xbar, e, noise: (n, S)"
+    _chk_plants(AB_true, d[0], d[1], S)
+    _chk_step(d, S, x, cost, v, traj, ze1, u, iters, warm if o.warm_start else None, stats, x_restart, status, o.tube_packed)
+    if warm is not None:
+        _chk(warm)
+    with torch.cuda.device(x.device):
+        rc = _abi.lib().tz_closed_loop_step_plants(C.c_void_p(prog), C.byref(o), S, _ptr(x), _ptr(xbar), _ptr(e), _ptr(noise),
+                                                   _ptr(x_restart), _ptr(AB_true), _ptr(cost), _ptr(v), _ptr(traj), _ptr(ze1),
+                                                   _ptr(u), _ptr(status), _ptr(iters), _ptr(warm), _ptr(stats), _stream(x))
+    _abi.check(rc, "tz_closed_loop_step_plants")
+
+
+@torch.library.custom_op("tzddpc::closed_loop_run_plants",
+                         mutates_args=("x", "xbar", "e", "cost", "v", "traj", "ze1", "u", "x_hist", "xbar_hist", "e_hist", "status", "iters", "warm",
+                                       "stats"),
+                         device_types="cuda")
+def closed_loop_run_plants(prog: int, steps: int, x: Tensor, xbar: Tensor, e: Tensor, noise: Tensor, x_restart: Optional[Tensor],
+                           AB_true: Tensor, status: Tensor, cost: Optional[Tensor], v: Optional[Tensor], traj: Optional[Tensor],
+                           ze1: Optional[Tensor], u: Optional[Tensor], x_hist: Optional[Tensor], xbar_hist: Optional[Tensor],
+                           e_hist: Optional[Tensor], iters: Optional[Tensor], warm: Optional[Tensor], stats: Optional[Tensor],
+                           opts: List[float]) -> None:
+    """`closed_loop_run` with a plant per scenario: AB_true (n(n+m), S) in place of A_true, B_true."""
+    _chk(x), _chk(xbar), _chk(e), _chk(noise), _chk(status, torch.int32)
+    S = x.shape[1]
+    o = _opts(opts)
+    d = _abi.program_dims(prog)
+    n, m, nv, nt, nent, n_nz, warm_rows = d
+    assert steps >= 1 and x.shape == (n, S) and xbar.shape == x.shape and e.shape == x.shape, "x, xbar, e: (n, S)"
+    assert noise.shape == (steps, n, S), "noise: (steps, n, S)"
+    assert status.shape == (steps, S), "status: (steps, S)"
+    _chk_plants(AB_true, n, m, S)
+
+    def chk(t, shape, what, dtype=torch.float64):
+        if t is not None:
+            _chk(t, dtype)
+            assert tuple(t.shape) == shape, f"{what}: expected {shape}, got {tuple(t.shape)}"
+    chk(cost, (steps, S), "cost"), chk(iters, (steps, S), "iters", torch.int32), chk(v, (steps, nv, S), "v")
+    chk(traj, (steps, nt, S), "traj"), chk(ze1, (steps, n_nz if o.tube_packed else nent, S), "ze1"), chk(u, (steps, m, S), "u")
+    chk(x_hist, (steps, n, S), "x_hist"), chk(xbar_hist, (steps, n, S), "xbar_hist"), chk(e_hist, (steps, n, S), "e_hist")
+    chk(x_restart, (n, S), "x_restart")
+    if stats is not None:
+        _chk(stats)
+        assert stats.numel() >= steps * _abi.TZ_NSTATS, "stats: needs steps x TZ_NSTATS doubles"
+    _chk_opt(warm if o.warm_start else None, "warm", S, min_rows=warm_rows)
+    with torch.cuda.device(x.device):
+        rc = _abi.lib().tz_closed_loop_run_plants(C.c_void_p(prog), C.byref(o), S, int(steps), _ptr(x), _ptr(xbar), _ptr(e), _ptr(noise),
+                                                  _ptr(x_restart), _ptr(AB_true), _ptr(cost), _ptr(v), _ptr(traj), _ptr(ze1),
+                                                  _ptr(u), _ptr(x_hist), _ptr(xbar_hist), _ptr(e_hist), _ptr(status), _ptr(iters),
+                                                  _ptr(warm), _ptr(stats), _stream(x))
+    _abi.check(rc, "tz_closed_loop_run_plants")
+
+
 @torch.library.custom_op("tzddpc::solve_set", mutates_args=("warm",), device_types="cuda")
 def solve_set(pset: int, dims: List[int], xbar0: Tensor, e0: Tensor, warm: Optional[Tensor], want_tube: bool,
               opts: List[float]) -> Tuple[Tensor, Tensor, Tensor, Tensor, Tensor, Tensor]:
@@ -235,6 +305,30 @@ def closed_loop_step_set(pset: int, x: Tensor, xbar: Tensor, e: Tensor, noise: T
                                                 _ptr(x_restart), _ptr(A_true), _ptr(B_true), _ptr(cost), _ptr(v), _ptr(traj),
                                                 _ptr(ze1), _ptr(u), _ptr(status), _ptr(iters), _ptr(warm), _ptr(stats), _stream(x))
     _abi.check(rc, "tz_closed_loop_step_set")
+
+
+@torch.library.custom_op("tzddpc::closed_loop_step_set_plants",
+                         mutates_args=("x", "xbar", "e", "cost", "v", "traj", "ze1", "u", "status", "iters", "warm", "stats"),
+                         device_types="cuda")
+def closed_loop_step_set_plants(pset: int, x: Tensor, xbar: Tensor, e: Tensor, noise: Tensor, x_restart: Optional[Tensor],
+                                AB_true: Tensor, status: Tensor, cost: Optional[Tensor], v: Optional[Tensor], traj: Optional[Tensor],
+                                ze1: Optional[Tensor], u: Optional[Tensor], iters: Optional[Tensor], warm: Optional[Tensor],
+                                stats: Optional[Tensor], opts: List[float]) -> None:
+    """`closed_loop_step_set` with a plant per scenario: AB_true (n(n+m), S) in place of A_true, B_true."""
+    _chk(x), _chk(xbar), _chk(e), _chk(noise), _chk(status, torch.int32)
+    S = x.shape[1]
+    o = _opts(opts)
+    d = _abi.program_dims(pset, True)
+    assert x.shape == (d[0], S) and xbar.shape == x.shape and e.shape == x.shape and noise.shape == x.shape, "x, xbar, e, noise: (n, S)"
+    _chk_plants(AB_true, d[0], d[1], S)
+    _chk_step(d, S, x, cost, v, traj, ze1, u, iters, warm if o.warm_start else None, stats, x_restart, status, o.tube_packed)
+    if warm is not None:
+        _chk(warm)
+    with torch.cuda.device(x.device):
+        rc = _abi.lib().tz_closed_loop_step_set_plants(C.c_void_p(pset), C.byref(o), S, _ptr(x), _ptr(xbar), _ptr(e), _ptr(noise),
+                                                       _ptr(x_restart), _ptr(AB_true), _ptr(cost), _ptr(v), _ptr(traj), _ptr(ze1),
+                                                       _ptr(u), _ptr(status), _ptr(iters), _ptr(warm), _ptr(stats), _stream(x))
+    _abi.check(rc, "tz_closed_loop_step_set_plants")
 
 
 @torch.library.custom_op("tzddpc::interval_hull", mutates_args=(), device_types="cuda")
@@ -329,16 +423,45 @@ def sample_noise(WZ: Tensor, S: int, vertex: bool, seed: int, scenario_offset: i
 @torch.library.custom_op("tzddpc::generate_trajectories", mutates_args=(), device_types="cuda")
 def generate_trajectories(A: Tensor, B: Tensor, X0Z: Tensor, UZ: Tensor, WZ: Tensor, S: int, T: int, seed: int,
                           scenario_offset: int) -> Tuple[Tensor, Tensor]:
-    """examples/utils.py:6-45 batched over S data sets on the device.  Returns U (S, T, m), X (S, T, n)."""
+    """examples/utils.py:6-45 batched over S data sets on the device.  A (n, n), B (n, m) shared by the data sets, or
+    A (S, n, n), B (S, n, m): data set s from the plant (A[s], B[s]).  Returns U (S, T, m), X (S, T, n)."""
     _chk(A), _chk(B), _chk(X0Z), _chk(UZ), _chk(WZ)
-    n, m = B.shape
+    per = B.dim() == 3
+    n, m = B.shape[-2:]
+    if per:
+        assert tuple(A.shape) == (S, n, n) and B.shape[0] == S, f"A, B: expected ({S}, n, n), ({S}, n, m), got {tuple(A.shape)}, {tuple(B.shape)}"
+    else:
+        assert tuple(A.shape) == (n, n) and B.dim() == 2, f"A, B: expected (n, n), (n, m), got {tuple(A.shape)}, {tuple(B.shape)}"
+    assert X0Z.shape[0] == n and WZ.shape[0] == n and UZ.shape[0] == m, "X0Z, WZ: n rows, UZ: m rows"
     U = torch.empty((S, T, m), dtype=torch.float64, device=A.device)
     X = torch.empty((S, T, n), dtype=torch.float64, device=A.device)
+    fn = _abi.lib().tz_generate_trajectories_plants if per else _abi.lib().tz_generate_trajectories
     with torch.cuda.device(A.device):
-        rc = _abi.lib().tz_generate_trajectories(S, T, n, m, X0Z.shape[1] - 1, UZ.shape[1] - 1, WZ.shape[1] - 1, _ptr(A), _ptr(B),
-                                                 _ptr(X0Z), _ptr(UZ), _ptr(WZ), seed, scenario_offset, _ptr(U), _ptr(X), _stream(A))
-    _abi.check(rc, "tz_generate_trajectories")
+        rc = fn(S, T, n, m, X0Z.shape[1] - 1, UZ.shape[1] - 1, WZ.shape[1] - 1, _ptr(A), _ptr(B),
+                _ptr(X0Z), _ptr(UZ), _ptr(WZ), seed, scenario_offset, _ptr(U), _ptr(X), _stream(A))
+    _abi.check(rc, "tz_generate_trajectories_plants" if per else "tz_generate_trajectories")
     return U, X
+
+
+@torch.library.custom_op("tzddpc::sample_plants", mutates_args=(), device_types="cuda")
+def sample_plants(AB: Tensor, Pinv: Tensor, WZ: Tensor, dataset: Optional[Tensor], S: int, seed: int, scenario_offset: int) -> Tensor:
+    """S plants drawn from the un-reduced model sets M_Sigma = (X1 - M_w) pinv([X0; U0]) of D data sets (tz_sample_plants):
+    AB (D, n, n+m), Pinv (D, T-1, n+m) as `identify` returns them, WZ (n, 1+gW); dataset (S,) int32 -- the data set of every
+    scenario -- or None (data set 0).  Philox stream (seed, scenario_offset + s, purpose 6).  Returns AB_true (n(n+m), S), the
+    layout of the *_plants closed-loop ops."""
+    _chk(AB), _chk(Pinv), _chk(WZ)
+    D, n, nm = AB.shape
+    assert Pinv.dim() == 3 and Pinv.shape[0] == D and Pinv.shape[2] == nm, f"Pinv: expected ({D}, T-1, {nm}), got {tuple(Pinv.shape)}"
+    assert WZ.dim() == 2 and WZ.shape[0] == n, f"WZ: expected ({n}, 1+gW), got {tuple(WZ.shape)}"
+    if dataset is not None:
+        _chk(dataset, torch.int32)
+        assert tuple(dataset.shape) == (S,), f"dataset: expected ({S},), got {tuple(dataset.shape)}"
+    out = torch.empty((n * nm, S), dtype=torch.float64, device=AB.device)
+    with torch.cuda.device(AB.device):
+        rc = _abi.lib().tz_sample_plants(S, D, Pinv.shape[1] + 1, n, nm - n, WZ.shape[1] - 1, _ptr(AB), _ptr(Pinv), _ptr(WZ),
+                                         _ptr(dataset), int(seed), int(scenario_offset), _ptr(out), _stream(AB))
+    _abi.check(rc, "tz_sample_plants")
+    return out
 
 
 @torch.library.custom_op("tzddpc::identify", mutates_args=(), device_types="cuda")

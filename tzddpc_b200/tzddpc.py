@@ -100,6 +100,7 @@ class TZDDPC(object):
     # the launch entry points (TZDDPCEnsemble swaps in the program-set variants)
     _solve_op = staticmethod(ops.solve)
     _step_op = staticmethod(ops.closed_loop_step)
+    _step_plants_op = staticmethod(ops.closed_loop_step_plants)
 
     def __init__(self, data: Data, device: Optional[Union[str, torch.device]] = None):
         """:param data: input/state data, each T x dim (tzddpc/tzddpc.py:20-28)."""
@@ -334,10 +335,43 @@ class TZDDPC(object):
         return (type(self)._step_op is TZDDPC._step_op and steps >= 2 and S < self.FUSED_RUN_MAX_BATCH
                 and str(self._program.bucket)[:2] in ("B0", "B1", "B2", "B3") and hasattr(ops, "closed_loop_run"))
 
+    def _plant_batch(self, A_true, B_true, S: int):
+        """The simulated plant as the closed-loop ops take it: (A, B, None) for one plant (n, n), (n, m) shared by the batch;
+        (None, None, AB_true) for a plant per scenario, A_true (S, n, n) and B_true (S, n, m) as numpy arrays or CUDA tensors,
+        with AB_true the (n(n+m), S) array of the *_plants ops."""
+        ndim = lambda a: a.dim() if isinstance(a, torch.Tensor) else np.ndim(a)          # noqa: E731
+        if ndim(A_true) == 2 and ndim(B_true) == 2:
+            return self._t(A_true), self._t(B_true), None
+        n, m = self.dim_x, self.dim_u
+        dev = lambda a: a.to(self.device, torch.float64) if isinstance(a, torch.Tensor) else self._t(a)     # noqa: E731
+        A, B = dev(A_true), dev(B_true)
+        assert tuple(A.shape) == (S, n, n) and tuple(B.shape) == (S, n, m), \
+            f"A_true, B_true: expected (n, n), (n, m) or ({S}, {n}, {n}), ({S}, {n}, {m}); got {tuple(A.shape)}, {tuple(B.shape)}"
+        return None, None, torch.cat([A, B], dim=2).reshape(S, n * (n + m)).t().contiguous()
+
+    def _split_plants(self, AB_true: torch.Tensor):
+        """(n(n+m), S) -> A (S, n, n), B (S, n, m)"""
+        n, m = self.dim_x, self.dim_u
+        AB = AB_true.t().reshape(-1, n, n + m)
+        return AB[:, :, :n].contiguous(), AB[:, :, n:].contiguous()
+
+    def sample_plants(self, S: int, seed: int, scenario_offset: int = 0):
+        """S plants [A B] drawn uniformly from the generator box of the data-consistent model set
+        M_Sigma = (X1 - M_w) pinv([X0; U0]) (tzddpc/tzddpc.py:81-83; the un-reduced set, whose every member the tube covers),
+        from the Philox stream (seed, scenario_offset + scenario, purpose 6): a scenario's plant does not depend on how the
+        batch is split.  Returns CUDA tensors A (S, n, n), B (S, n, m), for `simulate`."""
+        if getattr(self, "_Pinv", None) is None:
+            raise RuntimeError("sample_plants needs the pseudo-inverse pinv([X0; U0]) of the data: call build_zonotopes first")
+        AB = ops.sample_plants(self._t(self._AB)[None], self._Pinv[None].contiguous(), self._t(self.zonotopes.W.Z), None, int(S),
+                               int(seed), int(scenario_offset))
+        return self._split_plants(AB)
+
     def simulate(self, A_true: np.ndarray, B_true: np.ndarray, x0: np.ndarray, noise=None, keep_tubes: bool = False,
                  options: Optional[SolverOptions] = None, restart: bool = False, steps: Optional[int] = None,
                  seed: Optional[int] = None, vertex_noise: bool = False, scenario_offset: int = 0):
         """Run the closed loop for S scenarios in lock step.
+        A_true (n, n), B_true (n, m): the plant of every scenario; or A_true (S, n, n), B_true (S, n, m) (numpy arrays or CUDA
+        tensors, e.g. from `sample_plants`): scenario s runs on (A_true[s], B_true[s]).
         x0: (S, n); noise: (steps, S, n) array or CUDA tensor (steps, n, S) -- or None with `steps` and `seed`: the noise
         w_t = W.sample() (examples/2.pulley_sim.py:92; a random vertex of W with vertex_noise, examples/1.double_integrator_sim.py:85)
         is then drawn on the device from the Philox stream (seed, scenario_offset + scenario, t), so that a scenario sees the
@@ -363,7 +397,7 @@ class TZDDPC(object):
         f64 = dict(dtype=torch.float64, device=dev)
         x, xbar = self._t(x0.T), self._t(x0.T)
         e = torch.zeros((n, S), **f64)
-        At, Bt = self._t(A_true), self._t(B_true)
+        At, Bt, ABt = self._plant_batch(A_true, B_true, S)
         xs = torch.empty((steps + 1, n, S), **f64)
         xbars = torch.empty_like(xs)
         es = torch.empty_like(xs)
@@ -381,12 +415,20 @@ class TZDDPC(object):
         h = self._program.handle.value
         if isinstance(self, TZDDPC) and self._fused_run_ok(S, steps):      # (TZDDPCEnsemble borrows this method: step loop)
             # small batch: the whole run in ONE launch (tz_closed_loop_run; bit-equal to the step loop below)
-            ops.closed_loop_run(h, steps, x, xbar, e, w.contiguous(), xr, At, Bt, stat, costs, vs, None, tubes if keep_tubes else None,
-                                us, xs[1:], xbars[1:], es[1:], iters, warm, stats, o.pack())
+            if ABt is None:
+                ops.closed_loop_run(h, steps, x, xbar, e, w.contiguous(), xr, At, Bt, stat, costs, vs, None, tubes if keep_tubes else None,
+                                    us, xs[1:], xbars[1:], es[1:], iters, warm, stats, o.pack())
+            else:
+                ops.closed_loop_run_plants(h, steps, x, xbar, e, w.contiguous(), xr, ABt, stat, costs, vs, None,
+                                           tubes if keep_tubes else None, us, xs[1:], xbars[1:], es[1:], iters, warm, stats, o.pack())
         else:
             for t in range(steps):
-                self._step_op(h, x, xbar, e, w[t].contiguous(), xr, At, Bt, stat[t], costs[t], vs[t], None,
-                              tubes[t] if keep_tubes else None, us[t], iters[t], warm, stats[t], o.pack())
+                if ABt is None:
+                    self._step_op(h, x, xbar, e, w[t].contiguous(), xr, At, Bt, stat[t], costs[t], vs[t], None,
+                                  tubes[t] if keep_tubes else None, us[t], iters[t], warm, stats[t], o.pack())
+                else:
+                    self._step_plants_op(h, x, xbar, e, w[t].contiguous(), xr, ABt, stat[t], costs[t], vs[t], None,
+                                         tubes[t] if keep_tubes else None, us[t], iters[t], warm, stats[t], o.pack())
                 xs[t + 1], xbars[t + 1], es[t + 1] = x, xbar, e
         out = {"x": xs.permute(0, 2, 1).cpu().numpy(), "xbar": xbars.permute(0, 2, 1).cpu().numpy(),
                "e": es.permute(0, 2, 1).cpu().numpy(), "u": us.permute(0, 2, 1).cpu().numpy(),
