@@ -309,7 +309,13 @@ int tz_girard_reduce(int64_t S, int32_t n, int32_t g, double order, int32_t metr
  *   Zfinal: S x n x (1+gcap), gfinal[s] generators of the final zonotope (negative: gcap too small, truncated);
  *   hull_lo, hull_hi: S x steps x n interval hull of Z_{k+1} (tzddpc/tzddpc.py:191-197).
  * gcap >= max(g0, floor(n (order-1)) + n).  Column order of the pre-reduction block as pyzonotope's product:
- *   [C_K G | G^K_1 c, G^K_1 G | ... | G^D_1 z .. | G_W]; reduction as tz_girard_reduce. */
+ *   [C_K G | G^K_1 c, G^K_1 G | ... | G^D_1 z .. | G_W]; reduction as tz_girard_reduce.
+ * Two kernels, the same results bit for bit.  Where the pre-reduction block (n x g_pre doubles, g_pre =
+ * (NK+1) gcap + NK + ND + gW) fits in shared memory with the zonotope, the matrices and 9 bytes per column (220 KiB in
+ * all; at n = 5, m = 1 with the 25 + 30 + 1 generators of the stress workload: order <= 31), it is built there once per
+ * step.  Otherwise its entries are recomputed wherever the reduction reads them, and only two zonotopes, the matrices and
+ * the 9 bytes per column take shared memory (order <= 135 at that size).  Beyond that: TZ_EINVAL naming both sizes.
+ * The environment variable TZDDPC_ROLLOUT = resident / recompute (read per call) forces one of the two where it fits. */
 int tz_tube_rollout(int64_t S, int32_t n, int32_t m, int32_t NK, int32_t ND, int32_t gW, int32_t g0, int32_t steps,
                     double order, int32_t metric, const double* CK, const double* GK, const double* GD,
                     int32_t per_scenario_model, const double* Z0, const double* XU, const double* W, int32_t gcap,

@@ -7,6 +7,7 @@
 // contiguous so every global access is a full-line coalesced access, the generator block is
 // staged once in shared memory and never re-read from HBM.
 #include <cstdlib>
+#include <cstring>
 
 #include "tz_common.cuh"
 
@@ -194,16 +195,28 @@ __device__ __forceinline__ int block_exclusive_scan(int v, int* warp_tot, int& t
   return base + inc - v;
 }
 
-// Girard reduction of the generator block G (n x g, row pitch ldg; shared memory, or global memory that stays in L2
-// between the metric pass and the box / compaction passes) of one zonotope by one CTA.
+// Column source of girard_block: G(r, j) is entry r of generator j.  ResidentCols reads a block held in memory;
+// ProductCols (below, tube_rollout_recompute_kernel) evaluates the entry from the factors of the block instead.
+// kCountFromRegisters: loc[d] with a run-time d puts loc[] in 32 bytes of local memory; ProductCols selects the count
+// from registers instead.  ResidentCols keeps the indexed read, so girard_kernel and tube_rollout_kernel compile as before.
+struct ResidentCols {
+  static constexpr bool kCountFromRegisters = false;
+  const double* __restrict__ G;
+  int64_t ldg;
+  __device__ __forceinline__ double operator()(int r, int j) const { return G[(int64_t)r * ldg + j]; }
+};
+
+// Girard reduction of the generator block G (n x g; a ResidentCols block in shared memory, or in global memory that
+// stays in L2 between the metric pass and the box / compaction passes, or a ProductCols block) of one zonotope by one CTA.
+// The metric pass reads every column once, the box pass the reduced ones and the compaction the kept ones.
 // Writes the reduced generators to out[r * ldo + j] (global or shared), zero-pads up to gout_cap, returns the
 // number of generators written (negative: gout_cap too small).  key / flag: g-element scratch in shared memory.
 //   metric per column -> MSB-first radix select of the n_red-th smallest key (stops as soon as a digit bucket is
 //   consumed whole) -> ties by lowest index -> box of the selected columns -> stable compaction of the kept ones.
 // Every thread owns a CONTIGUOUS range of columns, so that ranks (ties, output positions) need one block scan each.
-__device__ int girard_block(int n, int g, double order, int metric, const double* __restrict__ G, int64_t ldg,
-                            unsigned long long* __restrict__ key, unsigned char* __restrict__ flag, double* __restrict__ out,
-                            int64_t ldo, int gout_cap) {
+template <class Cols>
+__device__ int girard_block(int n, int g, double order, int metric, const Cols G, unsigned long long* __restrict__ key,
+                            unsigned char* __restrict__ flag, double* __restrict__ out, int64_t ldo, int gout_cap) {
   __shared__ int hist[256];
   __shared__ int warp_tot[kGirardThreads / 32];
   __shared__ unsigned long long sel_prefix;
@@ -230,8 +243,8 @@ __device__ int girard_block(int n, int g, double order, int metric, const double
 #pragma unroll
       for (int i = 0; i < 8; ++i) {
         const bool in = r0 + i < n;
-        a[i] = in ? fabs(G[(int64_t)(r0 + i) * ldg + ja]) : 0.0;
-        c[i] = (in && hc) ? fabs(G[(int64_t)(r0 + i) * ldg + jc]) : 0.0;
+        a[i] = in ? fabs(G(r0 + i, ja)) : 0.0;
+        c[i] = (in && hc) ? fabs(G(r0 + i, jc)) : 0.0;
       }
 #pragma unroll
       for (int i = 0; i < 8; ++i) {
@@ -321,7 +334,14 @@ __device__ int girard_block(int n, int g, double order, int metric, const double
             if (acc + loc[i] >= rem) { d = i; break; }
             acc += loc[i];
           }
-          const int cnt = loc[d];
+          int cnt;
+          if constexpr (Cols::kCountFromRegisters) {
+            cnt = 0;
+#pragma unroll
+            for (int i = 0; i < 8; ++i) cnt = i == d ? loc[i] : cnt;
+          } else {
+            cnt = loc[d];
+          }
           const unsigned long long digit = (unsigned long long)(lane * 8 + d);
           if (acc + cnt == rem) {
             // the bucket is consumed whole: every key with this prefix and digit is reduced, no need to refine
@@ -367,8 +387,8 @@ __device__ int girard_block(int n, int g, double order, int metric, const double
 #pragma unroll
         for (int i = 0; i < 8; ++i) {
           const bool in = r0 + i < n;
-          a[i] = (fa && in) ? fabs(G[(int64_t)(r0 + i) * ldg + ja]) : 0.0;
-          c[i] = (fc && in) ? fabs(G[(int64_t)(r0 + i) * ldg + jc]) : 0.0;
+          a[i] = (fa && in) ? fabs(G(r0 + i, ja)) : 0.0;
+          c[i] = (fc && in) ? fabs(G(r0 + i, jc)) : 0.0;
         }
 #pragma unroll
         for (int i = 0; i < 8; ++i) { acc[i] += a[i]; acc[i] += c[i]; }
@@ -395,7 +415,7 @@ __device__ int girard_block(int n, int g, double order, int metric, const double
   for (int j = j0; j < j1; ++j) {
     if (flag[j] != 1) continue;
     if (pos < gout_cap)
-      for (int r = 0; r < n; ++r) out[(int64_t)r * ldo + pos] = G[(int64_t)r * ldg + j];
+      for (int r = 0; r < n; ++r) out[(int64_t)r * ldo + pos] = G(r, j);
     ++pos;
   }
   int written = kept;
@@ -430,7 +450,7 @@ __global__ void __launch_bounds__(kGirardThreads) girard_kernel(int n, int g, do
   const double* Zs = Z + s * (int64_t)n * ldz;
   double* Os = Zout + s * (int64_t)n * ldo;
   for (int r = tid; r < n; r += kGirardThreads) Os[(int64_t)r * ldo] = Zs[(int64_t)r * ldz];
-  const int written = girard_block(n, g, order, metric, Zs + 1, ldz, key, flag, Os + 1, ldo, gout_cap);
+  const int written = girard_block(n, g, order, metric, ResidentCols{Zs + 1, ldz}, key, flag, Os + 1, ldo, gout_cap);
   if (tid == 0) gout[s] = written;
 }
 
@@ -673,6 +693,47 @@ __global__ void __launch_bounds__(32) girard_warp_kernel(int n, int g, double or
   if (lane == 0) gout[s] = written;
 }
 
+// Column col of a tube step's pre-reduction block  [C_K G | G^K_1 c, G^K_1 G | ... | G^D_1 z .. G^D_ND z | G_W]
+// (pyzonotope column order, g generators in the current zonotope Zc = [c, G]): the product M v of a staged matrix and a
+// column of Zc or z_k, an FMA chain from 0.0 in q order, or a column of W.  The same map and chain as the loop that fills
+// Gp in tube_rollout_kernel (left as written there, so that kernel compiles as before): tube_rollout_recompute_kernel
+// evaluates an entry wherever girard_block reads the block, and gets the resident kernel's bits.
+struct ProductCols {
+  static constexpr bool kCountFromRegisters = true;
+  const double* MK;             // (NK + 1) x n x n : C_K, G^K_i
+  const double* MD;             // ND x n x p : G^D_i
+  const double* Zc;             // n x (1 + g), row pitch ldc
+  const double* zk;             // p
+  const double* W;              // n x (1 + gW), global
+  int n, p, NK, ND, gW, g, ldc;
+  struct Col {
+    const double* M;            // nullptr: a column of W
+    const double* v;            // the vector multiplied: a column of Zc (stride ldc) or z_k (stride 1)
+    int vstride, len;
+  };
+  __device__ __forceinline__ Col column(int col) const {
+    Col c;
+    if (col < g) { c.M = MK; c.v = Zc + 1 + col; c.vstride = ldc; c.len = n; }
+    else if (col < g + NK * (1 + g)) {
+      const int t = col - g, b = t / (1 + g), j = t - b * (1 + g);
+      c.M = MK + (size_t)(1 + b) * n * n; c.v = Zc + j; c.vstride = ldc; c.len = n;
+    } else if (col < g + NK * (1 + g) + ND) {
+      const int b = col - g - NK * (1 + g);
+      c.M = MD + (size_t)b * n * p; c.v = zk; c.vstride = 1; c.len = p;
+    } else {
+      c.M = nullptr; c.v = W + 1 + (col - g - NK * (1 + g) - ND); c.vstride = 1 + gW; c.len = 0;
+    }
+    return c;
+  }
+  __device__ __forceinline__ double entry(const Col& c, int r) const {
+    if (c.M == nullptr) return c.v[(int64_t)r * c.vstride];
+    double acc = 0.0;
+    for (int q = 0; q < c.len; ++q) acc = fma(c.M[r * c.len + q], c.v[(int64_t)q * c.vstride], acc);
+    return acc;
+  }
+  __device__ __forceinline__ double operator()(int r, int col) const { return entry(column(col), r); }
+};
+
 // ---------------------------------------------------------------------------------------
 // Tube rollout: `steps` reach-set steps of one scenario by one CTA, the zonotope never leaving shared memory:
 //   Z_{k+1} = reduce( M_K (x) Z_k  (+)  M_Delta (x) <z_k, 0>  (+)  W ,  order )          z_k = [xbar_k; v_k]
@@ -751,7 +812,7 @@ __global__ void __launch_bounds__(kGirardThreads) tube_rollout_kernel(
     }
     __syncthreads();
     if (tid < n) Zc[tid * ldc] = cnew[tid];
-    const int written = girard_block(n, gpre, order, metric, Gp, gpre, key, flag, Zc + 1, ldc, gcap);
+    const int written = girard_block(n, gpre, order, metric, ResidentCols{Gp, gpre}, key, flag, Zc + 1, ldc, gcap);
     if (tid == 0) { g_cur = written < 0 ? gcap : written; if (written < 0) overflow = 1; }
     __syncthreads();
     // ---- interval hull of Z_{k+1}: warp r handles row r
@@ -768,6 +829,77 @@ __global__ void __launch_bounds__(kGirardThreads) tube_rollout_kernel(
         }
       }
     }
+    __syncthreads();
+  }
+  for (int i = tid; i < n * ldc; i += kGirardThreads) Zfinal[s * (int64_t)n * ldc + i] = Zc[i];
+  if (tid == 0) gfinal[s] = overflow ? -g_cur : g_cur;       // negative: gcap was too small at some step (truncated)
+}
+
+// The same rollout without the pre-reduction block in shared memory: girard_block reads it through ProductCols, which
+// evaluates each entry from the current zonotope, z_k and the staged matrices (at most n + m FMAs) every time a pass
+// reads it, so the metric pass computes every column once and the box and compaction passes each column once more.
+// Shared memory per scenario is two zonotopes (the reduced one cannot overwrite the one its columns are computed from),
+// the matrices and 9 bytes of key and flag per pre-reduction column: 74 KiB at n = 5, order 40, where the resident
+// kernel needs 272 KiB.  Results are the resident kernel's bit for bit.
+__global__ void __launch_bounds__(kGirardThreads) tube_rollout_recompute_kernel(
+    int n, int m, int NK, int ND, int gW, int g0, int steps, double order, int metric, int gcap, int gpre_cap,
+    const double* __restrict__ CK, const double* __restrict__ GK, const double* __restrict__ GD, int per_scenario,
+    const double* __restrict__ Z0, const double* __restrict__ XU, const double* __restrict__ W,
+    double* __restrict__ Zfinal, int32_t* __restrict__ gfinal, double* __restrict__ hull_lo, double* __restrict__ hull_hi) {
+  extern __shared__ unsigned char smraw[];
+  const int p = n + m, tid = threadIdx.x;
+  const int64_t s = blockIdx.x;
+  const int ldc = 1 + gcap;
+  double* Zc = reinterpret_cast<double*>(smraw);                 // n x (1 + gcap): current zonotope [c, G]
+  double* Zn = Zc + (size_t)n * ldc;                             // n x (1 + gcap): the next one
+  double* MK = Zn + (size_t)n * ldc;                             // (NK + 1) x n x n : C_K, G^K_i
+  double* MD = MK + (size_t)(NK + 1) * n * n;                    // ND x n x p
+  double* zk = MD + (size_t)ND * n * p;                          // p
+  unsigned long long* key = reinterpret_cast<unsigned long long*>(zk + p + (p & 1));
+  unsigned char* flag = reinterpret_cast<unsigned char*>(key + gpre_cap);
+  __shared__ int g_cur, overflow;
+  const double* CKs = CK + (per_scenario ? s * (int64_t)n * n : 0);
+  const double* GKs = GK + (per_scenario ? s * (int64_t)NK * n * n : 0);
+  const double* GDs = GD + (per_scenario ? s * (int64_t)ND * n * p : 0);
+  for (int i = tid; i < n * n; i += kGirardThreads) MK[i] = CKs[i];
+  for (int i = tid; i < NK * n * n; i += kGirardThreads) MK[n * n + i] = GKs[i];
+  for (int i = tid; i < ND * n * p; i += kGirardThreads) MD[i] = GDs[i];
+  for (int i = tid; i < n * ldc; i += kGirardThreads) {        // zero padding: Zfinal is defined for steps = 0 too
+    const int r = i / ldc, j = i - r * ldc;
+    Zc[i] = j <= g0 ? Z0[s * (int64_t)n * (1 + g0) + (int64_t)r * (1 + g0) + j] : 0.0;
+  }
+  if (tid == 0) { g_cur = g0; overflow = 0; }
+  __syncthreads();
+  for (int k = 0; k < steps; ++k) {
+    const int g = g_cur;
+    const int gpre = (NK + 1) * g + NK + ND + gW;
+    if (tid < p) zk[tid] = XU[(s * (int64_t)steps + k) * p + tid];
+    __syncthreads();
+    // ---- centre: C_K c + c_W, as in tube_rollout_kernel
+    if (tid < n) {
+      double acc = W ? W[(int64_t)tid * (1 + gW)] : 0.0;
+      for (int q = 0; q < n; ++q) acc = fma(MK[tid * n + q], Zc[q * ldc], acc);
+      Zn[tid * ldc] = acc;
+    }
+    const ProductCols P{MK, MD, Zc, zk, W, n, p, NK, ND, gW, g, ldc};
+    const int written = girard_block(n, gpre, order, metric, P, key, flag, Zn + 1, ldc, gcap);
+    if (tid == 0) { g_cur = written < 0 ? gcap : written; if (written < 0) overflow = 1; }
+    __syncthreads();
+    // ---- interval hull of Z_{k+1}: warp r handles row r
+    {
+      const int gg = g_cur, lane = tid & 31;
+      for (int r = tid >> 5; r < n; r += kGirardThreads / 32) {
+        double acc = 0.0;
+        for (int j = 1 + lane; j <= gg; j += 32) acc += fabs(Zn[r * ldc + j]);
+        acc = warp_sum(acc);
+        if (lane == 0) {
+          const double c = Zn[r * ldc];
+          hull_lo[(s * (int64_t)steps + k) * n + r] = c - acc;
+          hull_hi[(s * (int64_t)steps + k) * n + r] = c + acc;
+        }
+      }
+    }
+    double* t = Zc; Zc = Zn; Zn = t;
     __syncthreads();
   }
   for (int i = tid; i < n * ldc; i += kGirardThreads) Zfinal[s * (int64_t)n * ldc + i] = Zc[i];
@@ -855,15 +987,33 @@ extern "C" int tz_tube_rollout(int64_t S, int32_t n, int32_t m, int32_t NK, int3
   const int gred = (int)floor((double)n * (order - 1.0)) + n;
   const int gmax = g0 > gred ? g0 : gred;
   TZ_REQUIRE(gcap >= gmax, "gcap must be at least max(g0, floor(n (order - 1)) + n) = %d", gmax);
-  const int64_t gpre_cap = (int64_t)(NK + 1) * gmax + NK + ND + gW;
+  // A step keeps up to floor(n * order) generators unreduced (girard_block reduces only when more than order * n are
+  // non-zero), which rounding can put above gred (order 1.2, n = 5: 6 against 5); a larger gcap then lets them through.
+  const int gkeep = (int)floor((double)n * order);
+  const int gstep = gkeep > gmax ? (gkeep < gcap ? gkeep : gcap) : gmax;      // bound on the generators entering a step
+  const int64_t gpre_cap = (int64_t)(NK + 1) * gstep + NK + ND + gW;
   const int p = n + m;
   const size_t smem = ((size_t)n * (1 + gcap) + (size_t)n * gpre_cap + (size_t)(NK + 1) * n * n + (size_t)ND * n * p + p + n + 2) *
                           sizeof(double) + (size_t)gpre_cap * sizeof(unsigned long long) + (size_t)gpre_cap + 16;
-  TZ_REQUIRE(smem <= 220 * 1024, "tube step (n=%d, %lld generators before reduction) needs %zu bytes of shared memory",
-             n, (long long)gpre_cap, smem);
-  if (smem + 8192 > 48 * 1024)
-    TZ_CUDA(cudaFuncSetAttribute(tube_rollout_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
-  tube_rollout_kernel<<<(unsigned)S, kGirardThreads, smem, (cudaStream_t)stream>>>(
+  // without the n x gpre_cap block, with a second zonotope: about a third of the resident size at n = 5
+  const size_t smem_rc = ((size_t)2 * n * (1 + gcap) + (size_t)(NK + 1) * n * n + (size_t)ND * n * p + p + 1) * sizeof(double) +
+                         (size_t)gpre_cap * sizeof(unsigned long long) + (size_t)gpre_cap + 16;
+  const size_t limit = 220 * 1024;
+  // The resident kernel wherever it fits; TZDDPC_ROLLOUT = resident / recompute (read per launch) forces one of the two,
+  // for comparisons of the two kernels.
+  bool recompute = smem > limit;
+  if (const char* e = getenv("TZDDPC_ROLLOUT")) {
+    TZ_REQUIRE(!strcmp(e, "resident") || !strcmp(e, "recompute"), "TZDDPC_ROLLOUT must be resident or recompute, not '%s'", e);
+    recompute = !strcmp(e, "recompute");
+  }
+  const size_t need = recompute ? smem_rc : smem;
+  TZ_REQUIRE(need <= limit,
+             "tube step (n=%d, %lld generators before reduction) needs %zu bytes of shared memory with the block resident and "
+             "%zu with it recomputed; at most %zu fit",
+             n, (long long)gpre_cap, smem, smem_rc, limit);
+  auto kernel = recompute ? tube_rollout_recompute_kernel : tube_rollout_kernel;
+  if (need + 8192 > 48 * 1024) TZ_CUDA(cudaFuncSetAttribute(kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)need));
+  kernel<<<(unsigned)S, kGirardThreads, need, (cudaStream_t)stream>>>(
       n, m, NK, ND, gW, g0, steps, order, metric, gcap, (int)gpre_cap, CK, GK, GD, per_scenario_model, Z0, XU, gW ? W : nullptr,
       Zfinal, gfinal, hull_lo, hull_hi);
   TZ_CUDA(cudaGetLastError());

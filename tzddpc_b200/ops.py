@@ -385,7 +385,11 @@ def tube_rollout(CK: Tensor, GK: Tensor, GD: Tensor, Z0: Tensor, XU: Tensor, W: 
     """Z_{k+1} = reduce(M_K x Z_k + M_Delta x <[xbar_k; v_k], 0> + W, order) for k < steps, zonotope resident in shared
     memory (tzddpc/tzddpc.py:175-186,205 + Zonotope.reduce).  CK: (n, n) or (S, n, n); GK: (NK, n, n) or (S, NK, n, n);
     GD: (ND, n, n+m) or (S, ND, n, n+m); Z0: (S, n, 1+g0); XU: (S, steps, n+m); W: (n, 1+gW).
-    Returns Zfinal (S, n, 1+gcap), gfinal (S), hull_lo, hull_hi (S, steps, n)."""
+    Returns Zfinal (S, n, 1+gcap), gfinal (S), hull_lo, hull_hi (S, steps, n).
+    Where the pre-reduction generator block fits in shared memory (order <= 31 for the 5-dim stress system) it is built
+    there every step (tube_rollout_kernel); beyond that its entries are recomputed wherever the Girard reduction reads them
+    (tube_rollout_recompute_kernel, order <= 135 there), with the same results bit for bit.  Larger orders raise, naming the
+    bytes both kernels need.  TZDDPC_ROLLOUT=resident / recompute forces one kernel where it fits (include/tzddpc.h)."""
     _chk(CK), _chk(GK), _chk(GD), _chk(Z0), _chk(XU)
     per = CK.dim() == 3
     S, n, ld0 = Z0.shape
