@@ -200,6 +200,18 @@ static int create_bucket(const TzProgramDesc& d, TzProgram* p, int id, HostImage
   return TZ_OK;
 }
 
+// the generic warp-per-scenario path (tz_big.cu) for a program no register-resident bucket serves; no packed image, no tables
+static int use_big_path(const TzProgramDesc* d, TzProgram* p) {
+  p->bucket = 4;
+  p->NZ = d->nz; p->NC = d->nc; p->G = 32;
+  p->nz = d->nz; p->nc = d->nc; p->n = d->n; p->m = d->m; p->N = d->horizon; p->nv = d->nv; p->g1 = d->g1; p->npar = d->npar;
+  for (int e = 0; e < d->n * (1 + d->g1); ++e)
+    if (d->ze1_ptr[e + 1] > d->ze1_ptr[e]) p->tube_ent.push_back(e);
+  p->aux.n_nz = (int)p->tube_ent.size();
+  p->aux.n = d->n; p->aux.m = d->m; p->aux.N = d->horizon; p->aux.nv = d->nv; p->aux.g1 = d->g1;
+  return TZ_OK;
+}
+
 // Everything of tz_program_create that runs on the host: validation, bucket choice, packing, tables.  No CUDA call.
 static int build_program_host(const TzProgramDesc* d, TzProgram* p, HostImage& img) {
   TZ_REQUIRE(d != nullptr, "null argument");
@@ -217,17 +229,7 @@ static int build_program_host(const TzProgramDesc* d, TzProgram* p, HostImage& i
   if (rc == TZ_ERANGE && fits<BK>(*d)) rc = create_bucket<BK>(*d, p, ID, img);
   TZ_TRY(B0, 0) TZ_TRY(B1, 1) TZ_TRY(B2, 2) TZ_TRY(B3, 3)
 #undef TZ_TRY
-  if (rc == TZ_ERANGE && big_fits(*d)) {
-    // larger than every register-resident bucket: the generic warp-per-scenario path (tz_big.cu); no packed image, no tables
-    p->bucket = 4;
-    p->NZ = d->nz; p->NC = d->nc; p->G = 32;
-    p->nz = d->nz; p->nc = d->nc; p->n = d->n; p->m = d->m; p->N = d->horizon; p->nv = d->nv; p->g1 = d->g1; p->npar = d->npar;
-    for (int e = 0; e < d->n * (1 + d->g1); ++e)
-      if (d->ze1_ptr[e + 1] > d->ze1_ptr[e]) p->tube_ent.push_back(e);
-    p->aux.n_nz = (int)p->tube_ent.size();
-    p->aux.n = d->n; p->aux.m = d->m; p->aux.N = d->horizon; p->aux.nv = d->nv; p->aux.g1 = d->g1;
-    return TZ_OK;
-  }
+  if (rc == TZ_ERANGE && big_fits(*d)) return use_big_path(d, p);
   if (rc != TZ_OK) {
     if (rc == TZ_ERANGE) {
       const RowClasses c = classify(*d, nullptr);
@@ -311,6 +313,13 @@ static int build_program_host(const TzProgramDesc* d, TzProgram* p, HostImage& i
   const size_t ndbl = o_zrow + (size_t)n_zrow_half, nint = ent.size() + idx.size();
   const size_t smem_tab = (ndbl + (size_t)n * n + (size_t)n * d->m) * sizeof(double) + nint * sizeof(int32_t);
   if (smem_tab > kMaxTabBytes) {
+    // the rows fit a register bucket but its tables do not fit the shared memory staged for them (n = 8, m = 4, N = 2 needs
+    // 25 KiB): the generic path serves the program instead
+    if (big_fits(*d)) {
+      *p = TzProgram();
+      img = HostImage();
+      return use_big_path(d, p);
+    }
     return fail(TZ_ERANGE, "program tables need %zu bytes of shared memory (limit %d)", smem_tab, kMaxTabBytes);
   }
   std::vector<unsigned char>& host = img.aux;
