@@ -643,12 +643,14 @@ int big_launch(const BigProgram* bp, const SolverParams& sp, const StepArgs& a, 
   g.a = a;
   const size_t smem = (size_t)kBigWarps * bp->dev.scratch_doubles * sizeof(double);
   if (smem > 200 * 1024) return fail(TZ_ERANGE, "program needs %zu bytes of shared memory per CTA", smem);
-  auto kernel = a.AB_true != nullptr ? big_step_kernel<true> : big_step_kernel<false>;
-  TZ_CUDA(cudaFuncSetAttribute(kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
   const unsigned grid = (unsigned)((a.S + kBigWarps - 1) / kBigWarps);
-  kernel<<<grid, kBigWarps * 32, smem, st>>>(g);
-  TZ_CUDA(cudaGetLastError());
-  return TZ_OK;
+  return with_plant(a, [&](auto pl) {
+    constexpr auto kernel = big_step_kernel<decltype(pl)::value>;
+    TZ_CUDA(cudaFuncSetAttribute(kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
+    kernel<<<grid, kBigWarps * 32, smem, st>>>(g);
+    TZ_CUDA(cudaGetLastError());
+    return TZ_OK;
+  });
 }
 
 }  // namespace tz

@@ -524,29 +524,24 @@ int fast_resident(const TzProgram* p, int tpb, int nslot, int h = 1) {
   return by_smem < by_regs ? (by_smem > 0 ? by_smem : 1) : by_regs;
 }
 
-template <class BK, int TPB, int NSLOT, int H, bool PL>
-int launch_fast_tpb_pl(const TzProgram* p, const SolverParams& sp, const StepArgs& a, const SetEntry* entries, const int32_t* tile_prog,
-                       cudaStream_t st) {
-  constexpr auto kernel = fast_step_kernel<BK, TPB, NSLOT, H, PL>;
-  const size_t slot = fast_slot_bytes<BK>(p, H);
-  constexpr size_t om_bytes = sizeof(double) * (BK::NW + 3 * (BK::NPAR / 2)) * TPB + sizeof(int) * TPB;      // om + the H > 1 flags
-  const size_t smem = (NSLOT > 1 ? NSLOT : 1) * slot + om_bytes;
-  static std::atomic<unsigned long long> configured{0ull};
-  const size_t smem_max = (NSLOT > 1 ? NSLOT : 1) * (((sizeof(QpProg<BK>) + 15) & ~(size_t)15) + kMaxTabBytes) + om_bytes;
-  if (const int rc = ensure_dynamic_smem(kernel, (int)smem_max, p->device, configured)) return rc;
-  const int64_t nblk = (a.S + TPB - 1) / TPB;
-  const int64_t wave = (int64_t)p->num_sms * fast_resident<BK>(p, TPB, NSLOT, H);
-  const unsigned grid = (unsigned)(NSLOT == 0 ? (nblk < wave ? nblk : wave) : nblk);
-  TZ_CUDA(launch_kernel(kernel, grid, TPB * H, smem, st, pdl_enabled(a.S),
-                        reinterpret_cast<const QpProg<BK>*>(p->packed_dev), p->aux, sp, a, entries, tile_prog, (int)slot));
-  return TZ_OK;
-}
-
 template <class BK, int TPB, int NSLOT, int H = 1>
 int launch_fast_tpb(const TzProgram* p, const SolverParams& sp, const StepArgs& a, const SetEntry* entries, const int32_t* tile_prog,
                     cudaStream_t st) {
-  return a.AB_true != nullptr ? launch_fast_tpb_pl<BK, TPB, NSLOT, H, true>(p, sp, a, entries, tile_prog, st)
-                              : launch_fast_tpb_pl<BK, TPB, NSLOT, H, false>(p, sp, a, entries, tile_prog, st);
+  const size_t slot = fast_slot_bytes<BK>(p, H);
+  constexpr size_t om_bytes = sizeof(double) * (BK::NW + 3 * (BK::NPAR / 2)) * TPB + sizeof(int) * TPB;      // om + the H > 1 flags
+  const size_t smem = (NSLOT > 1 ? NSLOT : 1) * slot + om_bytes;
+  const size_t smem_max = (NSLOT > 1 ? NSLOT : 1) * (((sizeof(QpProg<BK>) + 15) & ~(size_t)15) + kMaxTabBytes) + om_bytes;
+  const int64_t nblk = (a.S + TPB - 1) / TPB;
+  const int64_t wave = (int64_t)p->num_sms * fast_resident<BK>(p, TPB, NSLOT, H);
+  const unsigned grid = (unsigned)(NSLOT == 0 ? (nblk < wave ? nblk : wave) : nblk);
+  return with_plant(a, [&](auto pl) {
+    constexpr auto kernel = fast_step_kernel<BK, TPB, NSLOT, H, decltype(pl)::value>;
+    static std::atomic<unsigned long long> configured{0ull};
+    if (const int rc = ensure_dynamic_smem(kernel, (int)smem_max, p->device, configured)) return rc;
+    TZ_CUDA(launch_kernel(kernel, grid, TPB * H, smem, st, pdl_enabled(a.S),
+                          reinterpret_cast<const QpProg<BK>*>(p->packed_dev), p->aux, sp, a, entries, tile_prog, (int)slot));
+    return TZ_OK;
+  });
 }
 
 // CTA size by batch size, measured on 148 SMs (profiles/r2_fast_cta_size_sweep.txt; ms per dense 5-dim step):

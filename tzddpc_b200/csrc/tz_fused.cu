@@ -528,31 +528,43 @@ static int vec2_ok(const StepArgs& a) {
   return ok ? 1 : 0;
 }
 
+// What a launch over one program and over a program set (program p the first of the set) do before choosing the kernels:
+// the device check, the output layout (vec2), the solver options, and whether to take the hot path.  The hot path is the hint
+// mode of the two-variable programs: fast_step_kernel (one thread per scenario, closed-form certificate) decides every
+// scenario whose hint still holds; the 16-scenario tiles it defers are listed in the warm-start scratch (rows 2G: counters,
+// 2G + 1: list) and solved by the step kernel right behind it.  Batches below kHotMinBatch scenarios and fused runs stay on
+// the step kernel: one launch instead of two -- batch-1 latency.
+static int prepare(const TzProgram* p, const char* what, const TzSolverOpts* o, const StepArgs& a_in, StepArgs* a, SolverParams* sp,
+                   bool* hot) {
+  int cur = -1;
+  TZ_CUDA(cudaGetDevice(&cur));
+  TZ_REQUIRE(cur == p->device, "the %s was created on CUDA device %d, the current device is %d", what, p->device, cur);
+  *a = a_in;
+  a->vec2 = vec2_ok(*a);
+  *sp = to_params(o);
+  TZ_REQUIRE(sp->max_iter >= 1 && sp->rho > 0 && sp->rho_act > 0 && sp->rho_inact > 0 && sp->alpha > 0 && sp->alpha < 2,
+             "bad solver options");
+  *hot = p->bucket == 0 && sp->hot && sp->warm == 2 && a->warm != nullptr && a->q_in == nullptr && a->S >= kHotMinBatch &&
+         a->nsteps <= 1;
+  if (*hot) {
+    a->defer = reinterpret_cast<int32_t*>(a->warm + (int64_t)(2 * B0::G) * a->ld);
+    a->defer_list = reinterpret_cast<int32_t*>(a->warm + (int64_t)(2 * B0::G + 1) * a->ld);
+    a->list_mode = 0;
+  }
+  return TZ_OK;
+}
+
 static int launch(const TzProgram* p, const TzSolverOpts* o, const StepArgs& a_in, void* stream) {
   TZ_REQUIRE(p != nullptr, "null program");
   TZ_REQUIRE(a_in.S >= 0, "negative batch");
   if (a_in.S == 0) return TZ_OK;
-  {
-    int cur = -1;
-    TZ_CUDA(cudaGetDevice(&cur));
-    TZ_REQUIRE(cur == p->device, "the program was created on CUDA device %d, the current device is %d", p->device, cur);
-  }
-  StepArgs a = a_in;
-  a.vec2 = vec2_ok(a);
-  const SolverParams sp = to_params(o);
-  TZ_REQUIRE(sp.max_iter >= 1 && sp.rho > 0 && sp.rho_act > 0 && sp.rho_inact > 0 && sp.alpha > 0 && sp.alpha < 2,
-             "bad solver options");
+  StepArgs a;
+  SolverParams sp;
+  bool hot;
+  if (const int rc = prepare(p, "program", o, a_in, &a, &sp, &hot)) return rc;
   cudaStream_t st = reinterpret_cast<cudaStream_t>(stream);
-  // (batches below kHotMinBatch scenarios stay on the ADMM kernel: one launch instead of two -- batch-1 latency)
-  if (p->bucket == 0 && sp.hot && sp.warm == 2 && a.warm != nullptr && a.q_in == nullptr && a.S >= kHotMinBatch && a.nsteps <= 1) {
-    // hint mode of the two-variable programs: fast_step_kernel (one thread per scenario, closed-form certificate) decides
-    // every scenario whose hint still holds; the 16-scenario tiles it defers are listed in the warm-start scratch (rows
-    // 2G: counters, 2G + 1: list) and solved by step_kernel right behind it
-    a.defer = reinterpret_cast<int32_t*>(a.warm + (int64_t)(2 * B0::G) * a.ld);
-    a.defer_list = reinterpret_cast<int32_t*>(a.warm + (int64_t)(2 * B0::G + 1) * a.ld);
-    a.list_mode = 0;
-    const int rc = launch_fast<B0>(p, sp, a, st);
-    if (rc != TZ_OK) return rc;
+  if (hot) {
+    if (const int rc = launch_fast<B0>(p, sp, a, st)) return rc;
     a.list_mode = 1;
     return launch_bucket<B0>(p, sp, a, st);
   }
@@ -578,16 +590,16 @@ extern "C" int tz_solve(const TzProgram* prog, const TzSolverOpts* opts, int64_t
   return launch(prog, opts, a, stream);
 }
 
-// The arguments of one closed-loop step.  The plant is either shared (A_true, B_true) or per scenario (AB_true, the _plants entry
-// points); the arguments are checked before any CUDA call.
-static int closed_loop_args(int64_t S, double* x, double* xbar, double* e, const double* noise, const double* x_restart,
+// The arguments of one closed-loop step.  The plant is either shared (A_true, B_true) or, with `plants` (the _plants entry
+// points), per scenario (AB_true); the arguments are checked before any CUDA call.
+static int closed_loop_args(int64_t S, double* x, double* xbar, double* e, const double* noise, const double* x_restart, bool plants,
                             const double* A_true, const double* B_true, const double* AB_true, double* cost, double* v,
                             double* xbar_traj, double* ze1, double* u_out, int32_t* status, int32_t* iters, double* warm,
                             double* stats, StepArgs* out) {
-  if (AB_true == nullptr)
-    TZ_REQUIRE(S == 0 || (x && xbar && e && A_true && B_true && status), "x, xbar, e, A_true, B_true, status are required");
+  if (plants)
+    TZ_REQUIRE(S == 0 || (x && xbar && e && AB_true && status), "x, xbar, e, AB_true, status are required");
   else
-    TZ_REQUIRE(S == 0 || (x && xbar && e && status), "x, xbar, e, AB_true, status are required");
+    TZ_REQUIRE(S == 0 || (x && xbar && e && A_true && B_true && status), "x, xbar, e, A_true, B_true, status are required");
   StepArgs a{};
   a.S = S; a.ld = S; a.xbar0 = xbar; a.e0 = e; a.x = x; a.xbar = xbar; a.e = e; a.noise = noise; a.x_restart = x_restart; a.A_true = A_true; a.B_true = B_true;
   a.cost = cost; a.v = v; a.xbar_traj = xbar_traj; a.ze1 = ze1; a.u_out = u_out; a.status = status; a.iters = iters;
@@ -603,8 +615,8 @@ extern "C" int tz_closed_loop_step(const TzProgram* prog, const TzSolverOpts* op
                                    double* cost, double* v, double* xbar_traj, double* ze1, double* u_out,
                                    int32_t* status, int32_t* iters, double* warm, double* stats, void* stream) {
   StepArgs a;
-  if (const int rc = closed_loop_args(S, x, xbar, e, noise, x_restart, A_true, B_true, nullptr, cost, v, xbar_traj, ze1, u_out, status,
-                                      iters, warm, stats, &a)) return rc;
+  if (const int rc = closed_loop_args(S, x, xbar, e, noise, x_restart, false, A_true, B_true, nullptr, cost, v, xbar_traj, ze1, u_out,
+                                      status, iters, warm, stats, &a)) return rc;
   return launch(prog, opts, a, stream);
 }
 
@@ -612,23 +624,22 @@ extern "C" int tz_closed_loop_step_plants(const TzProgram* prog, const TzSolverO
                                           double* e, const double* noise, const double* x_restart, const double* AB_true,
                                           double* cost, double* v, double* xbar_traj, double* ze1, double* u_out,
                                           int32_t* status, int32_t* iters, double* warm, double* stats, void* stream) {
-  TZ_REQUIRE(S == 0 || AB_true != nullptr, "AB_true is required");
   StepArgs a;
-  if (const int rc = closed_loop_args(S, x, xbar, e, noise, x_restart, nullptr, nullptr, AB_true, cost, v, xbar_traj, ze1, u_out,
+  if (const int rc = closed_loop_args(S, x, xbar, e, noise, x_restart, true, nullptr, nullptr, AB_true, cost, v, xbar_traj, ze1, u_out,
                                       status, iters, warm, stats, &a)) return rc;
   return launch(prog, opts, a, stream);
 }
 
 // ---- fused run: K closed-loop steps in one launch (small batches: the launch per step is what the step costs) -----------
 static int closed_loop_run(const TzProgram* prog, const TzSolverOpts* opts, int64_t S, int32_t nsteps, double* x, double* xbar,
-                           double* e, const double* noise, const double* x_restart, const double* A_true, const double* B_true,
-                           const double* AB_true, double* cost, double* v, double* xbar_traj, double* ze1, double* u_out,
+                           double* e, const double* noise, const double* x_restart, bool plants, const double* A_true,
+                           const double* B_true, const double* AB_true, double* cost, double* v, double* xbar_traj, double* ze1, double* u_out,
                            double* x_hist, double* xbar_hist, double* e_hist, int32_t* status, int32_t* iters, double* warm,
                            double* stats, void* stream) {
   TZ_REQUIRE(prog != nullptr, "null program");
   TZ_REQUIRE(nsteps >= 1, "nsteps must be >= 1");
   StepArgs a;
-  if (const int rc = closed_loop_args(S, x, xbar, e, noise, x_restart, A_true, B_true, AB_true, cost, v, xbar_traj, ze1, u_out,
+  if (const int rc = closed_loop_args(S, x, xbar, e, noise, x_restart, plants, A_true, B_true, AB_true, cost, v, xbar_traj, ze1, u_out,
                                       status, iters, warm, stats, &a)) return rc;
   TZ_REQUIRE(prog->bucket >= 0 && prog->bucket <= 3, "tz_closed_loop_run serves the register-bucket programs (up to 12 variables)");
   a.nsteps = nsteps; a.x_hist = x_hist; a.xbar_hist = xbar_hist; a.e_hist = e_hist;
@@ -641,8 +652,8 @@ extern "C" int tz_closed_loop_run(const TzProgram* prog, const TzSolverOpts* opt
                                   const double* B_true, double* cost, double* v, double* xbar_traj, double* ze1, double* u_out,
                                   double* x_hist, double* xbar_hist, double* e_hist, int32_t* status, int32_t* iters, double* warm,
                                   double* stats, void* stream) {
-  return closed_loop_run(prog, opts, S, nsteps, x, xbar, e, noise, x_restart, A_true, B_true, nullptr, cost, v, xbar_traj, ze1, u_out,
-                         x_hist, xbar_hist, e_hist, status, iters, warm, stats, stream);
+  return closed_loop_run(prog, opts, S, nsteps, x, xbar, e, noise, x_restart, false, A_true, B_true, nullptr, cost, v, xbar_traj, ze1,
+                         u_out, x_hist, xbar_hist, e_hist, status, iters, warm, stats, stream);
 }
 
 extern "C" int tz_closed_loop_run_plants(const TzProgram* prog, const TzSolverOpts* opts, int64_t S, int32_t nsteps, double* x,
@@ -650,8 +661,7 @@ extern "C" int tz_closed_loop_run_plants(const TzProgram* prog, const TzSolverOp
                                          double* cost, double* v, double* xbar_traj, double* ze1, double* u_out, double* x_hist,
                                          double* xbar_hist, double* e_hist, int32_t* status, int32_t* iters, double* warm,
                                          double* stats, void* stream) {
-  TZ_REQUIRE(S == 0 || AB_true != nullptr, "AB_true is required");
-  return closed_loop_run(prog, opts, S, nsteps, x, xbar, e, noise, x_restart, nullptr, nullptr, AB_true, cost, v, xbar_traj, ze1,
+  return closed_loop_run(prog, opts, S, nsteps, x, xbar, e, noise, x_restart, true, nullptr, nullptr, AB_true, cost, v, xbar_traj, ze1,
                          u_out, x_hist, xbar_hist, e_hist, status, iters, warm, stats, stream);
 }
 
@@ -752,30 +762,20 @@ static int launch_set(const TzProgramSet* s, const TzSolverOpts* o, const StepAr
   TZ_REQUIRE(a_in.S == s->begin.back(), "batch of %lld scenarios, the set was created for %lld", (long long)a_in.S,
              (long long)s->begin.back());
   if (a_in.S == 0) return TZ_OK;
-  StepArgs a = a_in;
-  a.vec2 = vec2_ok(a);             // (every program starts on a multiple of 16 scenarios: alignment carries over)
-  for (size_t j = 0; j + 1 < s->begin.size(); ++j)
-    if ((s->begin[j + 1] - s->begin[j]) % 2 != 0) a.vec2 = 0;
-  const SolverParams sp = to_params(o);
-  TZ_REQUIRE(sp.max_iter >= 1 && sp.rho > 0 && sp.rho_act > 0 && sp.rho_inact > 0 && sp.alpha > 0 && sp.alpha < 2,
-             "bad solver options");
   const TzProgram* p0 = s->progs[0];
   const int np = (int)s->progs.size();
   if (np == 1) return launch(p0, o, a_in, stream);       // one program: exactly step_kernel (tiles strided over the grid)
+  StepArgs a;
+  SolverParams sp;
+  bool hot;
+  if (const int rc = prepare(p0, "program set", o, a_in, &a, &sp, &hot)) return rc;
+  for (size_t j = 0; j + 1 < s->begin.size(); ++j)       // (every program starts on a multiple of 16 scenarios: alignment carries over)
+    if ((s->begin[j + 1] - s->begin[j]) % 2 != 0) a.vec2 = 0;
   cudaStream_t st = reinterpret_cast<cudaStream_t>(stream);
-  {
-    int cur = -1;
-    TZ_CUDA(cudaGetDevice(&cur));
-    TZ_REQUIRE(cur == p0->device, "the program set was created on CUDA device %d, the current device is %d", p0->device, cur);
-  }
-  if (p0->bucket == 0 && sp.hot && sp.warm == 2 && a.warm != nullptr && a.q_in == nullptr && a.S >= kHotMinBatch) {
+  if (hot) {
     // the hot path over a set: fast_step_kernel looks the program of every 16-scenario tile up, the tiles it defers are
-    // solved by step_kernel_set_list (same scratch layout as the single-program path)
-    a.defer = reinterpret_cast<int32_t*>(a.warm + (int64_t)(2 * B0::G) * a.ld);
-    a.defer_list = reinterpret_cast<int32_t*>(a.warm + (int64_t)(2 * B0::G + 1) * a.ld);
-    a.list_mode = 0;
-    const int rc = launch_fast_set<B0>(p0, sp, a, s->entries_dev, s->tile_prog_dev, s->block, st);
-    if (rc != TZ_OK) return rc;
+    // solved by step_kernel_set_list
+    if (const int rc = launch_fast_set<B0>(p0, sp, a, s->entries_dev, s->tile_prog_dev, s->block, st)) return rc;
     a.list_mode = 1;
     return launch_bucket_set_list<B0>(p0, s->entries_dev, s->tile_prog_dev, sp, a, st);
   }
@@ -804,8 +804,8 @@ extern "C" int tz_closed_loop_step_set(const TzProgramSet* set, const TzSolverOp
                                        double* u_out, int32_t* status, int32_t* iters, double* warm, double* stats,
                                        void* stream) {
   StepArgs a;
-  if (const int rc = closed_loop_args(S, x, xbar, e, noise, x_restart, A_true, B_true, nullptr, cost, v, xbar_traj, ze1, u_out, status,
-                                      iters, warm, stats, &a)) return rc;
+  if (const int rc = closed_loop_args(S, x, xbar, e, noise, x_restart, false, A_true, B_true, nullptr, cost, v, xbar_traj, ze1, u_out,
+                                      status, iters, warm, stats, &a)) return rc;
   return launch_set(set, opts, a, stream);
 }
 
@@ -813,9 +813,8 @@ extern "C" int tz_closed_loop_step_set_plants(const TzProgramSet* set, const TzS
                                               double* e, const double* noise, const double* x_restart, const double* AB_true,
                                               double* cost, double* v, double* xbar_traj, double* ze1, double* u_out,
                                               int32_t* status, int32_t* iters, double* warm, double* stats, void* stream) {
-  TZ_REQUIRE(S == 0 || AB_true != nullptr, "AB_true is required");
   StepArgs a;
-  if (const int rc = closed_loop_args(S, x, xbar, e, noise, x_restart, nullptr, nullptr, AB_true, cost, v, xbar_traj, ze1, u_out,
+  if (const int rc = closed_loop_args(S, x, xbar, e, noise, x_restart, true, nullptr, nullptr, AB_true, cost, v, xbar_traj, ze1, u_out,
                                       status, iters, warm, stats, &a)) return rc;
   return launch_set(set, opts, a, stream);
 }
@@ -868,7 +867,6 @@ StreamPool* stream_pool(int device, int nchunks) {
 }
 
 struct HostStep {
-  int resident = 0;          // 1: tz_closed_loop_run_host (state stays on the device between calls)
   int upload_state = 1;      // copy x, xbar, e (and x_restart) up before the step
   int download_state = 1;    // copy xbar and e down after the step (x always comes down)
   double *x, *xbar, *e;
@@ -928,7 +926,7 @@ int closed_loop_host(const TzProgram* p, const TzSolverOpts* opts, int64_t S, co
       err = h2d(dx, hs.x, n, s0, cnt, st);
       if (err == cudaSuccess) err = h2d(dxb, hs.xbar, n, s0, cnt, st);
       if (err == cudaSuccess) err = h2d(de, hs.e, n, s0, cnt, st);
-      if (err == cudaSuccess && hs.resident && hs.x_restart) err = h2d(dxr, hs.x_restart, n, s0, cnt, st);
+      if (err == cudaSuccess && hs.x_restart) err = h2d(dxr, hs.x_restart, n, s0, cnt, st);
     }
     if (err == cudaSuccess) err = h2d(dw, hs.noise, n, s0, cnt, st);
     if (err != cudaSuccess) break;
@@ -936,7 +934,7 @@ int closed_loop_host(const TzProgram* p, const TzSolverOpts* opts, int64_t S, co
     StepArgs a{};
     a.S = cnt; a.ld = S;
     a.xbar0 = dxb + s0; a.e0 = de + s0; a.x = dx + s0; a.xbar = dxb + s0; a.e = de + s0; a.noise = dw + s0;
-    a.x_restart = (hs.resident && hs.x_restart) ? dxr + s0 : nullptr;
+    a.x_restart = hs.x_restart ? dxr + s0 : nullptr;
     a.A_true = dA; a.B_true = dB;
     a.cost = hs.cost ? dcost + s0 : nullptr;
     a.v = hs.v ? dv + s0 : nullptr;
@@ -976,12 +974,9 @@ extern "C" int tz_closed_loop_step_host(const TzProgram* prog, const TzSolverOpt
   TZ_REQUIRE(prog && dev_scratch, "null argument");
   TZ_REQUIRE(S == 0 || (x_host && xbar_host && e_host && noise_host && A_true_host && B_true_host && status_host),
              "x, xbar, e, noise, A_true, B_true, status are required");
-  if (S == 0) return TZ_OK;
-  HostStep hs;
-  hs.x = x_host; hs.xbar = xbar_host; hs.e = e_host; hs.x_restart = nullptr; hs.noise = noise_host; hs.A_true = A_true_host;
-  hs.B_true = B_true_host; hs.cost = cost_host; hs.v = v_host; hs.traj = xbar_traj_host; hs.ze1 = ze1_host; hs.u = nullptr;
-  hs.status = status_host;
-  return closed_loop_host(prog, opts, S, hs, dev_scratch, nchunks);
+  // the resident path with the state uploaded before and downloaded after the step (flags 3), no restart state, no u
+  return tz_closed_loop_run_host(prog, opts, S, 3, x_host, xbar_host, e_host, nullptr, noise_host, A_true_host, B_true_host, cost_host,
+                                 v_host, xbar_traj_host, ze1_host, nullptr, status_host, dev_scratch, nchunks);
 }
 
 extern "C" int tz_closed_loop_run_host(const TzProgram* prog, const TzSolverOpts* opts, int64_t S, int32_t flags, double* x_host,
@@ -997,7 +992,7 @@ extern "C" int tz_closed_loop_run_host(const TzProgram* prog, const TzSolverOpts
   TZ_REQUIRE(S == 0 || !down || (xbar_host && e_host), "flags & 2 (download xbar and e): xbar, e are required");
   if (S == 0) return TZ_OK;
   HostStep hs;
-  hs.resident = 1; hs.upload_state = up ? 1 : 0; hs.download_state = down ? 1 : 0;
+  hs.upload_state = up ? 1 : 0; hs.download_state = down ? 1 : 0;
   hs.x = x_host; hs.xbar = xbar_host; hs.e = e_host; hs.x_restart = x_restart_host; hs.noise = noise_host; hs.A_true = A_true_host;
   hs.B_true = B_true_host; hs.cost = cost_host; hs.v = v_host; hs.traj = xbar_traj_host; hs.ze1 = ze1_host; hs.u = u_host;
   hs.status = status_host;

@@ -5,19 +5,15 @@
 #include <atomic>
 #include <cmath>
 #include <new>
+#include <type_traits>
 #include <vector>
 
 #include "tz_admm.cuh"
 #include "tz_cert2.cuh"
 #include "tz_param.cuh"
 
-#ifndef TZ_NO_HINTS
 #define TZ_LIKELY(x) __builtin_expect(!!(x), 1)
 #define TZ_UNLIKELY(x) __builtin_expect(!!(x), 0)
-#else
-#define TZ_LIKELY(x) (x)
-#define TZ_UNLIKELY(x) (x)
-#endif
 
 namespace tz {
 
@@ -83,6 +79,13 @@ struct StepArgs {
   const double* AB_true;
 };
 
+// Calls f(std::true_type) for a plant per scenario (a.AB_true != NULL), f(std::false_type) for a plant shared by the batch:
+// the launchers pick the kernel instantiation of template parameter PL = decltype(arg)::value.
+template <class F>
+int with_plant(const StepArgs& a, F&& f) {
+  return a.AB_true != nullptr ? f(std::true_type{}) : f(std::false_type{});
+}
+
 // Shared-memory image of one CTA: the program (read-only after staging) and, per warp, the
 // exchange buffers between the solve phase and the output phase of a tile.
 template <class BK>
@@ -110,19 +113,8 @@ __device__ __forceinline__ Vec<1> vld(const double* p, Vec<1>*) { return Vec<1>{
 __device__ __forceinline__ Vec<2> vld(const double* p, Vec<2>*) { const double2 t = *reinterpret_cast<const double2*>(p); return Vec<2>{t.x, t.y}; }
 __device__ __forceinline__ void vst(double* p, Vec<1> v) { *p = v.a; }
 __device__ __forceinline__ void vst(double* p, Vec<2> v) { *reinterpret_cast<double2*>(p) = make_double2(v.a, v.b); }
-#ifndef TZ_ZST
-#define TZ_ZST 1
-#endif
-#if TZ_ZST == 0
-__device__ __forceinline__ void vstcs(double* p, Vec<1> v) { *p = v.a; }
-__device__ __forceinline__ void vstcs(double* p, Vec<2> v) { *reinterpret_cast<double2*>(p) = make_double2(v.a, v.b); }
-#elif TZ_ZST == 1
 __device__ __forceinline__ void vstcs(double* p, Vec<1> v) { __stcs(p, v.a); }
 __device__ __forceinline__ void vstcs(double* p, Vec<2> v) { __stcs(reinterpret_cast<double2*>(p), make_double2(v.a, v.b)); }
-#else
-__device__ __forceinline__ void vstcs(double* p, Vec<1> v) { __stcg(p, v.a); }
-__device__ __forceinline__ void vstcs(double* p, Vec<2> v) { __stcg(reinterpret_cast<double2*>(p), make_double2(v.a, v.b)); }
-#endif
 __device__ __forceinline__ Vec<1> vfma(double c, Vec<1> x, Vec<1> acc) { return Vec<1>{fma(c, x.a, acc.a)}; }
 __device__ __forceinline__ Vec<2> vfma(double c, Vec<2> x, Vec<2> acc) { return Vec<2>{fma(c, x.a, acc.a), fma(c, x.b, acc.b)}; }
 __device__ __forceinline__ Vec<1> vfma2(Vec<1> c, Vec<1> x, Vec<1> acc) { return Vec<1>{fma(c.a, x.a, acc.a)}; }
@@ -893,10 +885,7 @@ __global__ void __launch_bounds__(BK::TPB, BK::MINB) step_kernel_set_list(const 
 }
 
 // ---- compiled buckets: <NZ, N2, NU, NL, G, NPAR, NAG, NCHK, MINB> -------------------------------
-#ifndef TZ_B0_MINB
-#define TZ_B0_MINB 3
-#endif
-using B0 = Bucket<2, 1, 3, 3, 4, 10, 2, 12, TZ_B0_MINB>;      // N = 2, m = 1, n <= 5: the three shipped examples (28 row slots)
+using B0 = Bucket<2, 1, 3, 3, 4, 10, 2, 12, 3>;      // N = 2, m = 1, n <= 5: the three shipped examples (28 row slots)
 using B1 = Bucket<4, 2, 4, 4, 8, 16, 8, 32, 3>;      // generic small   (80 row slots)
 using B2 = Bucket<8, 3, 5, 5, 8, 16, 24, 32, 2>;     // generic medium  (104 row slots, N = 3..4)
 using B3 = Bucket<12, 1, 4, 4, 8, 16, 24, 32, 1>;    // large           (72 row slots, nz <= 12: N = 5 of the complexity sweep)
@@ -938,70 +927,52 @@ constexpr int kMaxTabBytes = 24 * 1024;
 
 namespace tz {
 
-template <class BK, bool PL>
-int launch_bucket_pl(const TzProgram* p, const SolverParams& sp, const StepArgs& a, cudaStream_t st) {
-  constexpr auto kernel = step_kernel<BK, PL>;
-  const size_t smem = sizeof(Smem<BK>) + p->smem_tab;
+// Launches `kernel`, a step kernel of bucket BK, on `grid` CTAs with the shared memory of the bucket and program p's tables.
+// The kernel is a template argument so that every kernel keeps its own cache of the devices its attribute is set on.
+template <class BK, auto kernel, class... Args>
+int launch_step(const TzProgram* p, unsigned grid, cudaStream_t st, int64_t S, Args... args) {
   static std::atomic<unsigned long long> configured{0ull};
   if (const int rc = ensure_dynamic_smem(kernel, (int)(sizeof(Smem<BK>) + kMaxTabBytes), p->device, configured)) return rc;
+  TZ_CUDA(launch_kernel(kernel, grid, BK::TPB, sizeof(Smem<BK>) + p->smem_tab, st, pdl_enabled(S), args...));
+  return TZ_OK;
+}
+
+template <class BK>
+int launch_bucket(const TzProgram* p, const SolverParams& sp, const StepArgs& a, cudaStream_t st) {
   // persistent grid: one wave of CTAs (MINB per SM); every warp loops over tiles of SPW scenarios
   const int64_t ntiles = (a.S + BK::SPO - 1) / BK::SPO;
   const int64_t need = (ntiles + BK::WPB - 1) / BK::WPB;
   // (list mode -- the tiles fast_step_kernel deferred, normally none or a handful: one CTA per SM keeps the empty pass short)
   const int64_t wave = (int64_t)p->num_sms * (a.list_mode ? 1 : BK::MINB);
   const unsigned grid = (unsigned)(need < wave ? need : wave);
-  TZ_CUDA(launch_kernel(kernel, grid, BK::TPB, smem, st, pdl_enabled(a.S), reinterpret_cast<const QpProg<BK>*>(p->packed_dev), p->aux,
-                        sp, a));
-  return TZ_OK;
-}
-
-template <class BK>
-int launch_bucket(const TzProgram* p, const SolverParams& sp, const StepArgs& a, cudaStream_t st) {
-  return a.AB_true != nullptr ? launch_bucket_pl<BK, true>(p, sp, a, st) : launch_bucket_pl<BK, false>(p, sp, a, st);
+  return with_plant(a, [&](auto pl) {
+    return launch_step<BK, step_kernel<BK, decltype(pl)::value>>(p, grid, st, a.S, reinterpret_cast<const QpProg<BK>*>(p->packed_dev),
+                                                                 p->aux, sp, a);
+  });
 }
 
 // data-set axis: one launch over `nprog` programs (entries on the device); see step_kernel_set
-template <class BK, bool PL>
-int launch_bucket_set_pl(const TzProgram* p0, const SetEntry* entries_dev, int nprog, int64_t total_tiles, const SolverParams& sp,
-                         const StepArgs& a, cudaStream_t st) {
-  constexpr auto kernel = step_kernel_set<BK, PL>;
-  const size_t smem = sizeof(Smem<BK>) + p0->smem_tab;
-  static std::atomic<unsigned long long> configured{0ull};
-  if (const int rc = ensure_dynamic_smem(kernel, (int)(sizeof(Smem<BK>) + kMaxTabBytes), p0->device, configured)) return rc;
+template <class BK>
+int launch_bucket_set(const TzProgram* p0, const SetEntry* entries_dev, int nprog, int64_t total_tiles, const SolverParams& sp,
+                      const StepArgs& a, cudaStream_t st) {
   static_assert(BK::SPO == TZ_SPO_MIN, "tz_program_set_create counts output tiles of TZ_SPO_MIN scenarios");
   // one wave of CTAs, each with an equal contiguous share of the tiles of all programs (at least one tile per warp)
   const int64_t wave = (int64_t)p0->num_sms * BK::MINB;
   const int64_t need = (total_tiles + BK::WPB - 1) / BK::WPB;
   const unsigned grid = (unsigned)(need < wave ? need : wave);
-  TZ_CUDA(launch_kernel(kernel, grid, BK::TPB, smem, st, pdl_enabled(a.S), entries_dev, nprog, total_tiles, p0->aux, sp, a));
-  return TZ_OK;
-}
-
-template <class BK>
-int launch_bucket_set(const TzProgram* p0, const SetEntry* entries_dev, int nprog, int64_t total_tiles, const SolverParams& sp,
-                      const StepArgs& a, cudaStream_t st) {
-  return a.AB_true != nullptr ? launch_bucket_set_pl<BK, true>(p0, entries_dev, nprog, total_tiles, sp, a, st)
-                              : launch_bucket_set_pl<BK, false>(p0, entries_dev, nprog, total_tiles, sp, a, st);
-}
-
-template <class BK, bool PL>
-int launch_bucket_set_list_pl(const TzProgram* p0, const SetEntry* entries_dev, const int32_t* tile_prog, const SolverParams& sp,
-                              const StepArgs& a, cudaStream_t st) {
-  constexpr auto kernel = step_kernel_set_list<BK, PL>;
-  const size_t smem = sizeof(Smem<BK>) + p0->smem_tab;
-  static std::atomic<unsigned long long> configured{0ull};
-  if (const int rc = ensure_dynamic_smem(kernel, (int)(sizeof(Smem<BK>) + kMaxTabBytes), p0->device, configured)) return rc;
-  const int64_t ntiles = (a.S + BK::SPO - 1) / BK::SPO;
-  const unsigned grid = (unsigned)(ntiles < p0->num_sms ? ntiles : p0->num_sms);
-  TZ_CUDA(launch_kernel(kernel, grid, BK::TPB, smem, st, pdl_enabled(a.S), entries_dev, tile_prog, p0->aux, sp, a));
-  return TZ_OK;
+  return with_plant(a, [&](auto pl) {
+    return launch_step<BK, step_kernel_set<BK, decltype(pl)::value>>(p0, grid, st, a.S, entries_dev, nprog, total_tiles, p0->aux, sp, a);
+  });
 }
 
 template <class BK>
 int launch_bucket_set_list(const TzProgram* p0, const SetEntry* entries_dev, const int32_t* tile_prog, const SolverParams& sp,
                            const StepArgs& a, cudaStream_t st) {
-  return a.AB_true != nullptr ? launch_bucket_set_list_pl<BK, true>(p0, entries_dev, tile_prog, sp, a, st)
-                              : launch_bucket_set_list_pl<BK, false>(p0, entries_dev, tile_prog, sp, a, st);
+  const int64_t ntiles = (a.S + BK::SPO - 1) / BK::SPO;
+  const unsigned grid = (unsigned)(ntiles < p0->num_sms ? ntiles : p0->num_sms);
+  return with_plant(a, [&](auto pl) {
+    return launch_step<BK, step_kernel_set_list<BK, decltype(pl)::value>>(p0, grid, st, a.S, entries_dev, tile_prog, p0->aux, sp, a);
+  });
 }
 
 }  // namespace tz

@@ -955,9 +955,7 @@ extern "C" int tz_girard_reduce(int64_t S, int32_t n, int32_t g, double order, i
      // would idle.  Measured on B200 (n = 5, order 3, scratch/girard_small.py): warp kernel 2.0x / 1.7x / 1.1x faster at
      // g = 32 / 64 / 113, CTA kernel 1.2x / 1.6x / 1.7x faster at g = 256 / 512 / 1024 and 1.4-2.6x at the stress sizes.
     const size_t smw = (size_t)g * 9 + 256 * sizeof(int) + 32;
-    static const char* force = getenv("TZ_GIRARD_KERNEL");                 // "cta" / "warp": A/B switch for the benches
-    const bool want_warp = force ? (force[0] == 'w') : (g <= 128);
-    if (want_warp && n <= 8 && smw <= 56 * 1024) {
+    if (g <= 128 && n <= 8 && smw <= 56 * 1024) {
       if (smw + 8192 > 48 * 1024)
         TZ_CUDA(cudaFuncSetAttribute(girard_warp_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smw));
       girard_warp_kernel<<<(unsigned)S, 32, smw, (cudaStream_t)stream>>>(n, g, order, metric, Z, gout_cap, Zout, gout);

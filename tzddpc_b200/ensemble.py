@@ -109,8 +109,7 @@ class _LazyControllers:
 
 class TZDDPCEnsemble(object):
     _solve_op = staticmethod(ops.solve_set)
-    _step_op = staticmethod(ops.closed_loop_step_set)
-    _step_plants_op = staticmethod(ops.closed_loop_step_set_plants)
+    _step_ops = (ops.closed_loop_step_set, ops.closed_loop_step_set_plants)
 
     def __init__(self, controllers: Sequence[TZDDPC], scenarios_per_dataset: Union[int, Sequence[int]]):
         """controllers: D `TZDDPC` objects on which `build_problem` has been called with the same horizon, cost and

@@ -61,39 +61,95 @@ def _chk(t: Tensor, dtype=torch.float64):
     assert t.is_cuda and t.dtype == dtype and t.is_contiguous(), "expected a contiguous CUDA tensor of " + str(dtype)
 
 
-def _chk_opt(t: Optional[Tensor], what: str, S: int, rows: Optional[int] = None, min_rows: Optional[int] = None,
-             dtype=torch.float64):
+def _chk_opt(t: Optional[Tensor], what: str, shape: Tuple[int, ...], dtype=torch.float64):
     """Optional output / scratch tensors are handed to the kernels as raw pointers: the C ABI cannot know their sizes, so a
-    wrong dtype, a non-contiguous slice or too few rows would corrupt device memory silently."""
-    if t is None:
-        return
-    _chk(t, dtype)
-    shape = tuple(t.shape)
-    if rows is None and min_rows is None:
-        assert shape == (S,), f"{what}: expected shape ({S},), got {shape}"
-        return
-    assert len(shape) == 2 and shape[1] == S, f"{what}: expected (rows, {S}), got {shape}"
-    if rows is not None:
-        assert shape[0] == rows, f"{what}: expected {rows} rows, got {shape[0]}"
-    if min_rows is not None:
-        assert shape[0] >= min_rows, f"{what}: needs at least {min_rows} rows, got {shape[0]}"
+    wrong dtype, a non-contiguous slice or a wrong shape would corrupt device memory silently."""
+    if t is not None:
+        _chk(t, dtype)
+        assert tuple(t.shape) == shape, f"{what}: expected {shape}, got {tuple(t.shape)}"
 
 
-def _chk_step(prog_dims, S, x, cost, v, traj, ze1, u, iters, warm, stats, x_restart, status, packed):
-    n, m, nv, nt, nent, n_nz, warm_rows = prog_dims
-    for t, nm in ((x_restart, "x_restart"),):
-        _chk_opt(t, nm, S, rows=n)
-    _chk_opt(cost, "cost", S)
-    _chk_opt(status, "status", S, dtype=torch.int32)
-    _chk_opt(iters, "iters", S, dtype=torch.int32)
-    _chk_opt(v, "v", S, rows=nv)
-    _chk_opt(traj, "traj", S, rows=nt)
-    _chk_opt(ze1, "ze1", S, rows=(n_nz if packed else nent))
-    _chk_opt(u, "u", S, rows=m)
-    _chk_opt(warm, "warm", S, min_rows=warm_rows)
+def _chk_warm(warm: Optional[Tensor], S: int, min_rows: int, used: bool):
+    """The warm-start scratch (rows >= min_rows, S): a CUDA float64 tensor whenever given, its shape checked where `used`."""
+    if warm is None:
+        return
+    _chk(warm)
+    if used:
+        shape = tuple(warm.shape)
+        assert len(shape) == 2 and shape[1] == S, f"warm: expected (rows, {S}), got {shape}"
+        assert shape[0] >= min_rows, f"warm: needs at least {min_rows} rows, got {shape[0]}"
+
+
+def _solve(handle: int, is_set: bool, dims: List[int], xbar0: Tensor, e0: Tensor, warm: Optional[Tensor], want_tube: bool,
+           opts: List[float]) -> Tuple[Tensor, Tensor, Tensor, Tensor, Tensor, Tensor]:
+    """The body of `solve` (a program) and `solve_set` (a program set, `is_set`)."""
+    _chk(xbar0), _chk(e0)
+    n, nv, nt, nent = dims
+    S = xbar0.shape[1]
+    dev = xbar0.device
+    cost = torch.empty(S, dtype=torch.float64, device=dev)
+    v = torch.empty((nv, S), dtype=torch.float64, device=dev)
+    traj = torch.empty((nt, S), dtype=torch.float64, device=dev)
+    ze1 = torch.empty((nent if want_tube else 0, S), dtype=torch.float64, device=dev)
+    status = torch.empty(S, dtype=torch.int32, device=dev)
+    iters = torch.empty(S, dtype=torch.int32, device=dev)
+    o = _opts(opts)
+    d = _abi.program_dims(handle, is_set)
+    assert xbar0.shape == (d[0], S) and e0.shape == xbar0.shape, "xbar0, e0: (n, S)"
+    assert (nv, nt) == (d[2], d[3]) and (not want_tube or nent == (d[5] if o.tube_packed else d[4])), "dims do not match the program"
+    _chk_warm(warm, S, d[6], bool(o.warm_start))
+    name = "tz_solve_set" if is_set else "tz_solve"
+    with torch.cuda.device(dev):
+        rc = getattr(_abi.lib(), name)(C.c_void_p(handle), C.byref(o), S, _ptr(xbar0), _ptr(e0), _ptr(cost), _ptr(v), _ptr(traj),
+                                       _ptr(ze1) if want_tube else None, _ptr(status), _ptr(iters), _ptr(warm), _stream(xbar0))
+    _abi.check(rc, name)
+    return cost, v, traj, ze1, status, iters
+
+
+def _closed_loop(handle: int, is_set: bool, steps: Optional[int], x: Tensor, xbar: Tensor, e: Tensor, noise: Tensor,
+                 x_restart: Optional[Tensor], plant: Tuple[Tensor, ...], status: Tensor, cost: Optional[Tensor], v: Optional[Tensor],
+                 traj: Optional[Tensor], ze1: Optional[Tensor], u: Optional[Tensor], hist: Tuple[Optional[Tensor], ...],
+                 iters: Optional[Tensor], warm: Optional[Tensor], stats: Optional[Tensor], opts: List[float]) -> None:
+    """The body of every closed-loop op.  `handle` is a program, or a program set with `is_set` (tz_closed_loop_*_set).
+    `steps` None is one step (tz_closed_loop_step*); otherwise a fused run of `steps` steps (tz_closed_loop_run*), whose noise
+    and per-step outputs carry a leading `steps` dimension and `hist` = (x_hist, xbar_hist, e_hist).  `plant` is
+    (A_true, B_true), shared by the batch, or (AB_true,), a plant per scenario (tz_closed_loop_*_plants)."""
+    _chk(x), _chk(xbar), _chk(e), _chk(noise), _chk(status, torch.int32)
+    S = x.shape[1]
+    o = _opts(opts)
+    n, m, nv, nt, nent, n_nz, warm_rows = _abi.program_dims(handle, is_set)
+    if len(plant) == 2:
+        _chk(plant[0]), _chk(plant[1])
+    else:
+        _chk(plant[0])
+        assert tuple(plant[0].shape) == (n * (n + m), S), f"AB_true: expected ({n * (n + m)}, {S}), got {tuple(plant[0].shape)}"
+    lead, k, per = ((), 1, "") if steps is None else ((steps,), steps, "steps, ")
+    assert k >= 1 and x.shape == (n, S) and xbar.shape == x.shape and e.shape == x.shape, "x, xbar, e: (n, S)"
+    assert noise.shape == lead + (n, S), f"noise: ({per}n, S)"
+    assert status.shape == lead + (S,), f"status: ({per}S)"
+    rows = n_nz if o.tube_packed else nent
+    outs = [(cost, "cost", (S,)), (v, "v", (nv, S)), (traj, "traj", (nt, S)), (ze1, "ze1", (rows, S)), (u, "u", (m, S))]
+    outs += [(h, what, (n, S)) for h, what in zip(hist, ("x_hist", "xbar_hist", "e_hist"))]
+    for t, what, shape in outs:
+        _chk_opt(t, what, lead + shape)
+    _chk_opt(iters, "iters", lead + (S,), torch.int32)
+    _chk_opt(x_restart, "x_restart", (n, S))
     if stats is not None:
         _chk(stats)
-        assert stats.numel() >= _abi.TZ_NSTATS, "stats: needs TZ_NSTATS doubles"
+        assert stats.numel() >= k * _abi.TZ_NSTATS, f"stats: needs {k} x TZ_NSTATS doubles"
+    _chk_warm(warm, S, warm_rows, bool(o.warm_start))
+    name = ("tz_closed_loop_step" if steps is None else "tz_closed_loop_run") + ("_set" if is_set else "") + \
+        ("_plants" if len(plant) == 1 else "")
+    with torch.cuda.device(x.device):
+        rc = getattr(_abi.lib(), name)(C.c_void_p(handle), C.byref(o), S, *lead, _ptr(x), _ptr(xbar), _ptr(e), _ptr(noise), _ptr(x_restart),
+                                       *map(_ptr, plant), _ptr(cost), _ptr(v), _ptr(traj), _ptr(ze1), _ptr(u), *map(_ptr, hist),
+                                       _ptr(status), _ptr(iters), _ptr(warm), _ptr(stats), _stream(x))
+    _abi.check(rc, name)
+
+
+# The ops take no default values: torch strips trailing defaulted arguments, which breaks mutated Optional[Tensor] args.
+_STEP_MUTATES = ("x", "xbar", "e", "cost", "v", "traj", "ze1", "u", "status", "iters", "warm", "stats")
+_RUN_MUTATES = ("x", "xbar", "e", "cost", "v", "traj", "ze1", "u", "x_hist", "xbar_hist", "e_hist", "status", "iters", "warm", "stats")
 
 
 @torch.library.custom_op("tzddpc::solve", mutates_args=("warm",), device_types="cuda")
@@ -101,56 +157,20 @@ def solve(prog: int, dims: List[int], xbar0: Tensor, e0: Tensor, warm: Optional[
           opts: List[float]) -> Tuple[Tensor, Tensor, Tensor, Tensor, Tensor, Tensor]:
     """Batched TZDDPC.solve (tzddpc/tzddpc.py:357-377).  xbar0, e0: (n, S).  dims = [n, nv, (N+1)n, n(1+g1)].
     Returns cost (S), v (nv, S), xbar (., S), Ze1.Z (n(1+g1), S), status (S), iters (S)."""
-    _chk(xbar0), _chk(e0)
-    n, nv, nt, nent = dims
-    S = xbar0.shape[1]
-    dev = xbar0.device
-    cost = torch.empty(S, dtype=torch.float64, device=dev)
-    v = torch.empty((nv, S), dtype=torch.float64, device=dev)
-    traj = torch.empty((nt, S), dtype=torch.float64, device=dev)
-    ze1 = torch.empty((nent if want_tube else 0, S), dtype=torch.float64, device=dev)
-    status = torch.empty(S, dtype=torch.int32, device=dev)
-    iters = torch.empty(S, dtype=torch.int32, device=dev)
-    o = _opts(opts)
-    d = _abi.program_dims(prog)
-    assert xbar0.shape == (d[0], S) and e0.shape == xbar0.shape, "xbar0, e0: (n, S)"
-    assert (nv, nt) == (d[2], d[3]) and (not want_tube or nent == (d[5] if o.tube_packed else d[4])), "dims do not match the program"
-    _chk_opt(warm if o.warm_start else None, "warm", S, min_rows=d[6])
-    with torch.cuda.device(dev):
-        rc = _abi.lib().tz_solve(C.c_void_p(prog), C.byref(o), S, _ptr(xbar0), _ptr(e0), _ptr(cost), _ptr(v), _ptr(traj),
-                                 _ptr(ze1) if want_tube else None, _ptr(status), _ptr(iters), _ptr(warm), _stream(xbar0))
-    _abi.check(rc, "tz_solve")
-    return cost, v, traj, ze1, status, iters
+    return _solve(prog, False, dims, xbar0, e0, warm, want_tube, opts)
 
 
-@torch.library.custom_op("tzddpc::closed_loop_step",
-                         mutates_args=("x", "xbar", "e", "cost", "v", "traj", "ze1", "u", "status", "iters", "warm", "stats"),
-                         device_types="cuda")
+@torch.library.custom_op("tzddpc::closed_loop_step", mutates_args=_STEP_MUTATES, device_types="cuda")
 def closed_loop_step(prog: int, x: Tensor, xbar: Tensor, e: Tensor, noise: Tensor, x_restart: Optional[Tensor],
                      A_true: Tensor, B_true: Tensor, status: Tensor, cost: Optional[Tensor], v: Optional[Tensor], traj: Optional[Tensor],
                      ze1: Optional[Tensor], u: Optional[Tensor], iters: Optional[Tensor], warm: Optional[Tensor],
                      stats: Optional[Tensor], opts: List[float]) -> None:
-    # (no default values: torch strips trailing defaulted arguments, which breaks mutated Optional[Tensor] args)
     """One fused closed-loop step, in place on (x, xbar, e) -- examples/2.pulley_sim.py:81-96."""
-    _chk(x), _chk(xbar), _chk(e), _chk(noise), _chk(A_true), _chk(B_true), _chk(status, torch.int32)
-    S = x.shape[1]
-    o = _opts(opts)
-    d = _abi.program_dims(prog)
-    assert x.shape == (d[0], S) and xbar.shape == x.shape and e.shape == x.shape and noise.shape == x.shape, "x, xbar, e, noise: (n, S)"
-    _chk_step(d, S, x, cost, v, traj, ze1, u, iters, warm if o.warm_start else None, stats, x_restart, status, o.tube_packed)
-    if warm is not None:
-        _chk(warm)
-    with torch.cuda.device(x.device):
-        rc = _abi.lib().tz_closed_loop_step(C.c_void_p(prog), C.byref(o), S, _ptr(x), _ptr(xbar), _ptr(e), _ptr(noise),
-                                            _ptr(x_restart), _ptr(A_true), _ptr(B_true), _ptr(cost), _ptr(v), _ptr(traj), _ptr(ze1),
-                                            _ptr(u), _ptr(status), _ptr(iters), _ptr(warm), _ptr(stats), _stream(x))
-    _abi.check(rc, "tz_closed_loop_step")
+    _closed_loop(prog, False, None, x, xbar, e, noise, x_restart, (A_true, B_true), status, cost, v, traj, ze1, u, (), iters, warm,
+                 stats, opts)
 
 
-@torch.library.custom_op("tzddpc::closed_loop_run",
-                         mutates_args=("x", "xbar", "e", "cost", "v", "traj", "ze1", "u", "x_hist", "xbar_hist", "e_hist", "status", "iters", "warm",
-                                       "stats"),
-                         device_types="cuda")
+@torch.library.custom_op("tzddpc::closed_loop_run", mutates_args=_RUN_MUTATES, device_types="cuda")
 def closed_loop_run(prog: int, steps: int, x: Tensor, xbar: Tensor, e: Tensor, noise: Tensor, x_restart: Optional[Tensor],
                     A_true: Tensor, B_true: Tensor, status: Tensor, cost: Optional[Tensor], v: Optional[Tensor], traj: Optional[Tensor],
                     ze1: Optional[Tensor], u: Optional[Tensor], x_hist: Optional[Tensor], xbar_hist: Optional[Tensor], e_hist: Optional[Tensor],
@@ -158,103 +178,30 @@ def closed_loop_run(prog: int, steps: int, x: Tensor, xbar: Tensor, e: Tensor, n
     """`steps` fused closed-loop steps in ONE launch (tz_closed_loop_run): the loop of examples/2.pulley_sim.py:81-96 for a small
     batch.  noise: (steps, n, S); per-step outputs are step-major: status / iters / cost (steps, S), v (steps, nv, S),
     traj (steps, (N+1)n, S), ze1 (steps, rows, S), u (steps, m, S), x_hist / xbar_hist / e_hist (steps, n, S), stats (steps, TZ_NSTATS)."""
-    _chk(x), _chk(xbar), _chk(e), _chk(noise), _chk(A_true), _chk(B_true), _chk(status, torch.int32)
-    S = x.shape[1]
-    o = _opts(opts)
-    d = _abi.program_dims(prog)
-    n, m, nv, nt, nent, n_nz, warm_rows = d
-    assert steps >= 1 and x.shape == (n, S) and xbar.shape == x.shape and e.shape == x.shape, "x, xbar, e: (n, S)"
-    assert noise.shape == (steps, n, S), "noise: (steps, n, S)"
-    assert status.shape == (steps, S), "status: (steps, S)"
-
-    def chk(t, shape, what, dtype=torch.float64):
-        if t is not None:
-            _chk(t, dtype)
-            assert tuple(t.shape) == shape, f"{what}: expected {shape}, got {tuple(t.shape)}"
-    chk(cost, (steps, S), "cost"), chk(iters, (steps, S), "iters", torch.int32), chk(v, (steps, nv, S), "v")
-    chk(traj, (steps, nt, S), "traj"), chk(ze1, (steps, n_nz if o.tube_packed else nent, S), "ze1"), chk(u, (steps, m, S), "u")
-    chk(x_hist, (steps, n, S), "x_hist"), chk(xbar_hist, (steps, n, S), "xbar_hist"), chk(e_hist, (steps, n, S), "e_hist")
-    chk(x_restart, (n, S), "x_restart")
-    if stats is not None:
-        _chk(stats)
-        assert stats.numel() >= steps * _abi.TZ_NSTATS, "stats: needs steps x TZ_NSTATS doubles"
-    _chk_opt(warm if o.warm_start else None, "warm", S, min_rows=warm_rows)
-    with torch.cuda.device(x.device):
-        rc = _abi.lib().tz_closed_loop_run(C.c_void_p(prog), C.byref(o), S, int(steps), _ptr(x), _ptr(xbar), _ptr(e), _ptr(noise),
-                                           _ptr(x_restart), _ptr(A_true), _ptr(B_true), _ptr(cost), _ptr(v), _ptr(traj), _ptr(ze1),
-                                           _ptr(u), _ptr(x_hist), _ptr(xbar_hist), _ptr(e_hist), _ptr(status), _ptr(iters), _ptr(warm),
-                                           _ptr(stats), _stream(x))
-    _abi.check(rc, "tz_closed_loop_run")
+    _closed_loop(prog, False, steps, x, xbar, e, noise, x_restart, (A_true, B_true), status, cost, v, traj, ze1, u,
+                 (x_hist, xbar_hist, e_hist), iters, warm, stats, opts)
 
 
-def _chk_plants(AB_true: Tensor, n: int, m: int, S: int) -> None:
-    """AB_true: (n(n+m), S), entry (i, k) of scenario s's [A_true B_true] at [i (n+m) + k, s] -- the layout sample_plants returns."""
-    _chk(AB_true)
-    assert tuple(AB_true.shape) == (n * (n + m), S), f"AB_true: expected ({n * (n + m)}, {S}), got {tuple(AB_true.shape)}"
-
-
-@torch.library.custom_op("tzddpc::closed_loop_step_plants",
-                         mutates_args=("x", "xbar", "e", "cost", "v", "traj", "ze1", "u", "status", "iters", "warm", "stats"),
-                         device_types="cuda")
+@torch.library.custom_op("tzddpc::closed_loop_step_plants", mutates_args=_STEP_MUTATES, device_types="cuda")
 def closed_loop_step_plants(prog: int, x: Tensor, xbar: Tensor, e: Tensor, noise: Tensor, x_restart: Optional[Tensor],
                             AB_true: Tensor, status: Tensor, cost: Optional[Tensor], v: Optional[Tensor], traj: Optional[Tensor],
                             ze1: Optional[Tensor], u: Optional[Tensor], iters: Optional[Tensor], warm: Optional[Tensor],
                             stats: Optional[Tensor], opts: List[float]) -> None:
-    """`closed_loop_step` with a plant per scenario: AB_true (n(n+m), S) in place of A_true, B_true."""
-    _chk(x), _chk(xbar), _chk(e), _chk(noise), _chk(status, torch.int32)
-    S = x.shape[1]
-    o = _opts(opts)
-    d = _abi.program_dims(prog)
-    assert x.shape == (d[0], S) and xbar.shape == x.shape and e.shape == x.shape and noise.shape == x.shape, "x, xbar, e, noise: (n, S)"
-    _chk_plants(AB_true, d[0], d[1], S)
-    _chk_step(d, S, x, cost, v, traj, ze1, u, iters, warm if o.warm_start else None, stats, x_restart, status, o.tube_packed)
-    if warm is not None:
-        _chk(warm)
-    with torch.cuda.device(x.device):
-        rc = _abi.lib().tz_closed_loop_step_plants(C.c_void_p(prog), C.byref(o), S, _ptr(x), _ptr(xbar), _ptr(e), _ptr(noise),
-                                                   _ptr(x_restart), _ptr(AB_true), _ptr(cost), _ptr(v), _ptr(traj), _ptr(ze1),
-                                                   _ptr(u), _ptr(status), _ptr(iters), _ptr(warm), _ptr(stats), _stream(x))
-    _abi.check(rc, "tz_closed_loop_step_plants")
+    """`closed_loop_step` with a plant per scenario: AB_true (n(n+m), S) in place of A_true, B_true; entry (i, k) of scenario s's
+    [A_true B_true] at [i (n+m) + k, s] -- the layout sample_plants returns."""
+    _closed_loop(prog, False, None, x, xbar, e, noise, x_restart, (AB_true,), status, cost, v, traj, ze1, u, (), iters, warm, stats,
+                 opts)
 
 
-@torch.library.custom_op("tzddpc::closed_loop_run_plants",
-                         mutates_args=("x", "xbar", "e", "cost", "v", "traj", "ze1", "u", "x_hist", "xbar_hist", "e_hist", "status", "iters", "warm",
-                                       "stats"),
-                         device_types="cuda")
+@torch.library.custom_op("tzddpc::closed_loop_run_plants", mutates_args=_RUN_MUTATES, device_types="cuda")
 def closed_loop_run_plants(prog: int, steps: int, x: Tensor, xbar: Tensor, e: Tensor, noise: Tensor, x_restart: Optional[Tensor],
                            AB_true: Tensor, status: Tensor, cost: Optional[Tensor], v: Optional[Tensor], traj: Optional[Tensor],
                            ze1: Optional[Tensor], u: Optional[Tensor], x_hist: Optional[Tensor], xbar_hist: Optional[Tensor],
                            e_hist: Optional[Tensor], iters: Optional[Tensor], warm: Optional[Tensor], stats: Optional[Tensor],
                            opts: List[float]) -> None:
     """`closed_loop_run` with a plant per scenario: AB_true (n(n+m), S) in place of A_true, B_true."""
-    _chk(x), _chk(xbar), _chk(e), _chk(noise), _chk(status, torch.int32)
-    S = x.shape[1]
-    o = _opts(opts)
-    d = _abi.program_dims(prog)
-    n, m, nv, nt, nent, n_nz, warm_rows = d
-    assert steps >= 1 and x.shape == (n, S) and xbar.shape == x.shape and e.shape == x.shape, "x, xbar, e: (n, S)"
-    assert noise.shape == (steps, n, S), "noise: (steps, n, S)"
-    assert status.shape == (steps, S), "status: (steps, S)"
-    _chk_plants(AB_true, n, m, S)
-
-    def chk(t, shape, what, dtype=torch.float64):
-        if t is not None:
-            _chk(t, dtype)
-            assert tuple(t.shape) == shape, f"{what}: expected {shape}, got {tuple(t.shape)}"
-    chk(cost, (steps, S), "cost"), chk(iters, (steps, S), "iters", torch.int32), chk(v, (steps, nv, S), "v")
-    chk(traj, (steps, nt, S), "traj"), chk(ze1, (steps, n_nz if o.tube_packed else nent, S), "ze1"), chk(u, (steps, m, S), "u")
-    chk(x_hist, (steps, n, S), "x_hist"), chk(xbar_hist, (steps, n, S), "xbar_hist"), chk(e_hist, (steps, n, S), "e_hist")
-    chk(x_restart, (n, S), "x_restart")
-    if stats is not None:
-        _chk(stats)
-        assert stats.numel() >= steps * _abi.TZ_NSTATS, "stats: needs steps x TZ_NSTATS doubles"
-    _chk_opt(warm if o.warm_start else None, "warm", S, min_rows=warm_rows)
-    with torch.cuda.device(x.device):
-        rc = _abi.lib().tz_closed_loop_run_plants(C.c_void_p(prog), C.byref(o), S, int(steps), _ptr(x), _ptr(xbar), _ptr(e), _ptr(noise),
-                                                  _ptr(x_restart), _ptr(AB_true), _ptr(cost), _ptr(v), _ptr(traj), _ptr(ze1),
-                                                  _ptr(u), _ptr(x_hist), _ptr(xbar_hist), _ptr(e_hist), _ptr(status), _ptr(iters),
-                                                  _ptr(warm), _ptr(stats), _stream(x))
-    _abi.check(rc, "tz_closed_loop_run_plants")
+    _closed_loop(prog, False, steps, x, xbar, e, noise, x_restart, (AB_true,), status, cost, v, traj, ze1, u,
+                 (x_hist, xbar_hist, e_hist), iters, warm, stats, opts)
 
 
 @torch.library.custom_op("tzddpc::solve_set", mutates_args=("warm",), device_types="cuda")
@@ -262,73 +209,27 @@ def solve_set(pset: int, dims: List[int], xbar0: Tensor, e0: Tensor, warm: Optio
               opts: List[float]) -> Tuple[Tensor, Tensor, Tensor, Tensor, Tensor, Tensor]:
     """`solve` over a program set (data-set axis: scenarios [begin[j], begin[j+1]) use the program of data set j).
     dims = [n, nv, (N+1)n, tube rows]."""
-    _chk(xbar0), _chk(e0)
-    n, nv, nt, nent = dims
-    S = xbar0.shape[1]
-    dev = xbar0.device
-    cost = torch.empty(S, dtype=torch.float64, device=dev)
-    v = torch.empty((nv, S), dtype=torch.float64, device=dev)
-    traj = torch.empty((nt, S), dtype=torch.float64, device=dev)
-    ze1 = torch.empty((nent if want_tube else 0, S), dtype=torch.float64, device=dev)
-    status = torch.empty(S, dtype=torch.int32, device=dev)
-    iters = torch.empty(S, dtype=torch.int32, device=dev)
-    o = _opts(opts)
-    d = _abi.program_dims(pset, True)
-    assert xbar0.shape == (d[0], S) and e0.shape == xbar0.shape, "xbar0, e0: (n, S)"
-    assert (nv, nt) == (d[2], d[3]) and (not want_tube or nent == (d[5] if o.tube_packed else d[4])), "dims do not match the program"
-    _chk_opt(warm if o.warm_start else None, "warm", S, min_rows=d[6])
-    with torch.cuda.device(dev):
-        rc = _abi.lib().tz_solve_set(C.c_void_p(pset), C.byref(o), S, _ptr(xbar0), _ptr(e0), _ptr(cost), _ptr(v), _ptr(traj),
-                                     _ptr(ze1) if want_tube else None, _ptr(status), _ptr(iters), _ptr(warm), _stream(xbar0))
-    _abi.check(rc, "tz_solve_set")
-    return cost, v, traj, ze1, status, iters
+    return _solve(pset, True, dims, xbar0, e0, warm, want_tube, opts)
 
 
-@torch.library.custom_op("tzddpc::closed_loop_step_set",
-                         mutates_args=("x", "xbar", "e", "cost", "v", "traj", "ze1", "u", "status", "iters", "warm", "stats"),
-                         device_types="cuda")
+@torch.library.custom_op("tzddpc::closed_loop_step_set", mutates_args=_STEP_MUTATES, device_types="cuda")
 def closed_loop_step_set(pset: int, x: Tensor, xbar: Tensor, e: Tensor, noise: Tensor, x_restart: Optional[Tensor],
                          A_true: Tensor, B_true: Tensor, status: Tensor, cost: Optional[Tensor], v: Optional[Tensor],
                          traj: Optional[Tensor], ze1: Optional[Tensor], u: Optional[Tensor], iters: Optional[Tensor],
                          warm: Optional[Tensor], stats: Optional[Tensor], opts: List[float]) -> None:
     """`closed_loop_step` over a program set: every data set's scenarios are stepped with that data set's program, one launch."""
-    _chk(x), _chk(xbar), _chk(e), _chk(noise), _chk(A_true), _chk(B_true), _chk(status, torch.int32)
-    S = x.shape[1]
-    o = _opts(opts)
-    d = _abi.program_dims(pset, True)
-    assert x.shape == (d[0], S) and xbar.shape == x.shape and e.shape == x.shape and noise.shape == x.shape, "x, xbar, e, noise: (n, S)"
-    _chk_step(d, S, x, cost, v, traj, ze1, u, iters, warm if o.warm_start else None, stats, x_restart, status, o.tube_packed)
-    if warm is not None:
-        _chk(warm)
-    with torch.cuda.device(x.device):
-        rc = _abi.lib().tz_closed_loop_step_set(C.c_void_p(pset), C.byref(o), S, _ptr(x), _ptr(xbar), _ptr(e), _ptr(noise),
-                                                _ptr(x_restart), _ptr(A_true), _ptr(B_true), _ptr(cost), _ptr(v), _ptr(traj),
-                                                _ptr(ze1), _ptr(u), _ptr(status), _ptr(iters), _ptr(warm), _ptr(stats), _stream(x))
-    _abi.check(rc, "tz_closed_loop_step_set")
+    _closed_loop(pset, True, None, x, xbar, e, noise, x_restart, (A_true, B_true), status, cost, v, traj, ze1, u, (), iters, warm,
+                 stats, opts)
 
 
-@torch.library.custom_op("tzddpc::closed_loop_step_set_plants",
-                         mutates_args=("x", "xbar", "e", "cost", "v", "traj", "ze1", "u", "status", "iters", "warm", "stats"),
-                         device_types="cuda")
+@torch.library.custom_op("tzddpc::closed_loop_step_set_plants", mutates_args=_STEP_MUTATES, device_types="cuda")
 def closed_loop_step_set_plants(pset: int, x: Tensor, xbar: Tensor, e: Tensor, noise: Tensor, x_restart: Optional[Tensor],
                                 AB_true: Tensor, status: Tensor, cost: Optional[Tensor], v: Optional[Tensor], traj: Optional[Tensor],
                                 ze1: Optional[Tensor], u: Optional[Tensor], iters: Optional[Tensor], warm: Optional[Tensor],
                                 stats: Optional[Tensor], opts: List[float]) -> None:
     """`closed_loop_step_set` with a plant per scenario: AB_true (n(n+m), S) in place of A_true, B_true."""
-    _chk(x), _chk(xbar), _chk(e), _chk(noise), _chk(status, torch.int32)
-    S = x.shape[1]
-    o = _opts(opts)
-    d = _abi.program_dims(pset, True)
-    assert x.shape == (d[0], S) and xbar.shape == x.shape and e.shape == x.shape and noise.shape == x.shape, "x, xbar, e, noise: (n, S)"
-    _chk_plants(AB_true, d[0], d[1], S)
-    _chk_step(d, S, x, cost, v, traj, ze1, u, iters, warm if o.warm_start else None, stats, x_restart, status, o.tube_packed)
-    if warm is not None:
-        _chk(warm)
-    with torch.cuda.device(x.device):
-        rc = _abi.lib().tz_closed_loop_step_set_plants(C.c_void_p(pset), C.byref(o), S, _ptr(x), _ptr(xbar), _ptr(e), _ptr(noise),
-                                                       _ptr(x_restart), _ptr(AB_true), _ptr(cost), _ptr(v), _ptr(traj), _ptr(ze1),
-                                                       _ptr(u), _ptr(status), _ptr(iters), _ptr(warm), _ptr(stats), _stream(x))
-    _abi.check(rc, "tz_closed_loop_step_set_plants")
+    _closed_loop(pset, True, None, x, xbar, e, noise, x_restart, (AB_true,), status, cost, v, traj, ze1, u, (), iters, warm, stats,
+                 opts)
 
 
 @torch.library.custom_op("tzddpc::interval_hull", mutates_args=(), device_types="cuda")

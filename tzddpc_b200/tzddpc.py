@@ -97,10 +97,10 @@ class TZDDPC(object):
     MdataK: MatrixZonotope
     theta: Theta
 
-    # the launch entry points (TZDDPCEnsemble swaps in the program-set variants)
+    # the launch entry points (TZDDPCEnsemble swaps in the program-set variants); the step ops for a shared plant and for a
+    # plant per scenario
     _solve_op = staticmethod(ops.solve)
-    _step_op = staticmethod(ops.closed_loop_step)
-    _step_plants_op = staticmethod(ops.closed_loop_step_plants)
+    _step_ops = (ops.closed_loop_step, ops.closed_loop_step_plants)
 
     def __init__(self, data: Data, device: Optional[Union[str, torch.device]] = None):
         """:param data: input/state data, each T x dim (tzddpc/tzddpc.py:20-28)."""
@@ -332,22 +332,22 @@ class TZDDPC(object):
     FUSED_RUN_MAX_BATCH = 256
 
     def _fused_run_ok(self, S: int, steps: int) -> bool:
-        return (type(self)._step_op is TZDDPC._step_op and steps >= 2 and S < self.FUSED_RUN_MAX_BATCH
+        return (type(self)._step_ops is TZDDPC._step_ops and steps >= 2 and S < self.FUSED_RUN_MAX_BATCH
                 and str(self._program.bucket)[:2] in ("B0", "B1", "B2", "B3") and hasattr(ops, "closed_loop_run"))
 
     def _plant_batch(self, A_true, B_true, S: int):
-        """The simulated plant as the closed-loop ops take it: (A, B, None) for one plant (n, n), (n, m) shared by the batch;
-        (None, None, AB_true) for a plant per scenario, A_true (S, n, n) and B_true (S, n, m) as numpy arrays or CUDA tensors,
-        with AB_true the (n(n+m), S) array of the *_plants ops."""
+        """The simulated plant as the closed-loop ops take it: (A, B) for one plant (n, n), (n, m) shared by the batch;
+        (AB_true,) for a plant per scenario, A_true (S, n, n) and B_true (S, n, m) as numpy arrays or CUDA tensors, with
+        AB_true the (n(n+m), S) array of the *_plants ops."""
         ndim = lambda a: a.dim() if isinstance(a, torch.Tensor) else np.ndim(a)          # noqa: E731
         if ndim(A_true) == 2 and ndim(B_true) == 2:
-            return self._t(A_true), self._t(B_true), None
+            return self._t(A_true), self._t(B_true)
         n, m = self.dim_x, self.dim_u
         dev = lambda a: a.to(self.device, torch.float64) if isinstance(a, torch.Tensor) else self._t(a)     # noqa: E731
         A, B = dev(A_true), dev(B_true)
         assert tuple(A.shape) == (S, n, n) and tuple(B.shape) == (S, n, m), \
             f"A_true, B_true: expected (n, n), (n, m) or ({S}, {n}, {n}), ({S}, {n}, {m}); got {tuple(A.shape)}, {tuple(B.shape)}"
-        return None, None, torch.cat([A, B], dim=2).reshape(S, n * (n + m)).t().contiguous()
+        return (torch.cat([A, B], dim=2).reshape(S, n * (n + m)).t().contiguous(),)
 
     def _split_plants(self, AB_true: torch.Tensor):
         """(n(n+m), S) -> A (S, n, n), B (S, n, m)"""
@@ -397,7 +397,8 @@ class TZDDPC(object):
         f64 = dict(dtype=torch.float64, device=dev)
         x, xbar = self._t(x0.T), self._t(x0.T)
         e = torch.zeros((n, S), **f64)
-        At, Bt, ABt = self._plant_batch(A_true, B_true, S)
+        plant = self._plant_batch(A_true, B_true, S)
+        per_scenario = len(plant) == 1
         xs = torch.empty((steps + 1, n, S), **f64)
         xbars = torch.empty_like(xs)
         es = torch.empty_like(xs)
@@ -415,20 +416,14 @@ class TZDDPC(object):
         h = self._program.handle.value
         if isinstance(self, TZDDPC) and self._fused_run_ok(S, steps):      # (TZDDPCEnsemble borrows this method: step loop)
             # small batch: the whole run in ONE launch (tz_closed_loop_run; bit-equal to the step loop below)
-            if ABt is None:
-                ops.closed_loop_run(h, steps, x, xbar, e, w.contiguous(), xr, At, Bt, stat, costs, vs, None, tubes if keep_tubes else None,
-                                    us, xs[1:], xbars[1:], es[1:], iters, warm, stats, o.pack())
-            else:
-                ops.closed_loop_run_plants(h, steps, x, xbar, e, w.contiguous(), xr, ABt, stat, costs, vs, None,
-                                           tubes if keep_tubes else None, us, xs[1:], xbars[1:], es[1:], iters, warm, stats, o.pack())
+            run = ops.closed_loop_run_plants if per_scenario else ops.closed_loop_run
+            run(h, steps, x, xbar, e, w.contiguous(), xr, *plant, stat, costs, vs, None, tubes, us, xs[1:], xbars[1:], es[1:], iters, warm,
+                stats, o.pack())
         else:
+            step = self._step_ops[per_scenario]
             for t in range(steps):
-                if ABt is None:
-                    self._step_op(h, x, xbar, e, w[t].contiguous(), xr, At, Bt, stat[t], costs[t], vs[t], None,
-                                  tubes[t] if keep_tubes else None, us[t], iters[t], warm, stats[t], o.pack())
-                else:
-                    self._step_plants_op(h, x, xbar, e, w[t].contiguous(), xr, ABt, stat[t], costs[t], vs[t], None,
-                                         tubes[t] if keep_tubes else None, us[t], iters[t], warm, stats[t], o.pack())
+                step(h, x, xbar, e, w[t].contiguous(), xr, *plant, stat[t], costs[t], vs[t], None, tubes[t] if keep_tubes else None, us[t],
+                     iters[t], warm, stats[t], o.pack())
                 xs[t + 1], xbars[t + 1], es[t + 1] = x, xbar, e
         out = {"x": xs.permute(0, 2, 1).cpu().numpy(), "xbar": xbars.permute(0, 2, 1).cpu().numpy(),
                "e": es.permute(0, 2, 1).cpu().numpy(), "u": us.permute(0, 2, 1).cpu().numpy(),
