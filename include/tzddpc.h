@@ -242,6 +242,19 @@ int tz_closed_loop_step_set_plants(const TzProgramSet* set, const TzSolverOpts* 
                                    const double* AB_true,
                                    double* cost, double* v, double* xbar_traj, double* ze1, double* u_out,
                                    int32_t* status, int32_t* iters, double* warm, double* stats, void* stream);
+/* tz_closed_loop_run / tz_closed_loop_run_plants over a program set: K closed-loop steps of every data set's scenarios in
+ * ONE launch, exactly K consecutive tz_closed_loop_step_set (_plants) calls, bit for bit (nsteps = 1 is one such call).
+ * The layout of tz_closed_loop_run: per-step blocks of S scenarios (K x n x S noise, K x S status, ...), the histories
+ * included.  S must be tz_program_set_scenarios(set); nsteps < 1 or another S is TZ_EINVAL. */
+int tz_closed_loop_run_set(const TzProgramSet* set, const TzSolverOpts* opts, int64_t S, int32_t nsteps, double* x, double* xbar,
+                           double* e, const double* noise, const double* x_restart, const double* A_true, const double* B_true,
+                           double* cost, double* v, double* xbar_traj, double* ze1, double* u_out, double* x_hist, double* xbar_hist,
+                           double* e_hist, int32_t* status, int32_t* iters, double* warm, double* stats, void* stream);
+int tz_closed_loop_run_set_plants(const TzProgramSet* set, const TzSolverOpts* opts, int64_t S, int32_t nsteps, double* x,
+                                  double* xbar, double* e, const double* noise, const double* x_restart, const double* AB_true,
+                                  double* cost, double* v, double* xbar_traj, double* ze1, double* u_out, double* x_hist,
+                                  double* xbar_hist, double* e_hist, int32_t* status, int32_t* iters, double* warm, double* stats,
+                                  void* stream);
 
 /* Same step with HOST buffers (pinned or pageable): H2D of (x, xbar, e, noise), the fused
  * kernel, D2H of every non-NULL output, chunked over `nchunks` internal streams so that

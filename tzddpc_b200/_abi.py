@@ -46,7 +46,8 @@ EXPORTS = ["tz_version", "tz_last_error", "tz_device_cc", "tz_program_create", "
            "tz_solve_set", "tz_closed_loop_step_set", "tz_gain_synthesis", "tz_gain_robust_samples", "tz_gain_adversary", "tz_program_dims",
            "tz_program_set_dims", "tz_closed_loop_run_host", "tz_program_create_batch",
            "tz_program_batch_get", "tz_program_batch_destroy", "tz_closed_loop_run", "tz_closed_loop_step_plants",
-           "tz_closed_loop_step_set_plants", "tz_closed_loop_run_plants", "tz_sample_plants", "tz_generate_trajectories_plants"]
+           "tz_closed_loop_step_set_plants", "tz_closed_loop_run_plants", "tz_sample_plants", "tz_generate_trajectories_plants",
+           "tz_closed_loop_run_set", "tz_closed_loop_run_set_plants"]
 
 
 def lib() -> C.CDLL:
@@ -107,6 +108,10 @@ def lib() -> C.CDLL:
     L.tz_closed_loop_step_set.argtypes = [vp, C.POINTER(TzSolverOpts), i64] + [vp] * 17
     L.tz_closed_loop_step_set_plants.restype = C.c_int
     L.tz_closed_loop_step_set_plants.argtypes = [vp, C.POINTER(TzSolverOpts), i64] + [vp] * 16
+    L.tz_closed_loop_run_set.restype = C.c_int
+    L.tz_closed_loop_run_set.argtypes = [vp, C.POINTER(TzSolverOpts), i64, C.c_int32] + [vp] * 20
+    L.tz_closed_loop_run_set_plants.restype = C.c_int
+    L.tz_closed_loop_run_set_plants.argtypes = [vp, C.POINTER(TzSolverOpts), i64, C.c_int32] + [vp] * 19
     L.tz_closed_loop_step_host_scratch_bytes.restype = C.c_size_t
     L.tz_closed_loop_step_host_scratch_bytes.argtypes = [vp, i64]
     L.tz_closed_loop_step_host.restype = C.c_int

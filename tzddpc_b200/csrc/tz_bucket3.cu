@@ -4,4 +4,5 @@
 namespace tz {
 template int launch_bucket<B3>(const TzProgram*, const SolverParams&, const StepArgs&, cudaStream_t);
 template int launch_bucket_set<B3>(const TzProgram*, const SetEntry*, int, int64_t, const SolverParams&, const StepArgs&, cudaStream_t);
+template int launch_bucket_set_run<B3>(const TzProgram*, const SetEntry*, int, int64_t, const SolverParams&, const StepArgs&, cudaStream_t);
 }

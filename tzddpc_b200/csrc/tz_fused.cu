@@ -34,6 +34,9 @@ extern template int launch_bucket<B3>(const TzProgram*, const SolverParams&, con
 extern template int launch_bucket_set<B1>(const TzProgram*, const SetEntry*, int, int64_t, const SolverParams&, const StepArgs&, cudaStream_t);
 extern template int launch_bucket_set<B2>(const TzProgram*, const SetEntry*, int, int64_t, const SolverParams&, const StepArgs&, cudaStream_t);
 extern template int launch_bucket_set<B3>(const TzProgram*, const SetEntry*, int, int64_t, const SolverParams&, const StepArgs&, cudaStream_t);
+extern template int launch_bucket_set_run<B1>(const TzProgram*, const SetEntry*, int, int64_t, const SolverParams&, const StepArgs&, cudaStream_t);
+extern template int launch_bucket_set_run<B2>(const TzProgram*, const SetEntry*, int, int64_t, const SolverParams&, const StepArgs&, cudaStream_t);
+extern template int launch_bucket_set_run<B3>(const TzProgram*, const SetEntry*, int, int64_t, const SolverParams&, const StepArgs&, cudaStream_t);
 
 constexpr int64_t kHotMinBatch = 256;
 
@@ -631,19 +634,23 @@ extern "C" int tz_closed_loop_step_plants(const TzProgram* prog, const TzSolverO
 }
 
 // ---- fused run: K closed-loop steps in one launch (small batches: the launch per step is what the step costs) -----------
-static int closed_loop_run(const TzProgram* prog, const TzSolverOpts* opts, int64_t S, int32_t nsteps, double* x, double* xbar,
-                           double* e, const double* noise, const double* x_restart, bool plants, const double* A_true,
-                           const double* B_true, const double* AB_true, double* cost, double* v, double* xbar_traj, double* ze1, double* u_out,
-                           double* x_hist, double* xbar_hist, double* e_hist, int32_t* status, int32_t* iters, double* warm,
-                           double* stats, void* stream) {
-  TZ_REQUIRE(prog != nullptr, "null program");
+// Of one program (prog, tz_closed_loop_run*) or of a program set (set, tz_closed_loop_run_set*, which check it; prog is then NULL).
+static int launch_set(const TzProgramSet* s, const TzSolverOpts* o, const StepArgs& a_in, void* stream);
+
+static int closed_loop_run(const TzProgram* prog, const TzProgramSet* set, const TzSolverOpts* opts, int64_t S, int32_t nsteps,
+                           double* x, double* xbar, double* e, const double* noise, const double* x_restart, bool plants,
+                           const double* A_true, const double* B_true, const double* AB_true, double* cost, double* v,
+                           double* xbar_traj, double* ze1, double* u_out, double* x_hist, double* xbar_hist, double* e_hist,
+                           int32_t* status, int32_t* iters, double* warm, double* stats, void* stream) {
+  TZ_REQUIRE(prog != nullptr || set != nullptr, "null program");
   TZ_REQUIRE(nsteps >= 1, "nsteps must be >= 1");
   StepArgs a;
   if (const int rc = closed_loop_args(S, x, xbar, e, noise, x_restart, plants, A_true, B_true, AB_true, cost, v, xbar_traj, ze1, u_out,
                                       status, iters, warm, stats, &a)) return rc;
-  TZ_REQUIRE(prog->bucket >= 0 && prog->bucket <= 3, "tz_closed_loop_run serves the register-bucket programs (up to 12 variables)");
   a.nsteps = nsteps; a.x_hist = x_hist; a.xbar_hist = xbar_hist; a.e_hist = e_hist;
   // (two-scenarios-per-lane output: vec2_ok wants an even batch, and then every per-step block starts 16-byte aligned too)
+  if (set != nullptr) return launch_set(set, opts, a, stream);   // (a set holds register-bucket programs only)
+  TZ_REQUIRE(prog->bucket >= 0 && prog->bucket <= 3, "tz_closed_loop_run serves the register-bucket programs (up to 12 variables)");
   return launch(prog, opts, a, stream);
 }
 
@@ -652,8 +659,8 @@ extern "C" int tz_closed_loop_run(const TzProgram* prog, const TzSolverOpts* opt
                                   const double* B_true, double* cost, double* v, double* xbar_traj, double* ze1, double* u_out,
                                   double* x_hist, double* xbar_hist, double* e_hist, int32_t* status, int32_t* iters, double* warm,
                                   double* stats, void* stream) {
-  return closed_loop_run(prog, opts, S, nsteps, x, xbar, e, noise, x_restart, false, A_true, B_true, nullptr, cost, v, xbar_traj, ze1,
-                         u_out, x_hist, xbar_hist, e_hist, status, iters, warm, stats, stream);
+  return closed_loop_run(prog, nullptr, opts, S, nsteps, x, xbar, e, noise, x_restart, false, A_true, B_true, nullptr, cost, v,
+                         xbar_traj, ze1, u_out, x_hist, xbar_hist, e_hist, status, iters, warm, stats, stream);
 }
 
 extern "C" int tz_closed_loop_run_plants(const TzProgram* prog, const TzSolverOpts* opts, int64_t S, int32_t nsteps, double* x,
@@ -661,8 +668,8 @@ extern "C" int tz_closed_loop_run_plants(const TzProgram* prog, const TzSolverOp
                                          double* cost, double* v, double* xbar_traj, double* ze1, double* u_out, double* x_hist,
                                          double* xbar_hist, double* e_hist, int32_t* status, int32_t* iters, double* warm,
                                          double* stats, void* stream) {
-  return closed_loop_run(prog, opts, S, nsteps, x, xbar, e, noise, x_restart, true, nullptr, nullptr, AB_true, cost, v, xbar_traj, ze1,
-                         u_out, x_hist, xbar_hist, e_hist, status, iters, warm, stats, stream);
+  return closed_loop_run(prog, nullptr, opts, S, nsteps, x, xbar, e, noise, x_restart, true, nullptr, nullptr, AB_true, cost, v,
+                         xbar_traj, ze1, u_out, x_hist, xbar_hist, e_hist, status, iters, warm, stats, stream);
 }
 
 // ---- tube pattern (packed Ze[1].Z) ------------------------------------------------------------------
@@ -764,7 +771,10 @@ static int launch_set(const TzProgramSet* s, const TzSolverOpts* o, const StepAr
   if (a_in.S == 0) return TZ_OK;
   const TzProgram* p0 = s->progs[0];
   const int np = (int)s->progs.size();
-  if (np == 1) return launch(p0, o, a_in, stream);       // one program: exactly step_kernel (tiles strided over the grid)
+  // a fused run (tz_closed_loop_run_set, nsteps >= 1) takes step_kernel_set_run whatever the set and the batch: it is the
+  // kernel that places the histories of every program, and prepare keeps a run of more than one step off the hot path
+  const bool run = a_in.nsteps >= 1;
+  if (np == 1 && !run) return launch(p0, o, a_in, stream);       // one program: exactly step_kernel (tiles strided over the grid)
   StepArgs a;
   SolverParams sp;
   bool hot;
@@ -772,19 +782,21 @@ static int launch_set(const TzProgramSet* s, const TzSolverOpts* o, const StepAr
   for (size_t j = 0; j + 1 < s->begin.size(); ++j)       // (every program starts on a multiple of 16 scenarios: alignment carries over)
     if ((s->begin[j + 1] - s->begin[j]) % 2 != 0) a.vec2 = 0;
   cudaStream_t st = reinterpret_cast<cudaStream_t>(stream);
-  if (hot) {
+  if (hot && !run) {
     // the hot path over a set: fast_step_kernel looks the program of every 16-scenario tile up, the tiles it defers are
     // solved by step_kernel_set_list
     if (const int rc = launch_fast_set<B0>(p0, sp, a, s->entries_dev, s->tile_prog_dev, s->block, st)) return rc;
     a.list_mode = 1;
     return launch_bucket_set_list<B0>(p0, s->entries_dev, s->tile_prog_dev, sp, a, st);
   }
+#define TZ_SET(BK) (run ? launch_bucket_set_run<BK> : launch_bucket_set<BK>)(p0, s->entries_dev, np, s->total_tiles, sp, a, st)
   switch (p0->bucket) {
-    case 0: return launch_bucket_set<B0>(p0, s->entries_dev, np, s->total_tiles, sp, a, st);
-    case 1: return launch_bucket_set<B1>(p0, s->entries_dev, np, s->total_tiles, sp, a, st);
-    case 2: return launch_bucket_set<B2>(p0, s->entries_dev, np, s->total_tiles, sp, a, st);
-    case 3: return launch_bucket_set<B3>(p0, s->entries_dev, np, s->total_tiles, sp, a, st);
+    case 0: return TZ_SET(B0);
+    case 1: return TZ_SET(B1);
+    case 2: return TZ_SET(B2);
+    case 3: return TZ_SET(B3);
   }
+#undef TZ_SET
   return fail(TZ_EINVAL, "corrupt program handle");
 }
 
@@ -817,6 +829,26 @@ extern "C" int tz_closed_loop_step_set_plants(const TzProgramSet* set, const TzS
   if (const int rc = closed_loop_args(S, x, xbar, e, noise, x_restart, true, nullptr, nullptr, AB_true, cost, v, xbar_traj, ze1, u_out,
                                       status, iters, warm, stats, &a)) return rc;
   return launch_set(set, opts, a, stream);
+}
+
+extern "C" int tz_closed_loop_run_set(const TzProgramSet* set, const TzSolverOpts* opts, int64_t S, int32_t nsteps, double* x,
+                                      double* xbar, double* e, const double* noise, const double* x_restart, const double* A_true,
+                                      const double* B_true, double* cost, double* v, double* xbar_traj, double* ze1, double* u_out,
+                                      double* x_hist, double* xbar_hist, double* e_hist, int32_t* status, int32_t* iters, double* warm,
+                                      double* stats, void* stream) {
+  TZ_REQUIRE(set != nullptr, "null program set");
+  return closed_loop_run(nullptr, set, opts, S, nsteps, x, xbar, e, noise, x_restart, false, A_true, B_true, nullptr, cost, v,
+                         xbar_traj, ze1, u_out, x_hist, xbar_hist, e_hist, status, iters, warm, stats, stream);
+}
+
+extern "C" int tz_closed_loop_run_set_plants(const TzProgramSet* set, const TzSolverOpts* opts, int64_t S, int32_t nsteps, double* x,
+                                             double* xbar, double* e, const double* noise, const double* x_restart,
+                                             const double* AB_true, double* cost, double* v, double* xbar_traj, double* ze1,
+                                             double* u_out, double* x_hist, double* xbar_hist, double* e_hist, int32_t* status,
+                                             int32_t* iters, double* warm, double* stats, void* stream) {
+  TZ_REQUIRE(set != nullptr, "null program set");
+  return closed_loop_run(nullptr, set, opts, S, nsteps, x, xbar, e, noise, x_restart, true, nullptr, nullptr, AB_true, cost, v,
+                         xbar_traj, ze1, u_out, x_hist, xbar_hist, e_hist, status, iters, warm, stats, stream);
 }
 
 extern "C" int tz_qp_solve(const TzProgram* prog, const TzSolverOpts* opts, int64_t S, const double* q, const double* l,

@@ -729,6 +729,27 @@ __device__ __forceinline__ void run_program(unsigned char* smem_raw, const QpPro
   }
 }
 
+// Step k of a fused run: noise and every per-step output advanced to their k-th block (blocks of leading dimension a.ld).
+// tube_rows: the rows of one Ze[1].Z block (0 without a tube).  step_kernel's fused run below spells the same offsets out:
+// written as a call to this function they change its register allocation (more spills).
+__device__ __forceinline__ StepArgs step_block(const StepArgs& a, const Aux& ax, const int64_t tube_rows, const int k) {
+  const int64_t LD = a.ld;
+  StepArgs ak = a;
+  if (ak.noise) ak.noise += (int64_t)k * ax.n * LD;
+  if (ak.cost) ak.cost += (int64_t)k * LD;
+  if (ak.v) ak.v += (int64_t)k * ax.nv * LD;
+  if (ak.xbar_traj) ak.xbar_traj += (int64_t)k * (ax.N + 1) * ax.n * LD;
+  if (ak.ze1) ak.ze1 += (int64_t)k * tube_rows * LD;
+  if (ak.u_out) ak.u_out += (int64_t)k * ax.m * LD;
+  ak.status += (int64_t)k * LD;
+  if (ak.iters) ak.iters += (int64_t)k * LD;
+  if (ak.stats) ak.stats += (int64_t)k * TZ_NSTATS;
+  if (ak.x_hist) ak.x_hist += (int64_t)k * ax.n * LD;
+  if (ak.xbar_hist) ak.xbar_hist += (int64_t)k * ax.n * LD;
+  if (ak.e_hist) ak.e_hist += (int64_t)k * ax.n * LD;
+  return ak;
+}
+
 // Persistent kernel of one program: one wave of CTAs.  PL: a plant per scenario (StepArgs::AB_true).
 template <class BK, bool PL = false>
 __global__ void __launch_bounds__(BK::TPB, BK::MINB) step_kernel(const QpProg<BK>* __restrict__ gpg, const Aux ax,
@@ -848,6 +869,57 @@ __global__ void __launch_bounds__(BK::TPB, BK::MINB) step_kernel_set(const SetEn
   }
 }
 
+// Fused run over a program set (tz_closed_loop_run_set): nsteps > 0 closed-loop steps in one launch.  The tiles are dealt
+// out as step_kernel_set deals them; scenarios are independent, so a warp keeps its tile of a (round, program) segment for
+// all steps, and the segment's steps run back to back behind one staging of the program image (as step_kernel's fused run
+// does for one program).  The per-step blocks are laid out with the batch's leading dimension (step_block on a0, before
+// shift_args narrows S to the program's scenarios); the histories, which shift_args leaves alone, start at the program's
+// first scenario.
+template <class BK, bool PL = false>
+__global__ void __launch_bounds__(BK::TPB, BK::MINB) step_kernel_set_run(const SetEntry* __restrict__ entries, const int nprog,
+                                                                        const int64_t total_tiles, const Aux ax0,
+                                                                        const SolverParams sp, const StepArgs a0) {
+  extern __shared__ __align__(16) unsigned char smem_raw[];
+  pdl_trigger();
+  pdl_wait();
+  const int64_t tube_rows = a0.ze1 ? (sp.tube_packed ? ax0.n_nz : ax0.n * (1 + ax0.g1)) : 0;
+  int staged = -1;                                 // program whose image is in shared memory
+  int lo = 0;
+  for (int64_t base = (int64_t)blockIdx.x * BK::WPB; base < total_tiles; base += (int64_t)gridDim.x * BK::WPB) {
+    const int64_t t1 = base + BK::WPB < total_tiles ? base + BK::WPB : total_tiles;
+    int hi = nprog - 1;                            // last program with tile_begin <= base (programs are visited in order)
+    while (lo < hi) {
+      const int mid = (lo + hi + 1) >> 1;
+      if (entries[mid].tile_begin <= base) lo = mid;
+      else hi = mid - 1;
+    }
+    int j = lo;
+    for (int64_t t = base; t < t1 && j < nprog; ++j) {
+      const SetEntry en = entries[j];
+      const int64_t ntl = (en.end - en.begin + BK::SPO - 1) / BK::SPO;
+      const int64_t tend = en.tile_begin + ntl < t1 ? en.tile_begin + ntl : t1;
+      if (tend <= t) continue;                     // (an empty program)
+      Aux ax = ax0;
+      ax.tab = en.tab;
+      const bool stage = staged != j;
+      if (stage && staged >= 0) __syncthreads();   // every warp is done with the previous program's image
+      staged = j;
+#pragma unroll 1
+      for (int k = 0; k < a0.nsteps; ++k) {
+        StepArgs a = shift_args<PL>(step_block(a0, ax0, tube_rows, k), en.begin, en.end - en.begin);
+        if (a.x_hist) a.x_hist += en.begin;
+        if (a.xbar_hist) a.xbar_hist += en.begin;
+        if (a.e_hist) a.e_hist += en.begin;
+        run_program<BK, PL>(smem_raw, reinterpret_cast<const QpProg<BK>*>(en.pg), ax, sp, a, t - en.tile_begin, BK::WPB,
+                            tend - en.tile_begin, (unsigned)((base + k) % 1024), stage && k == 0);
+        __threadfence_block();                     // step k + 1 of this warp's tile reads what step k stored
+        __syncwarp();
+      }
+      t = tend;
+    }
+  }
+}
+
 // The tiles fast_step_kernel deferred, for a program set: listed tile t (a global 16-scenario tile) belongs to program
 // tile_prog[t]; a CTA takes one listed tile at a time (its first warp solves it), re-staging the program image when the
 // program changes.  Every CTA takes an exit ticket and the last one clears the list, as step_kernel does.
@@ -962,6 +1034,20 @@ int launch_bucket_set(const TzProgram* p0, const SetEntry* entries_dev, int npro
   const unsigned grid = (unsigned)(need < wave ? need : wave);
   return with_plant(a, [&](auto pl) {
     return launch_step<BK, step_kernel_set<BK, decltype(pl)::value>>(p0, grid, st, a.S, entries_dev, nprog, total_tiles, p0->aux, sp, a);
+  });
+}
+
+// fused run over a program set (a.nsteps steps); see step_kernel_set_run.  The grid of launch_bucket_set.
+template <class BK>
+int launch_bucket_set_run(const TzProgram* p0, const SetEntry* entries_dev, int nprog, int64_t total_tiles, const SolverParams& sp,
+                          const StepArgs& a, cudaStream_t st) {
+  static_assert(BK::SPO == TZ_SPO_MIN, "tz_program_set_create counts output tiles of TZ_SPO_MIN scenarios");
+  const int64_t wave = (int64_t)p0->num_sms * BK::MINB;
+  const int64_t need = (total_tiles + BK::WPB - 1) / BK::WPB;
+  const unsigned grid = (unsigned)(need < wave ? need : wave);
+  return with_plant(a, [&](auto pl) {
+    return launch_step<BK, step_kernel_set_run<BK, decltype(pl)::value>>(p0, grid, st, a.S, entries_dev, nprog, total_tiles, p0->aux, sp,
+                                                                         a);
   });
 }
 

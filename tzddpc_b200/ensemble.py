@@ -5,7 +5,8 @@ The reference builds one `TZDDPC` object per data set -- one model M_Sigma (`tzd
 problem (`:132-241`) -- and runs the closed loops one after another (`examples/2.pulley_sim.py:62-103` repeats the whole
 script per run).  Here D controllers of identical structure are fused into a *program set* (`tz_program_set_create`):
 scenarios `[begin[j], begin[j+1])` of the batch are stepped with the program of data set j, all in ONE kernel launch per
-closed-loop step (`tz_closed_loop_step_set`).
+closed-loop step (`tz_closed_loop_step_set`), or -- below `FUSED_RUN_MAX_BATCH` scenarios -- in one launch for the whole
+run (`tz_closed_loop_run_set`).
 """
 from __future__ import annotations
 
@@ -110,6 +111,10 @@ class _LazyControllers:
 class TZDDPCEnsemble(object):
     _solve_op = staticmethod(ops.solve_set)
     _step_ops = (ops.closed_loop_step_set, ops.closed_loop_step_set_plants)
+    _run_ops = (ops.closed_loop_run_set, ops.closed_loop_run_set_plants)
+    # below FUSED_RUN_MAX_BATCH scenarios `simulate` runs the whole loop in one launch (tz_closed_loop_run_set), as TZDDPC does
+    FUSED_RUN_MAX_BATCH = TZDDPC.FUSED_RUN_MAX_BATCH
+    _fused_run_ok = TZDDPC._fused_run_ok
 
     def __init__(self, controllers: Sequence[TZDDPC], scenarios_per_dataset: Union[int, Sequence[int]]):
         """controllers: D `TZDDPC` objects on which `build_problem` has been called with the same horizon, cost and

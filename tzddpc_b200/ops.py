@@ -232,6 +232,29 @@ def closed_loop_step_set_plants(pset: int, x: Tensor, xbar: Tensor, e: Tensor, n
                  opts)
 
 
+@torch.library.custom_op("tzddpc::closed_loop_run_set", mutates_args=_RUN_MUTATES, device_types="cuda")
+def closed_loop_run_set(pset: int, steps: int, x: Tensor, xbar: Tensor, e: Tensor, noise: Tensor, x_restart: Optional[Tensor],
+                        A_true: Tensor, B_true: Tensor, status: Tensor, cost: Optional[Tensor], v: Optional[Tensor], traj: Optional[Tensor],
+                        ze1: Optional[Tensor], u: Optional[Tensor], x_hist: Optional[Tensor], xbar_hist: Optional[Tensor],
+                        e_hist: Optional[Tensor], iters: Optional[Tensor], warm: Optional[Tensor], stats: Optional[Tensor],
+                        opts: List[float]) -> None:
+    """`closed_loop_run` over a program set (tz_closed_loop_run_set): `steps` steps of every data set's scenarios in ONE launch,
+    bit-equal to `steps` calls of `closed_loop_step_set`; the layout of `closed_loop_run`."""
+    _closed_loop(pset, True, steps, x, xbar, e, noise, x_restart, (A_true, B_true), status, cost, v, traj, ze1, u,
+                 (x_hist, xbar_hist, e_hist), iters, warm, stats, opts)
+
+
+@torch.library.custom_op("tzddpc::closed_loop_run_set_plants", mutates_args=_RUN_MUTATES, device_types="cuda")
+def closed_loop_run_set_plants(pset: int, steps: int, x: Tensor, xbar: Tensor, e: Tensor, noise: Tensor, x_restart: Optional[Tensor],
+                               AB_true: Tensor, status: Tensor, cost: Optional[Tensor], v: Optional[Tensor], traj: Optional[Tensor],
+                               ze1: Optional[Tensor], u: Optional[Tensor], x_hist: Optional[Tensor], xbar_hist: Optional[Tensor],
+                               e_hist: Optional[Tensor], iters: Optional[Tensor], warm: Optional[Tensor], stats: Optional[Tensor],
+                               opts: List[float]) -> None:
+    """`closed_loop_run_set` with a plant per scenario: AB_true (n(n+m), S) in place of A_true, B_true."""
+    _closed_loop(pset, True, steps, x, xbar, e, noise, x_restart, (AB_true,), status, cost, v, traj, ze1, u,
+                 (x_hist, xbar_hist, e_hist), iters, warm, stats, opts)
+
+
 @torch.library.custom_op("tzddpc::interval_hull", mutates_args=(), device_types="cuda")
 def interval_hull(Z: Tensor) -> Tuple[Tensor, Tensor]:
     """Z: (S, n, 1+g) -> lo, hi (S, n).  Zonotope.interval (tzddpc/tzddpc.py:191-197)."""

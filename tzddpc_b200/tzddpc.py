@@ -97,10 +97,11 @@ class TZDDPC(object):
     MdataK: MatrixZonotope
     theta: Theta
 
-    # the launch entry points (TZDDPCEnsemble swaps in the program-set variants); the step ops for a shared plant and for a
-    # plant per scenario
+    # the launch entry points (TZDDPCEnsemble swaps in the program-set variants); the step ops and the fused-run ops, each for
+    # a shared plant and for a plant per scenario
     _solve_op = staticmethod(ops.solve)
     _step_ops = (ops.closed_loop_step, ops.closed_loop_step_plants)
+    _run_ops = (ops.closed_loop_run, ops.closed_loop_run_plants)
 
     def __init__(self, data: Data, device: Optional[Union[str, torch.device]] = None):
         """:param data: input/state data, each T x dim (tzddpc/tzddpc.py:20-28)."""
@@ -332,8 +333,7 @@ class TZDDPC(object):
     FUSED_RUN_MAX_BATCH = 256
 
     def _fused_run_ok(self, S: int, steps: int) -> bool:
-        return (type(self)._step_ops is TZDDPC._step_ops and steps >= 2 and S < self.FUSED_RUN_MAX_BATCH
-                and str(self._program.bucket)[:2] in ("B0", "B1", "B2", "B3") and hasattr(ops, "closed_loop_run"))
+        return steps >= 2 and S < self.FUSED_RUN_MAX_BATCH and str(self._program.bucket)[:2] in ("B0", "B1", "B2", "B3")
 
     def _plant_batch(self, A_true, B_true, S: int):
         """The simulated plant as the closed-loop ops take it: (A, B) for one plant (n, n), (n, m) shared by the batch;
@@ -414,9 +414,9 @@ class TZDDPC(object):
         xs[0], xbars[0], es[0] = x, xbar, e
         xr = x.clone() if restart else None
         h = self._program.handle.value
-        if isinstance(self, TZDDPC) and self._fused_run_ok(S, steps):      # (TZDDPCEnsemble borrows this method: step loop)
-            # small batch: the whole run in ONE launch (tz_closed_loop_run; bit-equal to the step loop below)
-            run = ops.closed_loop_run_plants if per_scenario else ops.closed_loop_run
+        if self._fused_run_ok(S, steps):
+            # small batch: the whole run in ONE launch (tz_closed_loop_run / _run_set; bit-equal to the step loop below)
+            run = self._run_ops[per_scenario]
             run(h, steps, x, xbar, e, w.contiguous(), xr, *plant, stat, costs, vs, None, tubes, us, xs[1:], xbars[1:], es[1:], iters, warm,
                 stats, o.pack())
         else:
