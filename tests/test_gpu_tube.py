@@ -34,8 +34,9 @@ def _model(seed, n=5, m=1, boxed=True):
 def _oracle_rollout(A, GK, GD, W, Z0, XU, order, metric):
     conv = oracle.Conventions(girard_metric=metric)
     n = A.shape[0]
+    W = np.zeros((n, 1)) if W is None else W                                    # no noise: W = <0, no generators>
     MK = oracle.MatrixZonotope(A, GK, conv)
-    MD = oracle.MatrixZonotope(np.zeros_like(GD[0]), GD, conv)
+    MD = oracle.MatrixZonotope(np.zeros(GD.shape[1:]), GD, conv)                # (GD may hold no generator)
     Wz = oracle.Zonotope(W[:, 0], W[:, 1:], conv)
     Z = oracle.Zonotope(Z0[:, 0], Z0[:, 1:], conv)
     hulls = []

@@ -931,15 +931,15 @@ extern "C" int tz_reach_step(int64_t S, int32_t n, int32_t p, int32_t N, int32_t
   cudaStream_t st = (cudaStream_t)stream;
   // exact-dimension fast paths: M_K (p = n) and M_Delta (p = n + 1) of the double integrator, the pulley and the 5-dim system
 #define TZ_FAST(NN, PP) \
-  if (n == NN && p == PP) return launch_reach_fast<NN, PP>(S, N, g, gW, C, Gm, per_scenario_model, Z, gW ? W : nullptr, Zout, st);
+  if (n == NN && p == PP) return launch_reach_fast<NN, PP>(S, N, g, gW, C, Gm, per_scenario_model, Z, W, Zout, st);
   TZ_FAST(2, 2) TZ_FAST(2, 3) TZ_FAST(4, 4) TZ_FAST(4, 5) TZ_FAST(5, 5) TZ_FAST(5, 6)
 #undef TZ_FAST
   if (n <= 8) {
     if (smem + 8192 > 48 * 1024) TZ_CUDA(cudaFuncSetAttribute(reach_kernel<8>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
-    reach_kernel<8><<<(unsigned)S, 256, smem, st>>>(n, p, N, g, gW, C, Gm, per_scenario_model, Z, gW ? W : nullptr, Zout);
+    reach_kernel<8><<<(unsigned)S, 256, smem, st>>>(n, p, N, g, gW, C, Gm, per_scenario_model, Z, W, Zout);
   } else {
     if (smem + 8192 > 48 * 1024) TZ_CUDA(cudaFuncSetAttribute(reach_kernel<16>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
-    reach_kernel<16><<<(unsigned)S, 256, smem, st>>>(n, p, N, g, gW, C, Gm, per_scenario_model, Z, gW ? W : nullptr, Zout);
+    reach_kernel<16><<<(unsigned)S, 256, smem, st>>>(n, p, N, g, gW, C, Gm, per_scenario_model, Z, W, Zout);
   }
   TZ_CUDA(cudaGetLastError());
   return TZ_OK;
@@ -1012,7 +1012,7 @@ extern "C" int tz_tube_rollout(int64_t S, int32_t n, int32_t m, int32_t NK, int3
   auto kernel = recompute ? tube_rollout_recompute_kernel : tube_rollout_kernel;
   if (need + 8192 > 48 * 1024) TZ_CUDA(cudaFuncSetAttribute(kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)need));
   kernel<<<(unsigned)S, kGirardThreads, need, (cudaStream_t)stream>>>(
-      n, m, NK, ND, gW, g0, steps, order, metric, gcap, (int)gpre_cap, CK, GK, GD, per_scenario_model, Z0, XU, gW ? W : nullptr,
+      n, m, NK, ND, gW, g0, steps, order, metric, gcap, (int)gpre_cap, CK, GK, GD, per_scenario_model, Z0, XU, W,
       Zfinal, gfinal, hull_lo, hull_hi);
   TZ_CUDA(cudaGetLastError());
   return TZ_OK;

@@ -69,6 +69,15 @@ def _chk_opt(t: Optional[Tensor], what: str, shape: Tuple[int, ...], dtype=torch
         assert tuple(t.shape) == shape, f"{what}: expected {shape}, got {tuple(t.shape)}"
 
 
+def _chk_W(W: Optional[Tensor], n: int) -> int:
+    """The noise zonotope W = [c_W, G_W] (n, 1+gW) of reach_step / tube_rollout, or None; returns gW."""
+    if W is None:
+        return 0
+    assert W.dim() == 2 and W.shape[1] >= 1, f"W: expected ({n}, 1+gW), got {tuple(W.shape)}"
+    _chk_opt(W, "W", (n, W.shape[1]))
+    return W.shape[1] - 1
+
+
 def _chk_warm(warm: Optional[Tensor], S: int, min_rows: int, used: bool):
     """The warm-start scratch (rows >= min_rows, S): a CUDA float64 tensor whenever given, its shape checked where `used`."""
     if warm is None:
@@ -271,16 +280,20 @@ def interval_hull(Z: Tensor) -> Tuple[Tensor, Tensor]:
 @torch.library.custom_op("tzddpc::reach_step", mutates_args=(), device_types="cuda")
 def reach_step(Cm: Tensor, Gm: Tensor, Z: Tensor, W: Optional[Tensor]) -> Tensor:
     """MatrixZonotope x Zonotope (+ W).  Cm: (n, p) or (S, n, p); Gm: (N, n, p) or (S, N, n, p);
-    Z: (S, p, 1+g); W: (n, 1+gW).  Returns (S, n, (N+1)(1+g)+gW)  (tzddpc/tzddpc.py:175-176,181,185,205)."""
-    _chk(Cm), _chk(Gm), _chk(Z)
-    per = Cm.dim() == 3
+    Z: (S, p, 1+g); W: (n, 1+gW).  Returns (S, n, (N+1)(1+g)+gW)  (tzddpc/tzddpc.py:175-176,181,185,205).
+    Every shape is checked here: the C ABI takes raw pointers, and a per-scenario Cm needs a per-scenario Gm."""
+    _chk(Z)
+    assert Z.dim() == 3, f"Z: expected (S, p, 1+g), got {tuple(Z.shape)}"
     S, p, ld = Z.shape
+    per = Cm.dim() == 3
+    lead = (S,) if per else ()
+    assert Cm.dim() in (2, 3) and Cm.shape[-2] >= 1, f"Cm: expected (n, {p}) or ({S}, n, {p}), got {tuple(Cm.shape)}"
     n = Cm.shape[-2]
+    _chk_opt(Cm, "Cm", lead + (n, p))
+    assert Gm.dim() == len(lead) + 3, f"Gm: expected {lead + ('N', n, p)} (shared / per scenario as Cm), got {tuple(Gm.shape)}"
     N = Gm.shape[-3]
-    assert Cm.shape[-1] == p and (N == 0 or Gm.shape[-1] == p)
-    gW = 0 if W is None else W.shape[1] - 1
-    if W is not None:
-        _chk(W)
+    _chk_opt(Gm, "Gm", lead + (N, n, p))
+    gW = _chk_W(W, n)
     out = torch.empty((S, n, (N + 1) * ld + gW), dtype=torch.float64, device=Z.device)
     with torch.cuda.device(Z.device):
         rc = _abi.lib().tz_reach_step(S, n, p, N, ld - 1, gW, _ptr(Cm), _ptr(Gm), int(per), _ptr(Z), _ptr(W), _ptr(out),
@@ -313,15 +326,22 @@ def tube_rollout(CK: Tensor, GK: Tensor, GD: Tensor, Z0: Tensor, XU: Tensor, W: 
     Where the pre-reduction generator block fits in shared memory (order <= 31 for the 5-dim stress system) it is built
     there every step (tube_rollout_kernel); beyond that its entries are recomputed wherever the Girard reduction reads them
     (tube_rollout_recompute_kernel, order <= 135 there), with the same results bit for bit.  Larger orders raise, naming the
-    bytes both kernels need.  TZDDPC_ROLLOUT=resident / recompute forces one kernel where it fits (include/tzddpc.h)."""
-    _chk(CK), _chk(GK), _chk(GD), _chk(Z0), _chk(XU)
-    per = CK.dim() == 3
+    bytes both kernels need.  TZDDPC_ROLLOUT=resident / recompute forces one kernel where it fits (include/tzddpc.h).
+    Every shape is checked here, as in reach_step: a per-scenario CK needs per-scenario GK and GD."""
+    _chk(Z0), _chk(XU)
+    assert Z0.dim() == 3 and Z0.shape[1] >= 1, f"Z0: expected (S, n, 1+g0), got {tuple(Z0.shape)}"
     S, n, ld0 = Z0.shape
+    assert XU.dim() == 3 and XU.shape[0] == S and XU.shape[2] > n, f"XU: expected ({S}, steps, {n}+m), got {tuple(XU.shape)}"
     steps, p = XU.shape[1], XU.shape[2]
+    per = CK.dim() == 3
+    lead = (S,) if per else ()
+    _chk_opt(CK, "CK", lead + (n, n))
+    assert GK.dim() == len(lead) + 3, f"GK: expected {lead + ('NK', n, n)} (shared / per scenario as CK), got {tuple(GK.shape)}"
+    assert GD.dim() == len(lead) + 3, f"GD: expected {lead + ('ND', n, p)} (shared / per scenario as CK), got {tuple(GD.shape)}"
     NK, ND = GK.shape[-3], GD.shape[-3]
-    gW = 0 if W is None else W.shape[1] - 1
-    if W is not None:
-        _chk(W)
+    _chk_opt(GK, "GK", lead + (NK, n, n))
+    _chk_opt(GD, "GD", lead + (ND, n, p))
+    gW = _chk_W(W, n)
     dev = Z0.device
     Zf = torch.empty((S, n, 1 + gcap), dtype=torch.float64, device=dev)
     gf = torch.empty(S, dtype=torch.int32, device=dev)
